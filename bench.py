@@ -41,7 +41,10 @@ UNIT = "Mpix/s"
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=40)
+    ap.add_argument("--steps", type=int, default=40,
+                    help="timed steps of the headline and of the per-stage split; the informational sub-records keep "
+                         "their own counts: strong scaling max(steps, 20), end to end max(4, steps // 2), multi-source "
+                         "max(5, steps // 2), eager reference on the GPU 6")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=32, help="per-GPU batch (weak scaling)")
@@ -63,7 +66,12 @@ def parse_args():
                          "items, no collective) -- sub-record strong_shard_emulation")
     ap.add_argument("--no-graph", action="store_true",
                     help="headline = the step launched from Python on one stream (default: CUDA-graph replay, two streams)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -153,6 +161,11 @@ class Stage2:
             noise=g.noise if self.noise_mode == "injected" else None,
             noise_mode="device" if self.noise_mode != "injected" else "reference")
         losses["loss"].backward()
+        # what a caller of the objective receives: the losses and the disparity gradients.  Detached: a loss kept with
+        # its grad_fn keeps this step's autograd graph alive, and the next CUDA-graph capture then fails on the stale
+        # AccumulateGrad nodes
+        self.outputs = {k.replace("/", "_"): v.detach() for k, v in losses.items()}
+        self.outputs.update({"grad_disp_%d" % s: d.grad for s, d in self.disps.items()})
         return losses["loss"]
 
 
@@ -197,6 +210,7 @@ class Stage1:
             if self.attack != "l0":
                 new_adv = torch.empty_like(self.adv)
                 self.peer.allreduce(average=True, linf=(self.adv, g.obj, 0.02, 0.1, new_adv))
+                self.outputs = {"adv_scene": adv_scene, "mask": mask_out, "patch": self.adv, "patch_next": new_adv}
                 self.adv = new_adv
                 return adv_scene
             grad_patch = self.peer.allreduce(average=True)[:self.adv.numel()].view_as(self.adv)
@@ -211,10 +225,15 @@ class Stage1:
             self.gbuf.div_(self.world)
         else:
             adv_scene, mask_out, grad_patch = ops.apply_patch_fwd_bwd(self.adv, g.mask, g.scenes, self.coeffs, g.upstream)
+        # what a caller of the step receives: the patched scenes, the resized mask, the patch gradient, the patch the
+        # step applied and the updated attack state
+        self.outputs = {"adv_scene": adv_scene, "mask": mask_out, "grad_patch": grad_patch, "patch": self.adv}
         if self.attack == "l0":
             self.l0.adam_step(grad_patch, 0.06, 0.1)
+            self.outputs.update(pattern_pos=self.l0.ppos, pattern_neg=self.l0.pneg)
         else:
             self.adv = ops.pgd_linf_step(self.adv, grad_patch, g.obj, alpha=0.02, eps=0.1)
+            self.outputs["patch_next"] = self.adv
         return adv_scene
 
 
@@ -237,6 +256,35 @@ def timed_loop(fn, steps, warmup, world):
         ms = float(t.item())
         torch.distributed.barrier()
     return ms / steps
+
+
+DUMP_MAX_ELEMENTS = 1 << 21     # per array (8 MB of fp32): at the default workload the whole dump is ~40 MB
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(outputs, out_dir):
+    """Writes every output as out_dir/<name>.npy in float32.  An array with more than DUMP_MAX_ELEMENTS elements is
+    replaced by a fixed sample of its flattened elements: DUMP_MAX_ELEMENTS seeded draws of an index, duplicates
+    dropped, in index order -- the same indices in every run, so that the dumps of two builds compare element for
+    element.  The objective's outputs repeat bit for bit; the patch gradient
+    is summed in no fixed order, so the attack state (patch, pattern_*) differs between two runs of the same build by
+    that rounding, amplified by every Adam iteration before the last timed step."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in sorted(outputs.items()):
+        flat = t.detach().float().reshape(-1)
+        if flat.numel() > DUMP_MAX_ELEMENTS:
+            idx = np.sort(np.random.default_rng(0).integers(0, flat.numel(), DUMP_MAX_ELEMENTS))
+            idx = idx[np.concatenate(([True], idx[1:] != idx[:-1]))]
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+            a = flat.cpu().numpy()
+        else:
+            a = flat.cpu().numpy().reshape(tuple(t.shape))
+        total += a.nbytes
+        if total > DUMP_MAX_BYTES:
+            raise RuntimeError("--dump-outputs: more than %d bytes" % DUMP_MAX_BYTES)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def stage1_stream(device):
@@ -606,6 +654,13 @@ def main():
         sampler.start()
         ms_step = timed_loop(step, args.steps, args.warmup, world)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        # the last timed step's results (a replay rewrites the tensors the capture allocated), before any other
+        # measurement below steps the attack state or the objective again
+        outputs = dict(s2.outputs)
+        if s1 is not None:
+            outputs.update(s1.outputs)
+        dump_outputs(outputs, args.dump_outputs)
 
     # per-stage split (same loop, one stage at a time)
     ms_s2 = timed_loop(s2.step, args.steps, 2, world)
