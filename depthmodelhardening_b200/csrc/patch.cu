@@ -148,7 +148,9 @@ __device__ __forceinline__ AaSpan aa_span(int i, int in_size, float scale) {
     AaSpan s;
     const float support = scale >= 1.0f ? scale : 1.0f;
     const float invscale = scale >= 1.0f ? 1.0f / scale : 1.0f;
-    const float center = scale * ((float)i + 0.5f);
+    // rounded before use: a bare product here would be contracted into the FMAs of `center - support` and
+    // `lo - center`, which moves the weights by up to ~3e-5 and can move the span start (ATen rounds it too)
+    const float center = mul_rn(scale, add_rn((float)i, 0.5f));
     s.lo = max((int)(center - support + 0.5f), 0);
     s.n = min((int)(center + support + 0.5f), in_size) - s.lo;
     s.n = min(s.n, AA_MAXT);
@@ -579,7 +581,7 @@ __device__ __forceinline__ float aa_weight_of(int o, int in_size, float scale, i
     // weight with which output index o reads input index ci (0 if outside its span)
     const float support = scale >= 1.0f ? scale : 1.0f;
     const float invscale = scale >= 1.0f ? 1.0f / scale : 1.0f;
-    const float center = scale * ((float)o + 0.5f);
+    const float center = mul_rn(scale, add_rn((float)o, 0.5f));     // rounded as in aa_span / aa_span3
     const int lo = max((int)(center - support + 0.5f), 0);
     int n = min((int)(center + support + 0.5f), in_size) - lo;
     n = min(n, AA_MAXT);

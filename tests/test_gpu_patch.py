@@ -92,29 +92,104 @@ def test_fused_patch_apply_vs_oracle(dev, batch):
     assert_close_arb(gp2, obj.grad, o64.grad, TOL, "grad patch (fast path)")
 
 
-@pytest.mark.parametrize("size", [(321, 1030), (200, 650), (375, 1242), (160, 512), (270, 900)])
+def resize_regime(in_hw, out_hw):
+    """The forward kernel dmh_patch_apply_fwd selects for a resize, restated op by op in float32 (aa_tile_extent
+    and the host selection of patch.cu): "3-tap 84x24" / "3-tap 104x30" (both scale factors < 1.5, tile extents
+    within the compile-time tile), "generic 8-tap" (larger down-scales) or "refused" (a factor >= 3)."""
+    f = np.float32
+    sy, sx = f(in_hw[0]) / f(out_hw[0]), f(in_hw[1]) / f(out_hw[1])
+    if sy >= 3 or sx >= 3:
+        return "refused"
+
+    def extent(tile, s):
+        support = s if s >= 1 else f(1)
+        return int(f(f(s * f(tile)) + f(f(2) * support)) + f(3))
+    if sy < 1.5 and sx < 1.5:
+        return "3-tap 84x24" if extent(64, sx) <= 84 and extent(16, sy) <= 24 else "3-tap 104x30"
+    return "generic 8-tap"
+
+
+def bwd_window_reach(in_size, out_size):
+    """patch_apply_bwd_kernel visits, for one canvas pixel ci, the outputs ox_a(ci) + k; the first 8 (MAXO) from
+    registers, the rest in its remainder loop.  Returns 1 + the largest k at which an output actually reads ci with a
+    non-zero weight (3-tap spans, float32 as in the kernel): above 8 the remainder loop contributes."""
+    f = np.float32
+    s = f(in_size) / f(out_size)
+    sup = s if s >= 1 else f(1)
+    inv = f(1) / s if s >= 1 else f(1)
+    o = np.arange(out_size)
+    center = (s * (o.astype(np.float32) + f(0.5))).astype(np.float32)
+    lo = np.maximum((center - sup + f(0.5)).astype(np.float32).astype(np.int64), 0)
+    n = np.minimum(np.minimum((center + sup + f(0.5)).astype(np.float32).astype(np.int64), in_size) - lo, 3)
+    reach = 0
+    for j in range(3):
+        arg = ((f(j) + (lo.astype(np.float32) - center)).astype(np.float32) + f(0.5)).astype(np.float32) * inv
+        ci = lo + j
+        live = (j < n) & (np.abs(arg) < 1)
+        ox_a = np.maximum(0, np.floor(((ci.astype(np.float32) - sup).astype(np.float32) - f(0.5)) / s).astype(np.int64) - 1)
+        if live.any():
+            reach = max(reach, int((o - ox_a)[live].max()) + 1)
+    return reach
+
+
+# the resize regime each output size of 375 x 1242 is meant to exercise: a retuned switch point fails loudly
+RAGGED_SIZES = {(321, 1030): "3-tap 84x24", (200, 650): "generic 8-tap", (375, 1242): "3-tap 84x24",
+                (160, 512): "generic 8-tap", (270, 900): "3-tap 104x30",
+                (307, 1000): "3-tap 84x24",        # top of the 84 x 24 tile (extents 84 / 24)
+                (306, 999): "3-tap 104x30",        # just over it (85 / 25)
+                (307, 999): "3-tap 104x30", (306, 1000): "3-tap 104x30",      # one axis over the limit each
+                (251, 829): "3-tap 104x30",        # scales 1.494 / 1.498: the 8-row vertical window can be full
+                (250, 828): "generic 8-tap",       # exactly 1.5
+                (126, 415): "generic 8-tap",       # 2.98 / 2.99: the largest shared-memory tile
+                (640, 2048): "3-tap 84x24", (750, 2484): "3-tap 84x24",      # up-scaling, within 8 outputs
+                (960, 3200): "3-tap 84x24"}        # up-scaling by 2.56 / 2.58
+# output sizes whose backward reads outputs beyond the 8 it keeps in registers (bwd_window_reach > 8)
+REMAINDER_SIZES = {(960, 3200)}
+
+
+@pytest.mark.parametrize("size", list(RAGGED_SIZES))
 def test_fused_patch_apply_ragged_output_sizes(dev, size):
-    """Output sizes that are not multiples of the 64 x 16 tile, both tap-count instantiations of the resize
-    (scale < 1.5: 3 taps per axis; larger down-scales: generic 8) and the identity resize: forward and the
-    gradient to the patch against the oracle."""
+    """Output sizes that are not multiples of the 64 x 16 tile, on both sides of every switch between the resize
+    kernels (3-tap windows in an 84 x 24 or a 104 x 30 tile, the generic 8-tap kernel), the identity resize and
+    up-scales, one of them far enough that the backward reads outputs beyond the 8 it keeps in registers: forward
+    and the gradient to the patch against the oracle, with the ellipse mask and with an all-ones mask that reaches
+    the patch border."""
     from depthmodelhardening_b200 import patch_ops
+    assert resize_regime((375, 1242), size) == RAGGED_SIZES[size]
+    assert (bwd_window_reach(1242, size[1]) > 8) == (size in REMAINDER_SIZES)
     pbt = synth.patch_batch(batch=2, seed=3)
     up = synth.randn((2, 3) + size, 904) * 1e-3
-    obj = pbt.obj.clone().requires_grad_(True)
-    adv_ref, m_ref = OQ.apply_patch(obj, pbt.mask, pbt.scenes, pbt.z0, pbt.alpha, P34, size=size)
-    (adv_ref * up).sum().backward()
-    o64 = pbt.obj.double().requires_grad_(True)
-    adv64, m64 = OQ.apply_patch(o64, pbt.mask.double(), pbt.scenes.double(), pbt.z0, pbt.alpha, P34, size=size)
-    (adv64 * up.double()).sum().backward()
     g = pbt.to(dev)
     co = patch_ops.homographies(pbt.z0, pbt.alpha, P34).to(dev)
-    obj_d = g.obj.clone().requires_grad_(True)
-    adv, m = patch_ops.apply_patch(obj_d, g.mask, g.scenes, co, size=size)
-    (adv * up.to(dev)).sum().backward()
-    assert torch.isfinite(adv).all() and torch.isfinite(m).all()
-    assert_close_arb(adv, adv_ref, adv64, TOL, "adv scene %s" % (size,))
-    assert_close_arb(m, m_ref, m64, TOL, "resized mask")
-    assert_close_arb(obj_d.grad, obj.grad, o64.grad, TOL, "grad patch")
+    for kind, mask in (("ellipse", pbt.mask), ("ones", torch.ones_like(pbt.mask))):
+        what = "%s %s" % (size, kind)
+        obj = pbt.obj.clone().requires_grad_(True)
+        adv_ref, m_ref = OQ.apply_patch(obj, mask, pbt.scenes, pbt.z0, pbt.alpha, P34, size=size)
+        (adv_ref * up).sum().backward()
+        o64 = pbt.obj.double().requires_grad_(True)
+        adv64, m64 = OQ.apply_patch(o64, mask.double(), pbt.scenes.double(), pbt.z0, pbt.alpha, P34, size=size)
+        (adv64 * up.double()).sum().backward()
+        obj_d = g.obj.clone().requires_grad_(True)
+        adv, m = patch_ops.apply_patch(obj_d, mask.to(dev), g.scenes, co, size=size)
+        (adv * up.to(dev)).sum().backward()
+        assert torch.isfinite(adv).all() and torch.isfinite(m).all()
+        assert_close_arb(adv, adv_ref, adv64, TOL, "adv scene " + what)
+        assert_close_arb(m, m_ref, m64, TOL, "resized mask " + what)
+        assert_close_arb(obj_d.grad, obj.grad, o64.grad, TOL, "grad patch " + what)
+
+
+@pytest.mark.parametrize("size", [(125, 414), (100, 400)])
+def test_fused_patch_apply_refuses_down_scale_of_3(dev, size):
+    """A down-scale factor of 3 or more needs anti-aliasing windows wider than the kernels' 8 taps: refused."""
+    from depthmodelhardening_b200 import patch_ops
+    assert resize_regime((375, 1242), size) == "refused"
+    g = synth.patch_batch(batch=2, seed=3).to(dev)
+    co = patch_ops.homographies(g.z0, g.alpha, P34).to(dev)
+    up = torch.zeros((2, 3) + size, device=dev)
+    with pytest.raises(RuntimeError, match="down-scale factor"):
+        patch_ops.apply_patch(g.obj, g.mask, g.scenes, co, size=size)
+    with pytest.raises(RuntimeError, match="down-scale factor"):
+        patch_ops.apply_patch_fwd_bwd(g.obj, g.mask, g.scenes, co, up, size=size)
 
 
 def test_fused_patch_apply_vs_golden(dev):
@@ -431,11 +506,13 @@ def _resnet18_monodepth2(dev):
     return _Monodepth2ResNet18().to(dev)
 
 
-@pytest.mark.parametrize("net", ["tiny", "resnet18"])
-def test_attack_classes_vs_oracle_loop_same_device(dev, calib, net):
+@pytest.mark.parametrize("net, dists", [("tiny", range(5, 10, 2)), ("resnet18", range(5, 10, 2)),
+                                        ("tiny", range(5, 31, 2))], ids=["tiny", "resnet18", "tiny-far"])
+def test_attack_classes_vs_oracle_loop_same_device(dev, calib, net, dists):
     """Our attack classes against the oracle's restatement of the reference loops, BOTH driven on the GPU with
     the same network, so the only difference is kernels vs torch ops.  `resnet18`: the random-init ResNet-18
-    monodepth2 encoder / decoder BASELINE.json names (_Monodepth2ResNet18)."""
+    monodepth2 encoder / decoder BASELINE.json names (_Monodepth2ResNet18).  `tiny-far`: the classes' own default
+    distances, 5-29 m."""
     import os
     from depthmodelhardening_b200 import attacks
     attacks.object_dataset_root = os.path.dirname(os.path.dirname(os.path.dirname(calib)))
@@ -446,7 +523,7 @@ def test_attack_classes_vs_oracle_loop_same_device(dev, calib, net):
     # the reference project's own ResnetEncoder / DepthDecoder, whose seeded weights differ from _Monodepth2ResNet18's)
     flips = 5e-3 if net == "tiny" else 2e-2
     l0_atol = 1e-4
-    dist, ang = list(range(5, 10, 2)), list(range(-30, 31, 5))
+    dist, ang = list(dists), list(range(-30, 31, 5))
     # ---- L-inf, 3 steps
     pl, fin = _placements(9, 3, (dist, ang), 3)
     ref = OQ.linf_attack(model, pbt.obj, pbt.mask, pbt.scenes, pl, fin, P34, eps=0.1, alpha=0.02)

@@ -289,14 +289,14 @@ def test_cuda_compose_is_bit_exact_on_identical_inputs(dev, flip):
 @pytest.mark.gpu
 def test_cuda_fused_compose_equals_warp_then_compose(dev):
     """dmh_compose_patch_u8 (warp inside, two patches, mask image) == dmh_perspective_fwd + dmh_compose_u8, bit for
-    bit, with and without the placement boxes, mixed flips."""
+    bit, with and without the placement boxes, mixed flips, near and far (15 m, 29 m) placements."""
     from depthmodelhardening_b200 import loader, patch_ops
     ben, adv, mask = patches()
     ben, adv, mask = ben.to(dev), adv.to(dev), mask.to(dev)
-    z0, al = [5.0, 6.5, 8.0, 9.0], [-30.0, -5.0, 10.0, 30.0]
+    z0, al = [5.0, 6.5, 8.0, 9.0, 15.0, 29.0], [-30.0, -5.0, 10.0, 30.0, -20.0, 25.0]
     place = patch_ops.homographies(z0, al, P34, K=LC.adv_K(), T=LC.STEREO_T).to(dev)
-    scenes = synth.frames_u8(55, batch=4).to(dev)
-    flip = torch.tensor([0, 1, 1, 0], dtype=torch.int32)
+    scenes = synth.frames_u8(55, batch=6).to(dev)
+    flip = torch.tensor([0, 1, 1, 0, 1, 0], dtype=torch.int32)
     hw = (synth.ORI_H, synth.ORI_W)
     mw = patch_ops.perspective_batch(mask, place, hw)
     ref_a = loader.compose_u8(scenes, patch_ops.perspective_batch(adv, place, hw), mw, flip)

@@ -81,25 +81,33 @@ def test_install_rebinds_reference_symbols():
 
 def test_placement_bbox_is_conservative():
     """Every canvas pixel that samples the patch (per the oracle's perspective warp of an all-ones
-    image) lies inside the host-computed bounding box the fused apply kernels use as a skip hint."""
+    image) lies inside the host-computed bounding box the fused apply kernels use as a skip hint: a few near
+    placements, and every distance and angle the attack classes draw (range(5, 31, 2) and the non-integer distances of
+    np.linspace(5, 30, 7), the 5-degree angle grid and the odd angles of range(-30, 31, 2))."""
     from oracle import patch as OQ
     zs = [5.0, 5.4, 7.0, 9.8, 6.2, 9.0]
     als = [-30.0, 30.0, 0.0, 25.0, -15.0, 5.0]
+    for z in sorted(set(float(z) for z in range(5, 31, 2)) | set(np.linspace(5, 30, 7).tolist())):
+        for a in range(-30, 31):
+            if a % 5 == 0 or a % 2 == 0:
+                zs.append(z)
+                als.append(float(a))
     ones = torch.ones(1, 1, 260, 300)
     place = patch_ops.homographies(zs, als, P34)
-    assert place.bbox.dtype == torch.int32 and place.bbox.shape == (6, 4)
-    assert place.shape == (6, 8)
+    assert place.bbox.dtype == torch.int32 and place.bbox.shape == (len(zs), 4)
+    assert place.shape == (len(zs), 8)
     padded, start = OQ.pad_to_canvas(ones)
     for i, (z, a) in enumerate(zip(zs, als)):
         end = OQ.corners_on_image(z, a, P34)
         warped = OQ.perspective_warp(padded, OQ.perspective_coeffs(start, end.tolist()))[0, 0]
         ys, xs = torch.nonzero(warped > 0, as_tuple=True)
         x0, y0, x1, y1 = place.bbox[i].tolist()
-        assert xs.numel() > 1000
-        assert int(xs.min()) >= x0 and int(xs.max()) <= x1 and int(ys.min()) >= y0 and int(ys.max()) <= y1
+        where = "z0=%g alpha=%g" % (z, a)
+        assert xs.numel() > 1000, where
+        assert int(xs.min()) >= x0 and int(xs.max()) <= x1 and int(ys.min()) >= y0 and int(ys.max()) <= y1, where
         # ... and is not vacuous: within a few pixels of the true extent
-        assert int(xs.min()) - x0 <= 8 and x1 - int(xs.max()) <= 8
-        assert place.bbox_wh[0] >= x1 - x0 + 1 and place.bbox_wh[1] >= y1 - y0 + 1
+        assert int(xs.min()) - x0 <= 8 and x1 - int(xs.max()) <= 8, where
+        assert place.bbox_wh[0] >= x1 - x0 + 1 and place.bbox_wh[1] >= y1 - y0 + 1, where
 
 
 def test_install_rebinds_every_patch_attack_class():
