@@ -55,9 +55,6 @@ SIGNATURES = {
     "dmh_photo_tiles": (_i, [_i, _i]),
     "dmh_photo_scale": (_i, [_f, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), _i, _f, _i, _i, _f, _f, _f, _f, _i, _i, _i,
                              _fl, _fl, _i, _fl, _f, _f, _f, _f, C.POINTER(C.c_void_p), _st]),
-    "dmh_photo_split_workspace_floats": (_ll, [_i, _i, _i]),
-    "dmh_photo_scale_split": (_i, [_f, _f, _f, _f, _i, _i, _f, _f, _f, _f, _i, _i, _i, _fl, _fl, _i, _fl, _f, _f, _f, _f,
-                                   _st]),
     "dmh_photo_multiscale": (_i, [_f, _f, _f, _i, C.POINTER(C.c_void_p), C.POINTER(C.c_int), C.POINTER(C.c_int), _f, _f, _f,
                                   C.POINTER(C.c_void_p), _i, _i, _i, _fl, _fl, _fl, C.POINTER(C.c_void_p),
                                   C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), _st]),
@@ -78,11 +75,6 @@ SIGNATURES = {
                                   _f, _st]),
     "dmh_objective_finish_workspace_bytes": (_ll, [_i, _i]),
     "dmh_disp_grad": (_i, [_f, _f, _f, _fl, _f, _f, _f, _fl, _i, _i, _i, _i, _i, _f, _st]),
-    "dmh_smooth_fused_multi": (_i, [_i, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), _i, C.POINTER(C.c_int),
-                                    C.POINTER(C.c_int), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), _st]),
-    "dmh_disp_grad_multi": (_i, [_i, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
-                                 C.POINTER(C.c_float), _f, C.POINTER(C.c_void_p), _f, _fl, _i, C.POINTER(C.c_int),
-                                 C.POINTER(C.c_int), _i, _i, C.POINTER(C.c_void_p), _st]),
     "dmh_compose_u8": (_i, [_f, _f, _f, _f, _i, _i, _i, _i, _f, _st]),
     "dmh_compose_patch_u8": (_i, [_f, _f, _f, _f, _f, _f, _f, _f, _i, _i, _i, _i, _i, _f, _f, _f, _st]),
     "dmh_lanczos_u8": (_i, [_f, _i, _i, _i, _i, _i, _f, _f, _i, _f, _f, _i, _f, _f, _f, _st]),

@@ -32,7 +32,7 @@ namespace {
 #define SF_RPW 4
 #define SF_BLOCKS(h, w) ((((w) + SF_TW - 1) / SF_TW) * (((h) + SF_TH - 1) / SF_TH))
 
-// (body shared by the per-scale launch and the all-scales launch: bx < SF_NB1 = block of this image)
+// bx < SF_NB1 = block of this image
 __device__ __forceinline__ void sf_mean_body(const float* __restrict__ disp, int hw, float* __restrict__ part, int b,
                                              int bx, float* red) {
     const float* d = disp + (size_t)b * hw;
@@ -67,30 +67,6 @@ sf_mean_kernel(const float* __restrict__ disp, int hw, float* __restrict__ part)
     sf_mean_body(disp, hw, part, blockIdx.y, blockIdx.x, red);
 }
 
-// all scales in one launch (dmh_smooth_fused_multi): per-scale arguments in a __grid_constant__ table
-#define SF_MAXS 8
-struct SfScale {
-    const float* disp;
-    const float* img;
-    float* ws;                   // [B*64 mean partials][B*nb*3 partials]
-    float* gN;
-    int h, w, gx, gy;
-    float inv_nx, inv_ny;
-    int vec;
-    int blk0;                    // first linear block of this scale in sf_main_multi_kernel's grid
-};
-struct SfMultiParams {
-    SfScale sc[SF_MAXS];
-    int S, B;
-};
-
-__global__ void __launch_bounds__(SF_THREADS)
-sf_mean_multi_kernel(const __grid_constant__ SfMultiParams p) {
-    __shared__ float red[32];
-    const SfScale& c = p.sc[blockIdx.z];
-    sf_mean_body(c.disp, c.h * c.w, c.ws, blockIdx.y, blockIdx.x, red);
-}
-
 // mean(disp_b) + 1e-7 from the 64 partials; called by the 32 lanes of one warp, same
 // summation order wherever it is used (forward normalisation and its backward)
 __device__ __forceinline__ float mean_eps_warp(const float* __restrict__ mean_part, int b, int hw) {
@@ -120,8 +96,8 @@ __device__ __forceinline__ void load_px4(const float* __restrict__ row, int x, i
     }
 }
 
-// (Every product-sum below is written with an explicit rounding sequence -- mul_rn / fmaf -- so that the per-scale and
-// the all-scales instantiation of this body cannot differ by the compiler's FMA contraction choices: measured, they did.)
+// (Every product-sum below is written with an explicit rounding sequence -- mul_rn / fmaf -- so that the result does
+// not depend on the compiler's FMA contraction choices.)
 // A16 forward + gradient w.r.t. the normalised disparity.  A lane owns 4 consecutive pixels of a row and
 // walks down SF_RPW rows keeping the previous row in registers, so every disparity / colour value is loaded
 // once per warp (128-bit loads) plus one row of overlap above and below; the edge weight exp(-mean_c|dI|)
@@ -269,21 +245,6 @@ sf_main_kernel(const float* __restrict__ disp, const float* __restrict__ img, in
                float* __restrict__ part) {
     sf_main_body<C>(disp, img, h, w, mean_part, inv_nx, inv_ny, vec, gN, part, blockIdx.x, blockIdx.y, blockIdx.z,
                     gridDim.x, gridDim.y);
-}
-
-// all scales in one launch: linear grid, the blocks of scale 0 (the largest) first
-__global__ void __launch_bounds__(SF_THREADS, 4)
-sf_main_multi_kernel(const __grid_constant__ SfMultiParams p) {
-    const int blk = blockIdx.x;
-    int s = 0;
-#pragma unroll 1
-    while (s + 1 < p.S && blk >= p.sc[s + 1].blk0) ++s;
-    const SfScale& c = p.sc[s];
-    const int r = blk - c.blk0, per = c.gx * c.gy;
-    const int b = r / per, t = r - b * per;
-    const int by = t / c.gx, bx = t - by * c.gx;
-    sf_main_body<3>(c.disp, c.img, c.h, c.w, c.ws, c.inv_nx, c.inv_ny, c.vec, c.gN, c.ws + (size_t)p.B * SF_NB1, bx, by, b,
-                    c.gx, c.gy);
 }
 
 #define FIN_MAXS 8
@@ -561,61 +522,6 @@ disp_grad_same_kernel(const float4* __restrict__ G4, const float4* __restrict__ 
                         blockIdx.x * blockDim.x + threadIdx.x, blockIdx.y);
 }
 
-// All scales of the backward in ONE launch (dmh_disp_grad_multi): linear grid of 256-thread CTAs, the blocks of the
-// same-size scale first, then the tall tiles of the integer factors 2 / 4 / 8.  Same arithmetic per output value as
-// the per-scale kernels above (their bodies).
-#define DG_MAXS 8
-struct DgScale {
-    const float* G;
-    const float* gN;
-    const float* img_scalars;
-    const float* g_scale;
-    float* grad;
-    float smooth_weight, sh, sw;
-    int h, w, R, gx, gy;         // R == 1: gx = blocks of 1024 float4 per image, gy unused
-    int blk0;
-};
-struct DgMultiParams {
-    DgScale sc[DG_MAXS];
-    const float* g_total;
-    const float* g_smooth;
-    float inv_S;
-    int S, B, H, W;
-};
-
-__global__ void __launch_bounds__(256, 3)
-disp_grad_multi_kernel(const __grid_constant__ DgMultiParams p) {
-    __shared__ float smem[DG_UP_SMEM(8)];
-    const int blk = blockIdx.x;
-    int s = 0;
-#pragma unroll 1
-    while (s + 1 < p.S && blk >= p.sc[s + 1].blk0) ++s;
-    const DgScale& c = p.sc[s];
-    const int r = blk - c.blk0;
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    if (c.R == 1) {
-        // four 128-bit chunks per thread (the all-scales kernel is register-capped by its up-sampling branches: fewer
-        // resident threads than the per-scale streaming kernel, so each keeps more loads in flight)
-        const int b = r / c.gx, bx = r - b * c.gx;
-#pragma unroll
-        for (int j = 0; j < 4; ++j)
-            disp_grad_same_body(reinterpret_cast<const float4*>(c.G), reinterpret_cast<const float4*>(c.gN), c.img_scalars,
-                                c.smooth_weight, p.g_total, c.g_scale, p.g_smooth, p.inv_S, (c.h * c.w) >> 2,
-                                reinterpret_cast<float4*>(c.grad), bx * 1024 + j * 256 + (int)threadIdx.x, b);
-        return;
-    }
-    const int per = c.gx * c.gy;
-    const int b = r / per, t = r - b * per;
-    const int by = t / c.gx, bx = t - by * c.gx;
-#define DMH_DGM(RR)                                                                                                       \
-    disp_grad_up_body<RR>(c.G, c.gN, c.img_scalars, c.smooth_weight, p.g_total, c.g_scale, p.g_smooth, p.inv_S, c.h, c.w, \
-                          p.H, p.W, c.sh, c.sw, c.grad, bx, by, b, lane, wid, smem)
-    if (c.R == 2) DMH_DGM(2);
-    else if (c.R == 4) DMH_DGM(4);
-    else DMH_DGM(8);
-#undef DMH_DGM
-}
-
 template <int R>
 __global__ void __launch_bounds__(256)
 disp_grad_kernel(const float* __restrict__ G_full, const float* __restrict__ gN,
@@ -763,38 +669,6 @@ int dmh_smooth_fused(const float* disp, const float* img, int B, int C, int h, i
     return DMH_OK;
 }
 
-/* All S scales of the smoothness term in TWO launches (sf_mean for every scale, then sf_main for every scale) instead
- * of 2 S: same arithmetic per value as dmh_smooth_fused, i.e. identical outputs.  3-channel images only. */
-int dmh_smooth_fused_multi(int S, const float* const* disp_host, const float* const* img_host, int B, const int* h_host,
-                           const int* w_host, float* const* ws_host, float* const* gN_host, dmh_stream_t stream) {
-    DMH_REQUIRE(disp_host && img_host && h_host && w_host && ws_host && gN_host, "dmh_smooth_fused_multi: null pointer");
-    DMH_REQUIRE(S >= 1 && S <= SF_MAXS && B > 0 && B <= 65535, "dmh_smooth_fused_multi: S=%d outside [1,%d] or bad B", S,
-                SF_MAXS);
-    SfMultiParams p;
-    memset(&p, 0, sizeof(p));
-    p.S = S; p.B = B;
-    long long blocks = 0;
-    for (int s = 0; s < S; ++s) {
-        const int h = h_host[s], w = w_host[s];
-        DMH_REQUIRE(disp_host[s] && img_host[s] && ws_host[s] && gN_host[s] && h >= 2 && w >= 2,
-                    "dmh_smooth_fused_multi: scale %d: null buffer or bad shape", s);
-        SfScale& c = p.sc[s];
-        c.disp = disp_host[s]; c.img = img_host[s]; c.ws = ws_host[s]; c.gN = gN_host[s];
-        c.h = h; c.w = w; c.gx = ceil_div(w, SF_TW); c.gy = ceil_div(h, SF_TH);
-        c.inv_nx = (float)(1.0 / ((double)B * h * (w - 1)));
-        c.inv_ny = (float)(1.0 / ((double)B * (h - 1) * w));
-        c.vec = (w % 4 == 0) && (((uintptr_t)c.disp | (uintptr_t)c.img | (uintptr_t)c.gN) % 16 == 0);
-        c.blk0 = (int)blocks;
-        blocks += (long long)c.gx * c.gy * B;
-    }
-    DMH_REQUIRE(blocks < (1ll << 31), "dmh_smooth_fused_multi: grid too large");
-    cudaStream_t st = (cudaStream_t)stream;
-    DMH_LAUNCH(sf_mean_multi_kernel, dim3(SF_NB1, B, S), SF_THREADS, 0, st)(p);
-    DMH_LAUNCH(sf_main_multi_kernel, (unsigned)blocks, SF_THREADS, 0, st)(p);
-    DMH_CHECK_LAUNCH("dmh_smooth_fused_multi");
-    return DMH_OK;
-}
-
 long long dmh_objective_finish_workspace_bytes(int S, int B) { return 16 + 24LL * S * B; }
 
 int dmh_objective_finish(int S, int B, const float* const* smooth_ws_host, const int* h_host, const int* w_host,
@@ -859,55 +733,6 @@ int dmh_disp_grad(const float* G_full, const float* gN, const float* img_scalars
     else DMH_DG(0);
 #undef DMH_DG
     DMH_CHECK_LAUNCH("dmh_disp_grad");
-    return DMH_OK;
-}
-
-/* The backward of all S scales in ONE launch: scale s as dmh_disp_grad(G_full[s], gN[s], img_scalars[s], ...) with
- * u_s = *g_total * inv_S + *g_scale[s].  Returns DMH_ERR_UNSUPPORTED (nothing launched) unless every scale is the
- * same-size case or an integer factor 2 / 4 / 8 with 16-byte aligned rows: the caller then uses dmh_disp_grad. */
-int dmh_disp_grad_multi(int S, const float* const* G_full_host, const float* const* gN_host,
-                        const float* const* img_scalars_host, const float* smooth_weight_host, const float* g_total,
-                        const float* const* g_scale_host, const float* g_smooth, float inv_S, int B, const int* h_host,
-                        const int* w_host, int H, int W, float* const* grad_disp_host, dmh_stream_t stream) {
-    DMH_REQUIRE(G_full_host && h_host && w_host && grad_disp_host && smooth_weight_host && (g_total || g_scale_host),
-                "dmh_disp_grad_multi: null pointer");
-    DMH_REQUIRE(S >= 1 && S <= DG_MAXS && B > 0 && B <= 65535, "dmh_disp_grad_multi: S=%d outside [1,%d] or bad B", S,
-                DG_MAXS);
-    DgMultiParams p;
-    memset(&p, 0, sizeof(p));
-    p.S = S; p.B = B; p.H = H; p.W = W; p.g_total = g_total; p.g_smooth = g_smooth; p.inv_S = inv_S;
-    long long blocks = 0;
-    for (int s = 0; s < S; ++s) {
-        const int h = h_host[s], w = w_host[s];
-        DMH_REQUIRE(G_full_host[s] && grad_disp_host[s] && h >= 1 && w >= 1 && H >= h && W >= w &&
-                        (long long)H * W < (1ll << 31),
-                    "dmh_disp_grad_multi: scale %d: null buffer or bad shape", s);
-        const float* gn = gN_host ? gN_host[s] : nullptr;
-        DMH_REQUIRE(!gn || (img_scalars_host && img_scalars_host[s]), "dmh_disp_grad_multi: gN given without img_scalars");
-        DMH_REQUIRE(g_total || (g_scale_host && g_scale_host[s]), "dmh_disp_grad_multi: scale %d has no upstream scalar", s);
-        int R = 0;
-        if (H % h == 0 && W % w == 0 && H / h == W / w) R = H / h;
-        const bool aligned = (uintptr_t)G_full_host[s] % 16 == 0 && W % 4 == 0;
-        const bool same_ok = R == 1 && ((size_t)h * w) % 4 == 0 && (uintptr_t)G_full_host[s] % 16 == 0 &&
-                             (uintptr_t)grad_disp_host[s] % 16 == 0 && (!gn || (uintptr_t)gn % 16 == 0);
-        if (!(same_ok || ((R == 2 || R == 4 || R == 8) && aligned))) {
-            set_error("dmh_disp_grad_multi: scale %d (%dx%d of %dx%d) needs the generic kernel; use dmh_disp_grad", s, h, w,
-                      H, W);
-            return DMH_ERR_UNSUPPORTED;
-        }
-        DgScale& c = p.sc[s];
-        c.G = G_full_host[s]; c.gN = gn; c.img_scalars = gn ? img_scalars_host[s] : nullptr;
-        c.g_scale = g_scale_host ? g_scale_host[s] : nullptr; c.grad = grad_disp_host[s];
-        c.smooth_weight = smooth_weight_host[s]; c.sh = (float)h / (float)H; c.sw = (float)w / (float)W;
-        c.h = h; c.w = w; c.R = R;
-        if (R == 1) { c.gx = ceil_div((int)(((size_t)h * w) / 4), 1024); c.gy = 1; }
-        else { c.gx = ceil_div(w, 32); c.gy = ceil_div(h, 64 / R); }
-        c.blk0 = (int)blocks;
-        blocks += (long long)c.gx * c.gy * B;
-    }
-    DMH_REQUIRE(blocks < (1ll << 31), "dmh_disp_grad_multi: grid too large");
-    DMH_LAUNCH(disp_grad_multi_kernel, (unsigned)blocks, 256, 0, (cudaStream_t)stream)(p);
-    DMH_CHECK_LAUNCH("dmh_disp_grad_multi");
     return DMH_OK;
 }
 

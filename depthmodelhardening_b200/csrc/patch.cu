@@ -20,8 +20,6 @@
 //   sample: grid_sample(bilinear, zeros, align_corners=False) (:545-561)
 //   resize: F.interpolate(bilinear, antialias=True, align_corners=False)
 //           (ATen UpSample.cuh upsample_antialias::_compute_weights*)
-#include <stdlib.h>
-
 #include <mutex>
 #include <vector>
 
@@ -832,14 +830,12 @@ namespace {
 // Weight tables of the 3-tap forward kernel, one per (device, sizes), built on first use: a 20 KB allocation and one
 // small launch on a private stream, waited for once.  Never built while the caller's stream is being captured (an
 // allocation would invalidate the capture): the kernel then computes its weights itself, as it does when the table
-// cannot be built -- same values either way.  DMH_AA_TABLE=0 disables the table.
+// cannot be built -- same values either way.
 struct AaTabEntry { int dev, ih, iw, oh, ow; float4* tab; };
 std::mutex g_aa_mu;
 std::vector<AaTabEntry> g_aa_tabs;
 
 const float4* aa_table_get(int ih, int iw, int oh, int ow, float sy, float sx, cudaStream_t st) {
-    static const bool enabled = [] { const char* e = getenv("DMH_AA_TABLE"); return !(e && atoi(e) == 0); }();
-    if (!enabled) return nullptr;
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) return nullptr;
     std::lock_guard<std::mutex> lk(g_aa_mu);

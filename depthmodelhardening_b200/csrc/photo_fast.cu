@@ -26,9 +26,7 @@
 // Roofline: HBM by traffic (40 B per target pixel, 419 MB per launch at B=32 -- ncu measures exactly that), but
 // instruction-issue bound in practice: ~745 lane-instructions / pixel at ~57 % issue utilisation (profiles/).
 //
-// Also here: ident_fast_kernel (identity reprojection loss + the packed copy, both tiles by TMA) and the
-// two-kernel alternative warp_pred_kernel + photo_fast_kernel<SPLIT> (dmh_photo_scale_split: bit-identical,
-// measured slower, opt-in).
+// Also here: ident_fast_kernel (identity reprojection loss + the packed copy, both tiles by TMA).
 //
 // Target tile staging: ONE elected thread issues a 4-D TMA load
 // (cp.async.bulk.tensor, box 40 x 36 x 3 x 1 at (x0-4, y0-2, 0, b) -- the innermost
@@ -53,12 +51,9 @@ namespace {
 // PK: pixel-packed source (128-bit taps); UP: the disparity map is smaller than the frame (scales 1..3).
 // SSIM is always on and the input is a disparity here (no_ssim, depth inputs and the materialised warped images
 // take the general kernel).
-// SPLIT: the warp was done by warp_pred_kernel (below): the warped tile arrives by a second TMA load from its padded,
-// reflect-bordered output and the backward factors D from global memory -- this kernel is then phases B and C only.
-template <bool TMA, bool FASTDIV, bool PK, bool UP, bool SPLIT, bool DH = false>
+template <bool TMA, bool FASTDIV, bool PK, bool UP, bool DH = false>
 __global__ void __launch_bounds__(FT_THREADS, 3)
-photo_fast_kernel(const FastParams p, const __grid_constant__ CUtensorMap tgt_map,
-                  const __grid_constant__ CUtensorMap pred_map) {
+photo_fast_kernel(const FastParams p, const __grid_constant__ CUtensorMap tgt_map) {
     extern __shared__ __align__(128) float smem[];
     __shared__ __align__(8) uint64_t tgt_bar;
     float* tgt = smem;                       // [3][36][40] (TMA destination: 128-byte aligned)
@@ -79,8 +74,7 @@ photo_fast_kernel(const FastParams p, const __grid_constant__ CUtensorMap tgt_ma
     const int N = H * W;                      // per-item offsets fit 32 bits (checked by the launcher)
     const float w_ssim = 0.85f / 3.0f, w_l1 = 0.15f / 3.0f;
 
-    if (SPLIT) {
-    } else if (tid < 12) {
+    if (tid < 12) {
         const int i = tid / 4, j = tid % 4;
         const float* k = p.K + b * 16 + i * 4;
         const float* tt = p.T + b * 16 + j;
@@ -97,10 +91,8 @@ photo_fast_kernel(const FastParams p, const __grid_constant__ CUtensorMap tgt_ma
         // ---- target tile by TMA: in flight during the whole gather phase
         if (tid == 0) {
             mbar_init(&tgt_bar, 1);
-            mbar_expect_tx(&tgt_bar, (3 * FT_NT + (SPLIT ? 3 * FT_N2 : 0)) * sizeof(float));
+            mbar_expect_tx(&tgt_bar, 3 * FT_NT * sizeof(float));
             tma_load_4d(tgt, &tgt_map, &tgt_bar, x0 - 2 - FT_TO, y0 - 2, 0, b);
-            // warped tile: the padded layout puts image column x at x + 2, so the halo start x0 - 2 is column x0
-            if (SPLIT) tma_load_4d(pred, &pred_map, &tgt_bar, x0, y0, 0, b);
         }
     } else if (tid < FT_R2 * 7) {
         // ---- target tile, 2-px reflect halo: 36 columns x 7 row groups = 252 threads, column index maths once
@@ -115,80 +107,78 @@ photo_fast_kernel(const FastParams p, const __grid_constant__ CUtensorMap tgt_ma
     __syncthreads();
     const int oc = tid & 31, os = tid >> 5;
     float D[4][3];
-    if (!SPLIT) {
-        Camera cam;
+    Camera cam;
 #pragma unroll
-        for (int i = 0; i < 12; ++i) cam.P[i] = cams[i];
+    for (int i = 0; i < 12; ++i) cam.P[i] = cams[i];
 #pragma unroll
-        for (int i = 0; i < 9; ++i) cam.iK[i] = cams[12 + i];
-        const float* sp = p.src + (size_t)b * (PK ? 4 : 3) * N;
-        const float* dp = p.disp.ptr + (size_t)b * (p.disp.h * p.disp.w);
+    for (int i = 0; i < 9; ++i) cam.iK[i] = cams[12 + i];
+    const float* sp = p.src + (size_t)b * (PK ? 4 : 3) * N;
+    const float* dp = p.disp.ptr + (size_t)b * (p.disp.h * p.disp.w);
 
-        // ---- phase A: warp.  A thread owns the interior pixels of column tid%32, rows 4*(tid/32)+k, plus one pixel
-        // of the halo ring.  Software-pipelined over those 5 pixels: all disparity loads, then the coordinate chains,
-        // then the gathers -- the memory latency is paid once per stage instead of once per pixel.
-        {
-            int hr, hc;
-            halo_rc(tid, hr, hc);
-            int py[5], pxx[5];
-            const int ixo = tile_to_img(x0 + oc, W);
+    // ---- phase A: warp.  A thread owns the interior pixels of column tid%32, rows 4*(tid/32)+k, plus one pixel
+    // of the halo ring.  Software-pipelined over those 5 pixels: all disparity loads, then the coordinate chains,
+    // then the gathers -- the memory latency is paid once per stage instead of once per pixel.
+    {
+        int hr, hc;
+        halo_rc(tid, hr, hc);
+        int py[5], pxx[5];
+        const int ixo = tile_to_img(x0 + oc, W);
 #pragma unroll
-            for (int k = 0; k < 4; ++k) { py[k] = tile_to_img(y0 + 4 * os + k, H); pxx[k] = ixo; }
-            py[4] = ext_to_img(y0 - 2 + hr, H);
-            pxx[4] = ext_to_img(x0 - 2 + hc, W);
-            float dv[5];
-            if (!UP) {
+        for (int k = 0; k < 4; ++k) { py[k] = tile_to_img(y0 + 4 * os + k, H); pxx[k] = ixo; }
+        py[4] = ext_to_img(y0 - 2 + hr, H);
+        pxx[4] = ext_to_img(x0 - 2 + hc, W);
+        float dv[5];
+        if (!UP) {
 #pragma unroll
-                for (int k = 0; k < 5; ++k) dv[k] = __ldg(dp + py[k] * W + pxx[k]);
-            } else {
-                const UpTap txo = up_tap(ixo, p.disp.sw, p.disp.w);        // shared by the 4 owned pixels
+            for (int k = 0; k < 5; ++k) dv[k] = __ldg(dp + py[k] * W + pxx[k]);
+        } else {
+            const UpTap txo = up_tap(ixo, p.disp.sw, p.disp.w);        // shared by the 4 owned pixels
 #pragma unroll
-                for (int k = 0; k < 4; ++k) dv[k] = up_sample(dp, p.disp.w, up_tap(py[k], p.disp.sh, p.disp.h), txo);
-                dv[4] = up_sample(dp, p.disp.w, up_tap(py[4], p.disp.sh, p.disp.h), up_tap(pxx[4], p.disp.sw, p.disp.w));
+            for (int k = 0; k < 4; ++k) dv[k] = up_sample(dp, p.disp.w, up_tap(py[k], p.disp.sh, p.disp.h), txo);
+            dv[4] = up_sample(dp, p.disp.w, up_tap(py[4], p.disp.sh, p.disp.h), up_tap(pxx[4], p.disp.sw, p.disp.w));
+        }
+        Tap tp[5];
+        float gax[5], gay[5];
+#pragma unroll
+        for (int k = 0; k < 5; ++k) tp[k] = pixel_tap<FASTDIV>(cam, p, pxx[k], py[k], dv[k], k < 4, gax[k], gay[k]);
+        // gathers: the taps of TWO pixels are requested before either is consumed
+#pragma unroll
+        for (int k0 = 0; k0 < 5; k0 += 2) {
+            float tv[2][3][4];
+#pragma unroll
+            for (int j = 0; j < 2; ++j) {
+                if (k0 + j < 5) load_taps<PK>(sp, N, W, tp[k0 + j], tv[j]);
             }
-            Tap tp[5];
-            float gax[5], gay[5];
 #pragma unroll
-            for (int k = 0; k < 5; ++k) tp[k] = pixel_tap<FASTDIV>(cam, p, pxx[k], py[k], dv[k], k < 4, gax[k], gay[k]);
-            // gathers: the taps of TWO pixels are requested before either is consumed
+            for (int j = 0; j < 2; ++j) {
+                const int k = k0 + j;
+                if (k >= 5) continue;
+                const Gathered g = combine_taps(tv[j], tp[k], k < 4);
+                const int r = 4 * os + k;
+                const int i2 = (k < 4) ? (r + 2) * FT_R2 + oc + 2 : hr * FT_R2 + hc;
 #pragma unroll
-            for (int k0 = 0; k0 < 5; k0 += 2) {
-                float tv[2][3][4];
+                for (int ch = 0; ch < 3; ++ch) pred[ch * FT_N2 + i2] = g.v[ch];
+                if (k < 4) {
 #pragma unroll
-                for (int j = 0; j < 2; ++j) {
-                    if (k0 + j < 5) load_taps<PK>(sp, N, W, tp[k0 + j], tv[j]);
-                }
-#pragma unroll
-                for (int j = 0; j < 2; ++j) {
-                    const int k = k0 + j;
-                    if (k >= 5) continue;
-                    const Gathered g = combine_taps(tv[j], tp[k], k < 4);
-                    const int r = 4 * os + k;
-                    const int i2 = (k < 4) ? (r + 2) * FT_R2 + oc + 2 : hr * FT_R2 + hc;
-#pragma unroll
-                    for (int ch = 0; ch < 3; ++ch) pred[ch * FT_N2 + i2] = g.v[ch];
-                    if (k < 4) {
-#pragma unroll
-                        for (int ch = 0; ch < 3; ++ch) D[k][ch] = g.dix[ch] * gax[k] + g.diy[ch] * gay[k];
-                    }
+                    for (int ch = 0; ch < 3; ++ch) D[k][ch] = g.dix[ch] * gax[k] + g.diy[ch] * gay[k];
                 }
             }
         }
-        // the remaining 16 pixels of the halo ring
-        if (tid < 272 - FT_THREADS) {
-            int r, c;
-            halo_rc(tid + FT_THREADS, r, c);
-            const int iy = ext_to_img(y0 - 2 + r, H), ix = ext_to_img(x0 - 2 + c, W);
-            const float dvh = UP ? up_sample(dp, p.disp.w, up_tap(iy, p.disp.sh, p.disp.h), up_tap(ix, p.disp.sw, p.disp.w))
-                                 : __ldg(dp + iy * W + ix);
-            float u0, u1;
-            const Tap th = pixel_tap<FASTDIV>(cam, p, ix, iy, dvh, false, u0, u1);
-            float tvh[3][4];
-            load_taps<PK>(sp, N, W, th, tvh);
-            const Gathered g = combine_taps(tvh, th, false);
+    }
+    // the remaining 16 pixels of the halo ring
+    if (tid < 272 - FT_THREADS) {
+        int r, c;
+        halo_rc(tid + FT_THREADS, r, c);
+        const int iy = ext_to_img(y0 - 2 + r, H), ix = ext_to_img(x0 - 2 + c, W);
+        const float dvh = UP ? up_sample(dp, p.disp.w, up_tap(iy, p.disp.sh, p.disp.h), up_tap(ix, p.disp.sw, p.disp.w))
+                             : __ldg(dp + iy * W + ix);
+        float u0, u1;
+        const Tap th = pixel_tap<FASTDIV>(cam, p, ix, iy, dvh, false, u0, u1);
+        float tvh[3][4];
+        load_taps<PK>(sp, N, W, th, tvh);
+        const Gathered g = combine_taps(tvh, th, false);
 #pragma unroll
-            for (int ch = 0; ch < 3; ++ch) pred[ch * FT_N2 + r * FT_R2 + c] = g.v[ch];
-        }
+        for (int ch = 0; ch < 3; ++ch) pred[ch * FT_N2 + r * FT_R2 + c] = g.v[ch];
     }
     // identity losses (+ tie-break noise) of this thread's phase-B pixels: requested before the barrier so
     // that their latency overlaps the other warps' gather.  Ring pixels outside the image are marked by a NaN
@@ -221,18 +211,6 @@ photo_fast_kernel(const FastParams p, const __grid_constant__ CUtensorMap tgt_ma
     float acc4[4] = {0.f, 0.f, 0.f, 0.f};
     const float loss_local = phase_b<DH, UP>(p, sm, tid, b, x0, y0, idv_pre, hflags, acc4);
     __syncthreads();
-    if (SPLIT) {
-        // d(pred)/d(disp) factors of this thread's 4 pixels, written by warp_pred_kernel (loaded here, not before
-        // phase B: 12 registers less across the SSIM phase)
-        const float* dg = p.dfac + (size_t)b * 3 * N + x0 + oc;
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const int y = y0 + 4 * os + k;
-            const bool in = y < H && x0 + oc < W;
-#pragma unroll
-            for (int ch = 0; ch < 3; ++ch) D[k][ch] = in ? __ldg(dg + ch * N + y * W) : 0.0f;
-        }
-    }
     phase_c<DH, UP>(p, sm, tid, b, x0, y0, D, acc4);
     const int blk = (b * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x;
     if (DH) {
@@ -248,313 +226,6 @@ photo_fast_kernel(const FastParams p, const __grid_constant__ CUtensorMap tgt_ma
     }
 }
 
-
-// ---------------------------------------------------------------------------
-// Producer / consumer form: a persistent CTA of 12 warps walks over the tiles.  Warps 8-11 (producers) gather the
-// warped tile of tile i+1 into the second shared-memory buffer and start its target TMA while warps 0-7 (consumers)
-// run phases B and C of tile i: neither the gather latency nor the phase barriers of one tile leave the SM's issue
-// slots idle.  Hand-off through mbarriers (full[s]: 128 producer arrivals + the TMA bytes; empty[s]: 256 consumer
-// arrivals); consumers synchronise among themselves with named barrier 1, producers with named barrier 2.  The
-// backward factors D travel through global memory (written by the producer, read back through L2 by the consumer
-// that owns the pixel in phase C).  2 CTAs per SM (108.6 KB each).  Same arithmetic, same bits as the fused kernel.
-#define PC_CONS 256
-#ifndef PC_PROD
-#define PC_PROD 256
-#endif
-#define PC_THREADS (PC_CONS + PC_PROD)
-#define PC_CTAS (PC_PROD == 128 ? 2 : 1)
-#define PC_HALVES (1024 / (PC_PROD * 4))          // groups of 4 rows per producer thread
-#define PC_NH ((272 + PC_PROD - 1) / PC_PROD)      // halo pixels per producer thread (the last one partial)
-
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void named_bar(int id, int count) {
-    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(count) : "memory");
-}
-
-template <bool FASTDIV, bool PK, bool UP>
-__global__ void __launch_bounds__(PC_THREADS, PC_CTAS)
-photo_pc_kernel(const FastParams p, const __grid_constant__ CUtensorMap tgt_map, int tiles_x, int tiles_y, int ntiles) {
-    extern __shared__ __align__(128) float smem[];
-    __shared__ __align__(8) uint64_t full_bar[2], empty_bar[2];
-    // buffers s = 0, 1: target tiles at smem + s * 3*FT_NT (TMA destinations, 128-byte aligned), warped tiles after
-    float4* q1 = reinterpret_cast<float4*>(smem + 6 * FT_NT + 6 * FT_N2);
-    float4* q2 = q1 + FT_N1;
-    float* q3 = reinterpret_cast<float*>(q2 + FT_N1);
-    float* cams = q3 + FT_N1;                 // [2][24]
-    float* red = cams + 48;                   // [32]
-    uint8_t* gate = reinterpret_cast<uint8_t*>(red + 32);
-
-    const int tid = threadIdx.x;
-    const int H = p.H, W = p.W, N = H * W;
-    if (tid == 0) {
-        mbar_init(&full_bar[0], PC_PROD + 1); mbar_init(&full_bar[1], PC_PROD + 1);
-        mbar_init(&empty_bar[0], PC_CONS); mbar_init(&empty_bar[1], PC_CONS);
-    }
-    __syncthreads();
-    const int per_img = tiles_x * tiles_y;
-
-    if (tid >= PC_CONS) {
-        // ================================================================ producers
-        const int pt = tid - PC_CONS;
-        const int pc_ = pt & 31, pw = pt >> 5;                       // column, row group of the interior
-        int it = 0;
-        for (int t = blockIdx.x; t < ntiles; t += gridDim.x, ++it) {
-            const int s = it & 1, ph = (it >> 1) & 1;
-            const int b = t / per_img, rem = t - b * per_img;
-            const int ty = rem / tiles_x, tx = rem - ty * tiles_x;
-            const int x0 = tx * FT_T, y0 = ty * FT_T;
-            mbar_wait(&empty_bar[s], ph ^ 1);
-            if (pt == 0) {
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                mbar_expect_tx(&full_bar[s], 3 * FT_NT * sizeof(float));
-                tma_load_4d(smem + s * 3 * FT_NT, &tgt_map, &full_bar[s], x0 - 2 - FT_TO, y0 - 2, 0, b);
-            }
-            float* cm = cams + 24 * s;
-            if (pt < 12) {
-                const int i = pt / 4, j = pt % 4;
-                const float* k = p.K + b * 16 + i * 4;
-                const float* tt = p.T + b * 16 + j;
-                float acc = __ldg(k) * __ldg(tt);
-                acc = fmaf(__ldg(k + 1), __ldg(tt + 4), acc);
-                acc = fmaf(__ldg(k + 2), __ldg(tt + 8), acc);
-                acc = fmaf(__ldg(k + 3), __ldg(tt + 12), acc);
-                cm[pt] = acc;
-            } else if (pt < 21) {
-                const int i = (pt - 12) / 3, j = (pt - 12) % 3;
-                cm[pt] = __ldg(p.inv_K + b * 16 + i * 4 + j);
-            }
-            named_bar(2, PC_PROD);
-            Camera cam;
-#pragma unroll
-            for (int i = 0; i < 12; ++i) cam.P[i] = cm[i];
-#pragma unroll
-            for (int i = 0; i < 9; ++i) cam.iK[i] = cm[12 + i];
-            const float* sp = p.src + (size_t)b * (PK ? 4 : 3) * N;
-            const float* dp = p.disp.ptr + (size_t)b * (p.disp.h * p.disp.w);
-            float* pred = smem + 6 * FT_NT + s * 3 * FT_N2;
-            float* dout = p.dfac_out + (size_t)b * 3 * N;
-            // ---- interior: column pc_, rows 8*pw .. 8*pw+7, four at a time (column taps shared)
-            const int ixo = tile_to_img(x0 + pc_, W);
-#pragma unroll 1
-            for (int half = 0; half < PC_HALVES; ++half) {
-                const int rb = 4 * PC_HALVES * pw + 4 * half;
-                int py[4];
-                float dv[4];
-#pragma unroll
-                for (int k = 0; k < 4; ++k) py[k] = tile_to_img(y0 + rb + k, H);
-                if (!UP) {
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) dv[k] = __ldg(dp + py[k] * W + ixo);
-                } else {
-                    const UpTap txo = up_tap(ixo, p.disp.sw, p.disp.w);
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) dv[k] = up_sample(dp, p.disp.w, up_tap(py[k], p.disp.sh, p.disp.h), txo);
-                }
-                Tap tp[4];
-                float gax[4], gay[4];
-#pragma unroll
-                for (int k = 0; k < 4; ++k) tp[k] = pixel_tap<FASTDIV>(cam, p, ixo, py[k], dv[k], true, gax[k], gay[k]);
-#pragma unroll
-                for (int k0 = 0; k0 < 4; k0 += 2) {
-                    float tv[2][3][4];
-#pragma unroll
-                    for (int j = 0; j < 2; ++j) load_taps<PK>(sp, N, W, tp[k0 + j], tv[j]);
-#pragma unroll
-                    for (int j = 0; j < 2; ++j) {
-                        const int k = k0 + j, r = rb + k;
-                        const Gathered g = combine_taps(tv[j], tp[k], true);
-                        const int i2 = (r + 2) * FT_R2 + pc_ + 2;
-                        const bool in = y0 + r < H && x0 + pc_ < W;
-#pragma unroll
-                        for (int ch = 0; ch < 3; ++ch) {
-                            pred[ch * FT_N2 + i2] = g.v[ch];
-                            if (in) dout[ch * N + (y0 + r) * W + x0 + pc_] = g.dix[ch] * gax[k] + g.diy[ch] * gay[k];
-                        }
-                    }
-                }
-            }
-            // ---- halo ring: 272 pixels, up to 3 per thread (the third only for the first 16 threads)
-            {
-                int hr[PC_NH], hc[PC_NH];
-                Tap th[PC_NH];
-                const int nh = pt < 272 - (PC_NH - 1) * PC_PROD ? PC_NH : PC_NH - 1;
-#pragma unroll
-                for (int j = 0; j < PC_NH; ++j) {
-                    if (j < nh) {
-                        halo_rc(pt + PC_PROD * j, hr[j], hc[j]);
-                        const int iy = ext_to_img(y0 - 2 + hr[j], H), ix = ext_to_img(x0 - 2 + hc[j], W);
-                        const float dvh = UP ? up_sample(dp, p.disp.w, up_tap(iy, p.disp.sh, p.disp.h),
-                                                         up_tap(ix, p.disp.sw, p.disp.w))
-                                             : __ldg(dp + iy * W + ix);
-                        float u0, u1;
-                        th[j] = pixel_tap<FASTDIV>(cam, p, ix, iy, dvh, false, u0, u1);
-                    }
-                }
-#pragma unroll
-                for (int j = 0; j < PC_NH; ++j) {
-                    if (j < nh) {
-                        float tvh[3][4];
-                        load_taps<PK>(sp, N, W, th[j], tvh);
-                        const Gathered g = combine_taps(tvh, th[j], false);
-#pragma unroll
-                        for (int ch = 0; ch < 3; ++ch) pred[ch * FT_N2 + hr[j] * FT_R2 + hc[j]] = g.v[ch];
-                    }
-                }
-            }
-            __threadfence_block();
-            mbar_arrive(&full_bar[s]);
-        }
-    } else {
-        // ================================================================ consumers
-        const int oc = tid & 31, os = tid >> 5;
-        int it = 0;
-        for (int t = blockIdx.x; t < ntiles; t += gridDim.x, ++it) {
-            const int s = it & 1, ph = (it >> 1) & 1;
-            const int b = t / per_img, rem = t - b * per_img;
-            const int ty = rem / tiles_x, tx = rem - ty * tiles_x;
-            const int x0 = tx * FT_T, y0 = ty * FT_T;
-            float idv_pre[FT_ROWS];
-            unsigned hflags;
-            prefetch_ident<false>(p, tid, b, x0, y0, idv_pre, hflags);
-            mbar_wait(&full_bar[s], ph);
-            float* tgt = smem + s * 3 * FT_NT;
-            if (x0 < 2 || y0 < 2 || x0 + FT_T + 2 > W || y0 + FT_T + 2 > H) {      // ReflectionPad2d(1) of the target
-                for (int i = tid; i < FT_N2; i += PC_CONS) {
-                    const int r = i / FT_R2, c = i - r * FT_R2;
-                    const int ey = y0 - 2 + r, ex = x0 - 2 + c;
-                    if (ey < 0 || ey >= H || ex < 0 || ex >= W) {
-                        const int sr = ext_to_img(ey, H) - (y0 - 2), sc = ext_to_img(ex, W) - (x0 - 2);
-#pragma unroll
-                        for (int ch = 0; ch < 3; ++ch)
-                            tgt[ch * FT_NT + r * FT_TP + c + FT_TO] = tgt[ch * FT_NT + sr * FT_TP + sc + FT_TO];
-                    }
-                }
-                named_bar(1, PC_CONS);
-            }
-            TileSmem sm;
-            sm.tgt = tgt; sm.pred = smem + 6 * FT_NT + s * 3 * FT_N2; sm.q1 = q1; sm.q2 = q2; sm.q3 = q3; sm.gate = gate;
-            float acc4[4];
-            const float loss_local = phase_b<false, UP>(p, sm, tid, b, x0, y0, idv_pre, hflags, acc4);
-            // backward factors of this thread's 4 pixels (written by the producer of this CTA: read through L2)
-            float D[4][3];
-            {
-                const float* dg = p.dfac_out + (size_t)b * 3 * N + x0 + oc;
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                    const int y = y0 + 4 * os + k;
-                    const bool in = y < H && x0 + oc < W;
-#pragma unroll
-                    for (int ch = 0; ch < 3; ++ch) D[k][ch] = in ? __ldcg(dg + ch * N + y * W) : 0.0f;
-                }
-            }
-            const float wsum = warp_sum(loss_local);
-            if ((tid & 31) == 0) red[tid >> 5] = wsum;
-            named_bar(1, PC_CONS);                                   // coefficient planes + red[] complete
-            phase_c<false, UP>(p, sm, tid, b, x0, y0, D, acc4);
-            if (tid == 0) {
-                float tot = 0.f;
-#pragma unroll
-                for (int i = 0; i < PC_CONS / 32; ++i) tot += red[i];
-                p.loss_partial[t] = tot;
-            }
-            mbar_arrive(&empty_bar[s]);                              // this thread is done with buffer s
-            named_bar(1, PC_CONS);                                   // nobody still reads the coefficient planes / red[]
-        }
-    }
-}
-
-// ---------------------------------------------------------------------------
-// Split design, kernel 1: the warp alone.  One thread per 4 pixels of a column (no halo: every pixel of the frame is
-// gathered exactly once, against 1.27x in the fused kernel), low register / no shared-memory footprint, i.e. enough
-// resident warps to hide the gather latency.  Writes
-//   predp (B,3,H+4,WP): the warped frame with a 2-pixel border, image pixel (x,y) at (x+2,y+2); the border holds the
-//          ReflectionPad2d mirror (columns -1 / W = columns 1 / W-2, rows alike; the outer border ring only needs to
-//          be finite), so that the loss kernel's TMA box starts on a 16-byte boundary and needs no patching;
-//   dfac  (B,3,H,W): d(pred_ch)/d(disp) * grad_scale (the collapsed backward chain of the gather).
-template <bool FASTDIV, bool PK, bool UP>
-__global__ void __launch_bounds__(FT_THREADS, 4)
-warp_pred_kernel(const FastParams p) {
-    __shared__ float cams[24];
-    const int tid = threadIdx.x;
-    const int H = p.H, W = p.W;
-    const int b = blockIdx.z;
-    const int x0 = blockIdx.x * FT_T, y0 = blockIdx.y * FT_T;
-    const int N = H * W;
-    if (tid < 12) {
-        const int i = tid / 4, j = tid % 4;
-        const float* k = p.K + b * 16 + i * 4;
-        const float* tt = p.T + b * 16 + j;
-        float acc = __ldg(k) * __ldg(tt);
-        acc = fmaf(__ldg(k + 1), __ldg(tt + 4), acc);
-        acc = fmaf(__ldg(k + 2), __ldg(tt + 8), acc);
-        acc = fmaf(__ldg(k + 3), __ldg(tt + 12), acc);
-        cams[tid] = acc;
-    } else if (tid < 21) {
-        const int i = (tid - 12) / 3, j = (tid - 12) % 3;
-        cams[tid] = __ldg(p.inv_K + b * 16 + i * 4 + j);
-    }
-    const int oc = tid & 31, os = tid >> 5;
-    const int px = min(x0 + oc, W - 1);
-    const float* dp = p.disp.ptr + (size_t)b * (p.disp.h * p.disp.w);
-    int py[4];
-    float dv[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) py[k] = min(y0 + 4 * os + k, H - 1);
-    if (!UP) {
-#pragma unroll
-        for (int k = 0; k < 4; ++k) dv[k] = __ldg(dp + py[k] * W + px);
-    } else {
-        const UpTap txo = up_tap(px, p.disp.sw, p.disp.w);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) dv[k] = up_sample(dp, p.disp.w, up_tap(py[k], p.disp.sh, p.disp.h), txo);
-    }
-    __syncthreads();
-    Camera cam;
-#pragma unroll
-    for (int i = 0; i < 12; ++i) cam.P[i] = cams[i];
-#pragma unroll
-    for (int i = 0; i < 9; ++i) cam.iK[i] = cams[12 + i];
-    const float* sp = p.src + (size_t)b * (PK ? 4 : 3) * N;
-    Tap tp[4];
-    float gax[4], gay[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) tp[k] = pixel_tap<FASTDIV>(cam, p, px, py[k], dv[k], true, gax[k], gay[k]);
-    if (x0 + oc >= W) return;
-    const int HP = H + 4, WP = p.WP;
-    // mirror column / row of the 2-pixel border this pixel also fills (-1: none)
-    const int xp = px + 2;
-    const int mxp = px == 1 ? 1 : (px == 2 ? 0 : (px == W - 2 ? W + 2 : (px == W - 3 ? W + 3 : -1)));
-    float* pb = p.predp + (size_t)b * 3 * HP * WP;
-    float* db = p.dfac_out + (size_t)b * 3 * N + px;
-#pragma unroll
-    for (int k0 = 0; k0 < 4; k0 += 2) {
-        float tv[2][3][4];
-#pragma unroll
-        for (int j = 0; j < 2; ++j) load_taps<PK>(sp, N, W, tp[k0 + j], tv[j]);
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-            const int k = k0 + j;
-            const int y = y0 + 4 * os + k;
-            if (y >= H) continue;
-            const Gathered g = combine_taps(tv[j], tp[k], true);
-            const int yp = y + 2;
-            const int myp = y == 1 ? 1 : (y == 2 ? 0 : (y == H - 2 ? H + 2 : (y == H - 3 ? H + 3 : -1)));
-#pragma unroll
-            for (int ch = 0; ch < 3; ++ch) {
-                float* pc = pb + (size_t)ch * HP * WP;
-                pc[yp * WP + xp] = g.v[ch];
-                if (mxp >= 0) pc[yp * WP + mxp] = g.v[ch];
-                if (myp >= 0) {
-                    pc[myp * WP + xp] = g.v[ch];
-                    if (mxp >= 0) pc[myp * WP + mxp] = g.v[ch];
-                }
-                db[ch * N + y * W] = g.dix[ch] * gax[k] + g.diy[ch] * gay[k];
-            }
-        }
-    }
-}
 
 // ---------------------------------------------------------------------------
 // Identity reprojection loss (M2/trainer.py:608-615): compute_reprojection_loss of the UN-warped
@@ -774,16 +445,11 @@ namespace dmh {
 
 int photo_fast_tiles(int H, int W) { return ceil_div(W, FT_T) * ceil_div(H, FT_T); }
 
-// floats of the split design's workspace: padded warped frame + backward factors
-long long photo_split_workspace_floats(int B, int H, int W) {
-    return (long long)B * 3 * ((long long)(H + 4) * ((W + 4 + 3) & ~3) + (long long)H * W);
-}
-
 // Called by dmh_photo_scale when F == 1 and no pose gradient is requested.
 int launch_photo_fast(const float* target, const float* src, const float* T, const float* disp, int disp_h,
                       int disp_w, const float* K, const float* inv_K, const float* ident, const float* noise, int B, int H, int W, float min_depth,
                       float max_depth, int flags, float grad_scale, float* loss_partial, float* grad_disp,
-                      uint8_t* sel, float* warped, float* split_ws, const FastDhArgs* dh, cudaStream_t st) {
+                      uint8_t* sel, float* warped, const FastDhArgs* dh, cudaStream_t st) {
     FastParams p;
     p.target = target; p.src = src; p.T = T; p.K = K;
     p.disp.ptr = disp; p.disp.h = disp_h; p.disp.w = disp_w; p.disp.sh = (float)disp_h / (float)H; p.disp.sw = (float)disp_w / (float)W; p.inv_K = inv_K; p.ident = ident;
@@ -793,7 +459,6 @@ int launch_photo_fast(const float* target, const float* src, const float* T, con
     p.ds.min_disp = is_depth ? 0.f : (float)(1.0 / (double)max_depth);
     p.ds.range = is_depth ? 0.f : (float)(1.0 / (double)min_depth - 1.0 / (double)max_depth);
     p.grad_scale = grad_scale;
-    p.dfac = nullptr; p.predp = nullptr; p.dfac_out = nullptr; p.WP = 0;
     p.hint_reproj = dh ? dh->hint_reproj : nullptr; p.hint_depth = dh ? dh->hint_depth : nullptr;
     p.hint_valid = dh ? dh->hint_valid : nullptr; p.grad_hint = dh ? dh->grad_hint : nullptr;
     p.dh_nblk = dh ? dh->nblk : 0;
@@ -803,7 +468,7 @@ int launch_photo_fast(const float* target, const float* src, const float* T, con
     cudaGetDevice(&dev);
     if (!configured_dev[dev & 63]) {
         cudaError_t e = cudaSuccess;
-#define DMH_FAST_FN(T_, D_, P_, U_) (const void*)photo_fast_kernel<T_, D_, P_, U_, false>
+#define DMH_FAST_FN(T_, D_, P_, U_) (const void*)photo_fast_kernel<T_, D_, P_, U_>
 #define DMH_FAST_FN4(P_, U_) DMH_FAST_FN(false, false, P_, U_), DMH_FAST_FN(false, true, P_, U_), \
                              DMH_FAST_FN(true, false, P_, U_), DMH_FAST_FN(true, true, P_, U_)
         const void* fns[16] = {DMH_FAST_FN4(false, false), DMH_FAST_FN4(false, true), DMH_FAST_FN4(true, false),
@@ -812,10 +477,7 @@ int launch_photo_fast(const float* target, const float* src, const float* T, con
 #undef DMH_FAST_FN
         for (int i = 0; i < 16 && e == cudaSuccess; ++i)
             e = cudaFuncSetAttribute(fns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute((const void*)photo_fast_kernel<true, false, false, false, true>,
-                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-#define DMH_DH_FN(T_, D_, P_, U_) (const void*)photo_fast_kernel<T_, D_, P_, U_, false, true>
+#define DMH_DH_FN(T_, D_, P_, U_) (const void*)photo_fast_kernel<T_, D_, P_, U_, true>
 #define DMH_DH_FN4(P_, U_) DMH_DH_FN(false, false, P_, U_), DMH_DH_FN(false, true, P_, U_), \
                            DMH_DH_FN(true, false, P_, U_), DMH_DH_FN(true, true, P_, U_)
         const void* dfns[16] = {DMH_DH_FN4(false, false), DMH_DH_FN4(false, true), DMH_DH_FN4(true, false),
@@ -849,99 +511,10 @@ int launch_photo_fast(const float* target, const float* src, const float* T, con
     const bool fastdiv = W > 1 && H > 1 && const_div_exact(W - 1, &p.rcw) && const_div_exact(H - 1, &p.rch);
     const bool packed = (flags & DMH_PHOTO_SRC_PACKED) != 0;
     const bool up = !(disp_h == H && disp_w == W);
-    if (split_ws && (flags & DMH_PHOTO_PIPELINED)) {
-        // ---- persistent producer / consumer kernel; the workspace holds the backward factors (B,3,H,W)
-        if (!use_tma) {
-            set_error("dmh_photo_scale_split(pipelined): needs TMA (W %% 4 == 0, 16-byte aligned frames)");
-            return DMH_ERR_INVALID;
-        }
-        p.dfac_out = split_ws;
-        p.dfac = split_ws;
-        const size_t smem_pc = sizeof(float) * (6 * FT_NT + 6 * FT_N2 + 9 * FT_N1 + 48 + 32) + FT_N1;
-        static bool pc_cfg[64] = {false};
-        static int pc_sms[64] = {0};
-        if (!pc_cfg[dev & 63]) {
-            cudaError_t e = cudaSuccess;
-            const void* fns[8] = {(const void*)photo_pc_kernel<false, false, false>, (const void*)photo_pc_kernel<false, false, true>,
-                                  (const void*)photo_pc_kernel<false, true, false>, (const void*)photo_pc_kernel<false, true, true>,
-                                  (const void*)photo_pc_kernel<true, false, false>, (const void*)photo_pc_kernel<true, false, true>,
-                                  (const void*)photo_pc_kernel<true, true, false>, (const void*)photo_pc_kernel<true, true, true>};
-            for (int i = 0; i < 8 && e == cudaSuccess; ++i)
-                e = cudaFuncSetAttribute(fns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_pc);
-            if (e == cudaSuccess) e = cudaDeviceGetAttribute(&pc_sms[dev & 63], cudaDevAttrMultiProcessorCount, dev);
-            if (e != cudaSuccess) {
-                set_error("dmh_photo_scale_split(pipelined): configuration failed: %s", cudaGetErrorString(e));
-                return DMH_ERR_CUDA;
-            }
-            pc_cfg[dev & 63] = true;
-        }
-        const int tiles_x = ceil_div(W, FT_T), tiles_y = ceil_div(H, FT_T), ntiles = tiles_x * tiles_y * B;
-        const int nblk = ntiles < PC_CTAS * pc_sms[dev & 63] ? ntiles : PC_CTAS * pc_sms[dev & 63];
-#define DMH_PC_GO(D_, P_, U_) DMH_LAUNCH((photo_pc_kernel<D_, P_, U_>), nblk, PC_THREADS, smem_pc, st)(p, map, tiles_x, tiles_y, ntiles)
-        if (fastdiv) {
-            if (packed && up) DMH_PC_GO(true, true, true);
-            else if (packed) DMH_PC_GO(true, true, false);
-            else if (up) DMH_PC_GO(true, false, true);
-            else DMH_PC_GO(true, false, false);
-        } else {
-            if (packed && up) DMH_PC_GO(false, true, true);
-            else if (packed) DMH_PC_GO(false, true, false);
-            else if (up) DMH_PC_GO(false, false, true);
-            else DMH_PC_GO(false, false, false);
-        }
-#undef DMH_PC_GO
-        return DMH_OK;
-    }
-    if (split_ws) {
-        // ---- split design: warp_pred_kernel (warp only, no halo) + the loss kernel fed by two TMA loads
-        if (!use_tma || W < 8 || H < 8) {
-            set_error("dmh_photo_scale_split: needs TMA (W %% 4 == 0, 16-byte aligned frames) and W, H >= 8");
-            return DMH_ERR_INVALID;
-        }
-        const int HP = H + 4, WP = (W + 4 + 3) & ~3;
-        p.predp = split_ws;
-        p.WP = WP;
-        p.dfac_out = split_ws + (size_t)B * 3 * HP * WP;
-        p.dfac = p.dfac_out;
-        CUtensorMap pmap;
-        memset(&pmap, 0, sizeof(pmap));
-        {
-            const cuuint64_t gdim[4] = {(cuuint64_t)(W + 4), (cuuint64_t)HP, 3, (cuuint64_t)B};
-            const cuuint64_t gstr[3] = {(cuuint64_t)WP * 4, (cuuint64_t)WP * HP * 4, (cuuint64_t)WP * HP * 12};
-            const cuuint32_t box[4] = {FT_R2, FT_R2, 3, 1};
-            const cuuint32_t estr[4] = {1, 1, 1, 1};
-            const CUresult r = tma_encoder()(&pmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, p.predp, gdim, gstr, box, estr,
-                                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                             CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (r != CUDA_SUCCESS || (uintptr_t)split_ws % 16 != 0) {
-                set_error("dmh_photo_scale_split: tensor map of the warped frame failed (workspace must be 16-byte aligned)");
-                return DMH_ERR_INVALID;
-            }
-        }
-#define DMH_WP_GO(D_, P_, U_) DMH_LAUNCH((warp_pred_kernel<D_, P_, U_>), grid, FT_THREADS, 0, st)(p)
-        if (fastdiv) {
-            if (packed && up) DMH_WP_GO(true, true, true);
-            else if (packed) DMH_WP_GO(true, true, false);
-            else if (up) DMH_WP_GO(true, false, true);
-            else DMH_WP_GO(true, false, false);
-        } else {
-            if (packed && up) DMH_WP_GO(false, true, true);
-            else if (packed) DMH_WP_GO(false, true, false);
-            else if (up) DMH_WP_GO(false, false, true);
-            else DMH_WP_GO(false, false, false);
-        }
-#undef DMH_WP_GO
-        {
-            cudaError_t e = cudaGetLastError();
-            if (e != cudaSuccess) { set_error("dmh_photo_scale_split: warp launch failed: %s", cudaGetErrorString(e)); return DMH_ERR_CUDA; }
-        }
-        DMH_LAUNCH((photo_fast_kernel<true, false, false, false, true>), grid, FT_THREADS, smem, st)(p, map, pmap);
-        return DMH_OK;
-    }
 #define DMH_FAST_GO(T_, D_, P_, U_)                                                                           \
     do {                                                                                                      \
-        if (dh) DMH_LAUNCH((photo_fast_kernel<T_, D_, P_, U_, false, true>), grid, FT_THREADS, smem, st)(p, map, map); \
-        else DMH_LAUNCH((photo_fast_kernel<T_, D_, P_, U_, false>), grid, FT_THREADS, smem, st)(p, map, map);   \
+        if (dh) DMH_LAUNCH((photo_fast_kernel<T_, D_, P_, U_, true>), grid, FT_THREADS, smem, st)(p, map); \
+        else DMH_LAUNCH((photo_fast_kernel<T_, D_, P_, U_>), grid, FT_THREADS, smem, st)(p, map);         \
     } while (0)
 #define DMH_FAST_GO2(P_, U_)                                           \
     do {                                                               \

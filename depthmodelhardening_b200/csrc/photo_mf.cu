@@ -575,7 +575,7 @@ photo_mf_kernel(const MfParams p, const __grid_constant__ CUtensorMap tgt_map) {
         v.disp.ptr = p.sc[s].disp; v.disp.h = p.sc[s].dh; v.disp.w = p.sc[s].dw;
         v.disp.sh = p.sc[s].sh; v.disp.sw = p.sc[s].sw;
         v.ds = p.ds; v.H = H; v.W = W; v.dh_nblk = 0;
-        v.grad_scale = p.grad_scale; v.rcw = p.rcw; v.rch = p.rch; v.stream = 0;
+        v.grad_scale = p.grad_scale; v.rcw = p.rcw; v.rch = p.rch;
 
         // running first-minimum of this thread's 5 ring pixels: identities (bi, idx_i) and reprojections (br, idx_r)
         float bi[FT_ROWS], br[FT_ROWS];

@@ -480,8 +480,7 @@ int photo_fast_tiles(int H, int W);
 int launch_photo_fast(const float* target, const float* src, const float* T, const float* disp, int disp_h,
                       int disp_w, const float* K, const float* inv_K, const float* ident, const float* noise, int B, int H, int W, float min_depth,
                       float max_depth, int flags, float grad_scale, float* loss_partial, float* grad_disp,
-                      uint8_t* sel, float* warped, float* split_ws, const FastDhArgs* dh, cudaStream_t st);
-long long photo_split_workspace_floats(int B, int H, int W);
+                      uint8_t* sel, float* warped, const FastDhArgs* dh, cudaStream_t st);
 int launch_ident_bf16(const uint16_t* target, const uint16_t* src, int B, int H, int W, int no_ssim, float* out,
                       float* packed, float* tgt_f32, cudaStream_t st);
 int launch_ident_fast(const float* target, const float* const* src_host, int F, int B, int H, int W, int no_ssim,
@@ -568,7 +567,7 @@ int dmh_photo_scale_dh(const float* target, const float* const* src_host, const 
         a.hint_reproj = hint_reproj; a.hint_depth = hint_depth; a.hint_valid = hint_valid; a.grad_hint = grad_disp_hint;
         a.nblk = nblk;
         const int rc = launch_photo_fast(target, src_host[0], T_host[0], disp, disp_h, disp_w, K, inv_K, ident, noise, B, H, W,
-                                         min_depth, max_depth, flags, 1.0f, sums_partial, grad_disp, sel, nullptr, nullptr, &a,
+                                         min_depth, max_depth, flags, 1.0f, sums_partial, grad_disp, sel, nullptr, &a,
                                          (cudaStream_t)stream);
         if (rc != DMH_OK) return rc;
         DMH_CHECK_LAUNCH("dmh_photo_scale_dh(fast)");
@@ -582,25 +581,6 @@ int dmh_photo_scale_dh(const float* target, const float* const* src_host, const 
                                    min_depth, max_depth, flags | DMH_PHOTO_FORCE_GENERIC, 1.0f, sums_partial, grad_disp,
                                    grad_P_partial, sel, nullptr, stream);
     g_dh_next.armed = false;
-    return rc;
-}
-
-// workspace handed from dmh_photo_scale_split to the shared launcher below (same thread, same call)
-static thread_local float* g_split_ws = nullptr;
-
-long long dmh_photo_split_workspace_floats(int B, int H, int W) { return photo_split_workspace_floats(B, H, W); }
-
-int dmh_photo_scale_split(const float* target, const float* src, const float* T, const float* disp, int disp_h, int disp_w,
-                          const float* K, const float* inv_K, const float* ident, const float* noise, int B, int H, int W,
-                          float min_depth, float max_depth, int flags, float grad_scale, float* workspace,
-                          float* loss_partial, float* grad_disp, uint8_t* sel, dmh_stream_t stream) {
-    DMH_REQUIRE(workspace, "dmh_photo_scale_split: null workspace");
-    const float* srcs[1] = {src};
-    const float* Ts[1] = {T};
-    g_split_ws = workspace;
-    const int rc = dmh_photo_scale(target, srcs, Ts, 1, disp, disp_h, disp_w, K, inv_K, ident, noise, B, H, W, min_depth,
-                                   max_depth, flags, grad_scale, loss_partial, grad_disp, nullptr, sel, nullptr, stream);
-    g_split_ws = nullptr;
     return rc;
 }
 
@@ -624,7 +604,6 @@ int dmh_photo_scale(const float* target, const float* const* src_host, const flo
     DMH_REQUIRE(!(flags & DMH_PHOTO_SRC_PACKED) || fast_ok,
                 "dmh_photo_scale: DMH_PHOTO_SRC_PACKED needs the single-source fast path (F == 1, SSIM on, disparity "
                 "input, no pose gradient, no warped output)");
-    DMH_REQUIRE(!g_split_ws || fast_ok, "dmh_photo_scale_split: needs the single-source fast path");
     if (fast_ok) {
         // single source frame, no pose gradient: the 32x32-tile fast kernel (photo_fast.cu).  It writes
         // fewer partial sums than dmh_photo_tiles() promises; zero the tail so the caller's reduction is exact.
@@ -637,7 +616,7 @@ int dmh_photo_scale(const float* target, const float* const* src_host, const flo
         }
         const int rc = launch_photo_fast(target, src_host[0], T_host[0], disp, disp_h, disp_w, K, inv_K, ident, noise, B, H, W, min_depth,
                                          max_depth, flags, grad_scale, loss_partial, grad_disp, sel,
-                                         warped_host ? warped_host[0] : nullptr, g_split_ws, nullptr, (cudaStream_t)stream);
+                                         warped_host ? warped_host[0] : nullptr, nullptr, (cudaStream_t)stream);
         if (rc != DMH_OK) return rc;
         DMH_CHECK_LAUNCH("dmh_photo_scale(fast)");
         return DMH_OK;

@@ -70,10 +70,6 @@ struct FastParams {
     float* grad_disp;
     uint8_t* sel;
     float* warped;               // (unused by the fast kernel; kept for the launcher)
-    const float* dfac;           // SPLIT: (B,3,H,W) d(pred)/d(disp) factors from warp_pred_kernel
-    float* predp;                // warp_pred_kernel output: (B,3,H+4,WP) warped frame, image pixel (x,y) at (x+2,y+2)
-    float* dfac_out;             // warp_pred_kernel output
-    int WP;                      // row pitch of predp (multiple of 4 floats)
     // depth-hints objective (DH/trainer.py:541-590, 666-713), DH instantiation only
     const float* hint_reproj;    // (B,1,H,W) hint reprojection loss + 1000*(1-valid); NULL: no hints
     const float* hint_depth;     // (B,1,H,W)

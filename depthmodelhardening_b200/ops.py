@@ -363,7 +363,6 @@ FLAG_NO_SSIM = 1
 FLAG_AVG_REPROJECTION = 2
 FLAG_INPUT_IS_DEPTH = 4
 FLAG_SRC_PACKED = 16
-FLAG_PIPELINED = 32
 
 
 class _PhotoScale(torch.autograd.Function):
@@ -432,37 +431,14 @@ import ctypes as _C
 import os as _os
 
 _SIDE_STREAMS = {}
-# single-source objective: the one fused kernel per scale (default) or the two-kernel form -- warp kernel without
-# halo + TMA-fed loss kernel, bit-identical results.  Measured on B200 at config 2 (profiles/r01_ncu_split.txt):
-# 142 + 261 us per scale against 369-393 us fused (the halo recomputation the split saves is paid back in
-# stores / loads of the warped frame and a loss kernel that starts on a cold TMA wait), so the default stays fused.
-SPLIT_PATH = _os.environ.get("DMH_SPLIT", "0") in ("1", "2")
-# DMH_SPLIT=2: the persistent producer / consumer kernel (one launch per scale, warp of tile i+1 beside SSIM of tile i;
-# bit-identical, measured 520-550 us per scale -- 16 warps per SM issue less than the fused kernel's 24)
-PIPELINED = _os.environ.get("DMH_SPLIT", "0") == "2"
 # all scales of the single-source objective in one launch (csrc/photo_ms.cu, bit-identical to the per-scale launches);
 # DMH_MULTISCALE=0 keeps one launch per scale
 MULTISCALE = _os.environ.get("DMH_MULTISCALE", "1") != "0"
 # several source frames and / or pose gradients: all sources and all scales in one launch of the tile kernel
 # (csrc/photo_mf.cu); DMH_MULTISOURCE=0 keeps the general per-scale kernel (csrc/photo_objective.cu)
 MULTISOURCE = _os.environ.get("DMH_MULTISOURCE", "1") != "0"
-# development switch: the single-source objective through the multi-source kernel's persistent (tile, scale) item loop
-# (same bits as dmh_photo_multiscale; measured slower / faster: DESIGN.md section 7)
-SINGLE_VIA_MF = _os.environ.get("DMH_SINGLE_VIA_MF", "0") == "1"
-# glue steps of all scales in one launch (csrc/objective_fused.cu; identical outputs) -- built, measured, NOT the default:
-#   DMH_SMOOTH_MULTI=1   dmh_smooth_fused_multi: 2 launches instead of 2 S
-#   DMH_DGRAD_MULTI=1    dmh_disp_grad_multi: 1 launch instead of S
-# On B200 (profiles/r02_kernel_ab.txt, blocks r3a-r3c) the merged launches are shorter in summed kernel time (smoothness
-# 112 vs 140 us at 32 items, 16 vs 45 us at 4) but the STEP is not faster: the per-scale launches run as independent
-# branches (streams / graph nodes) beside the photometric kernel, one merged launch is one serial node -- step 1.845 vs
-# 1.835 ms at 32 items, 0.276 vs 0.267 ms at 4 items per GPU; the merged backward is 30 us slower at 32 items.
-SMOOTH_MULTI = _os.environ.get("DMH_SMOOTH_MULTI", "0") != "0"
-DGRAD_MULTI = _os.environ.get("DMH_DGRAD_MULTI", "0") != "0"
-# (spreading the per-scale glue launches over 2 / 4 side streams instead of 1 + 2 was measured too: no change at 32
-# items, within the +-1.5 % run-to-run noise at 4 items per GPU -- not kept)
-
-
-_SMOOTH_PRIORITY = int(_os.environ.get("DMH_SMOOTH_PRIORITY", "-1"))    # development switch
+# The glue steps stay one launch per scale: those launches run as independent branches (streams / graph nodes) beside
+# the photometric kernel.  All-scales launches were measured on B200 and were no faster per step (DESIGN.md section 4).
 
 
 def _side_stream(dev, which=0):
@@ -471,7 +447,7 @@ def _side_stream(dev, which=0):
     key = (idx, which)
     st = _SIDE_STREAMS.get(key)
     if st is None:
-        st = _SIDE_STREAMS[key] = torch.cuda.Stream(device=idx, priority=_SMOOTH_PRIORITY if which == 0 else 0)
+        st = _SIDE_STREAMS[key] = torch.cuda.Stream(device=idx, priority=-1 if which == 0 else 0)
     return st
 
 
@@ -511,7 +487,7 @@ class _Objective(torch.autograd.Function):
         need_T = any(ctx.needs_input_grad[base + i] for i in range(n_src))
         # single source, no pose gradient: the per-scale kernel gathers from a pixel-packed (B,H,W,4) copy of the
         # source (one 128-bit load per bilinear tap), written once by the identity-loss kernel
-        packed = n_src == 1 and not need_T and not no_ssim and H * W < (1 << 28) and not (SINGLE_VIA_MF and not bf16_frames)
+        packed = n_src == 1 and not need_T and not no_ssim and H * W < (1 << 28)
         if bf16_frames and not (packed and target.data_ptr() % 16 == 0 and srcs[0].data_ptr() % 16 == 0):
             bf16_frames = False                             # general kernels: widen first
             target = colors[0] = f32c(target)
@@ -543,7 +519,6 @@ class _Objective(torch.autograd.Function):
         elif automask:
             check(lib.dmh_identity_loss(ptr(target), src_arr, n_src, B, H, W, no_ssim, ptr(ident), stream()),
                   "identity_loss")
-        split = packed and SPLIT_PATH and W % 4 == 0 and W >= 8 and H >= 8 and target.data_ptr() % 16 == 0
         tiles = lib.dmh_photo_tiles(H, W)
         G, gN, wss, parts, gPs, sels = [], [], [], [], [], []
         T_arr = ptr_array(Ts)
@@ -559,19 +534,13 @@ class _Objective(torch.autograd.Function):
             gN.append(torch.empty(B, 1, h, w, device=dev, dtype=torch.float32))
         side.wait_stream(cur)
         with torch.cuda.stream(side):
-            if SMOOTH_MULTI and S <= 8 and all(c.shape[1] == 3 for c in colors[:S]):
-                check(lib.dmh_smooth_fused_multi(S, ptr_array(disps), ptr_array(colors[:S]), B,
-                                                 (_C.c_int * S)(*[d.shape[2] for d in disps]),
-                                                 (_C.c_int * S)(*[d.shape[3] for d in disps]), ptr_array(wss),
-                                                 ptr_array(gN), stream()), "smooth_fused_multi")
-            else:
-                for s in range(S):
-                    d = disps[s]
-                    check(lib.dmh_smooth_fused(ptr(d), ptr(colors[s]), B, 3, d.shape[2], d.shape[3], ptr(wss[s]),
-                                               ptr(gN[s]), stream()), "smooth_fused")
+            for s in range(S):
+                d = disps[s]
+                check(lib.dmh_smooth_fused(ptr(d), ptr(colors[s]), B, 3, d.shape[2], d.shape[3], ptr(wss[s]),
+                                           ptr(gN[s]), stream()), "smooth_fused")
         # the per-scale launches are independent of each other: odd scales go to a second stream so that the
         # tail of one launch (10240 CTAs = 23.06 waves of 444) overlaps the head of the next
-        multiscale = (packed and MULTISCALE and not split and S <= 4 and W % 4 == 0 and target.data_ptr() % 16 == 0
+        multiscale = (packed and MULTISCALE and S <= 4 and W % 4 == 0 and target.data_ptr() % 16 == 0
                       and H * W < (1 << 27))
         if multisrc:
             tiles32 = ((H + 31) // 32) * ((W + 31) // 32)
@@ -618,21 +587,9 @@ class _Objective(torch.autograd.Function):
             sel = torch.empty(B, H, W, device=dev, dtype=torch.uint8) if want_sel else None
             with torch.cuda.stream(alt if (s & 1) else cur):
                 with _timed("photo_scale"):
-                    if split:
-                        # warp kernel (every pixel gathered once) + TMA-fed loss kernel; same bits as the fused kernel
-                        ws_split = torch.empty(lib.dmh_photo_split_workspace_floats(B, H, W), device=dev,
-                                               dtype=torch.float32)
-                        check(lib.dmh_photo_scale_split(ptr(target), ptr(src_pk), ptr(Ts[0]), ptr(d), h, w, ptr(k), ptr(ik),
-                                                        ptr(ident), ptr(noises[s]), B, H, W, min_depth, max_depth,
-                                                        flags | (FLAG_PIPELINED if PIPELINED else 0),
-                                                        inv_den, ptr(ws_split), ptr(part), ptr(g_full), ptr(sel), stream()),
-                                  "photo_scale_split")
-                        if s & 1:
-                            ws_split.record_stream(alt)
-                    else:
-                        check(lib.dmh_photo_scale(ptr(target), src_arr, T_arr, n_src, ptr(d), h, w, ptr(k), ptr(ik),
-                                                  ptr(ident), ptr(noises[s]), B, H, W, min_depth, max_depth, flags, inv_den,
-                                                  ptr(part), ptr(g_full), ptr(gP), ptr(sel), None, stream()), "photo_scale")
+                    check(lib.dmh_photo_scale(ptr(target), src_arr, T_arr, n_src, ptr(d), h, w, ptr(k), ptr(ik),
+                                              ptr(ident), ptr(noises[s]), B, H, W, min_depth, max_depth, flags, inv_den,
+                                              ptr(part), ptr(g_full), ptr(gP), ptr(sel), None, stream()), "photo_scale")
             G.append(g_full); parts.append(part); gPs.append(gP); sels.append(sel)
         cur.wait_stream(alt)
         cur.wait_stream(side)
@@ -676,32 +633,19 @@ class _Objective(torch.autograd.Function):
         dev = G[0].device
         cur, alt = torch.cuda.current_stream(dev), _side_stream(dev, 1)
         want = [bool(ctx.needs_input_grad[base + n_src + s]) for s in range(S)]
-        if DGRAD_MULTI and all(want) and S <= 8:
-            # one launch for all scales; falls through to the per-scale launches when a scale needs the generic kernel
-            gds = [torch.empty(B, 1, dshapes[s][2], dshapes[s][3], device=dev, dtype=torch.float32) for s in range(S)]
-            rc = lib.dmh_disp_grad_multi(S, ptr_array(list(G)), ptr_array(list(gN)),
-                                         ptr_array([img_scalars[s] for s in range(S)]), (_C.c_float * S)(*smooth_w),
-                                         ptr(gt), ptr_array([gs[s:s + 1] for s in range(S)]) if gs is not None else None,
-                                         None, 1.0 / S, B, (_C.c_int * S)(*[sh_[2] for sh_ in dshapes]),
-                                         (_C.c_int * S)(*[sh_[3] for sh_ in dshapes]), H, W, ptr_array(gds), stream())
-            if rc == 0:
-                grads_disp = [gds[s].view(dshapes[s]) for s in range(S)]
-            elif rc != _lib.ERR_UNSUPPORTED:
-                check(rc, "disp_grad_multi")
-        if not grads_disp:
-            alt.wait_stream(cur)
-            for s in range(S):
-                if not want[s]:
-                    grads_disp.append(None)
-                    continue
-                _, _, h, w = dshapes[s]
-                gd = torch.empty(B, 1, h, w, device=dev, dtype=torch.float32)
-                with torch.cuda.stream(alt if (s & 1) else cur):
-                    check(lib.dmh_disp_grad(ptr(G[s]), ptr(gN[s]), ptr(img_scalars[s]), smooth_w[s], ptr(gt),
-                                            ptr(gs[s:s + 1]) if gs is not None else None, None, 1.0 / S, B, h, w, H, W,
-                                            ptr(gd), stream()), "disp_grad")
-                grads_disp.append(gd.view(dshapes[s]))
-            cur.wait_stream(alt)
+        alt.wait_stream(cur)
+        for s in range(S):
+            if not want[s]:
+                grads_disp.append(None)
+                continue
+            _, _, h, w = dshapes[s]
+            gd = torch.empty(B, 1, h, w, device=dev, dtype=torch.float32)
+            with torch.cuda.stream(alt if (s & 1) else cur):
+                check(lib.dmh_disp_grad(ptr(G[s]), ptr(gN[s]), ptr(img_scalars[s]), smooth_w[s], ptr(gt),
+                                        ptr(gs[s:s + 1]) if gs is not None else None, None, 1.0 / S, B, h, w, H, W,
+                                        ptr(gd), stream()), "disp_grad")
+            grads_disp.append(gd.view(dshapes[s]))
+        cur.wait_stream(alt)
         g_T = [None] * n_src
         if need_T and ctx.gp_stacked:
             # multi-source kernel: sum over tiles and weighted sum over scales in one contraction, then the 4x4

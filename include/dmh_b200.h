@@ -168,7 +168,6 @@ int dmh_identity_loss_pack_bf16(const uint16_t* target_bf16, const uint16_t* src
 #define DMH_PHOTO_INPUT_IS_DEPTH 4
 #define DMH_PHOTO_FORCE_GENERIC 8 /* testing: never take the single-source fast kernel */
 #define DMH_PHOTO_SRC_PACKED 16 /* src_host[0] is the (B,H,W,4) layout of dmh_identity_loss_pack; F == 1, no pose grad */
-#define DMH_PHOTO_PIPELINED 32 /* dmh_photo_scale_split: one persistent producer / consumer kernel instead of two kernels */
 #define DMH_PHOTO_MAX_FRAMES 4
 int dmh_photo_tiles(int H, int W);           /* CTAs per batch item */
 int dmh_photo_scale(const float* target, const float* const* src_host, const float* const* T_host, int F,
@@ -176,18 +175,6 @@ int dmh_photo_scale(const float* target, const float* const* src_host, const flo
                     const float* noise, int B, int H, int W, float min_depth, float max_depth, int flags, float grad_scale,
                     float* loss_partial, float* grad_disp, float* grad_P_partial, uint8_t* sel,
                     float* const* warped_host, dmh_stream_t stream);
-
-/* Split form of the single-source fast path of dmh_photo_scale (F == 1, SSIM on, disparity input, no pose gradient):
- * kernel 1 warps the source frame once per pixel (no halo recomputation) into `workspace` -- the warped frame with a
- * 2-pixel reflect border plus the collapsed backward factors d(pred)/d(disp) -- kernel 2 stages the target and the
- * warped tile through shared memory by TMA and does SSIM + L1, the automask decision and the backward.  Results are
- * bit-identical to dmh_photo_scale.  workspace: dmh_photo_split_workspace_floats(B,H,W) floats, 16-byte aligned.
- * Needs W % 4 == 0, 16-byte aligned frames, W, H >= 8.  flags: DMH_PHOTO_SRC_PACKED allowed (src = packed copy).  */
-long long dmh_photo_split_workspace_floats(int B, int H, int W);
-int dmh_photo_scale_split(const float* target, const float* src, const float* T, const float* disp, int disp_h, int disp_w,
-                          const float* K, const float* inv_K, const float* ident, const float* noise, int B, int H, int W,
-                          float min_depth, float max_depth, int flags, float grad_scale, float* workspace,
-                          float* loss_partial, float* grad_disp, uint8_t* sel, dmh_stream_t stream);
 
 /* ALL scales of the single-source objective in one launch (DepthNetworks/monodepth2/trainer.py:476-523 and
  * :589-660 -- the `for scale in self.opt.scales` loops of generate_images_pred and compute_losses run inside the
@@ -276,18 +263,6 @@ int dmh_objective_finish(int S, int B, const float* const* smooth_ws_host, const
 int dmh_disp_grad(const float* G_full, const float* gN, const float* img_scalars, float smooth_weight,
                   const float* g_total, const float* g_scale, const float* g_smooth, float inv_S, int B, int h, int w,
                   int H, int W, float* grad_disp, dmh_stream_t stream);
-/* All-scales forms of the two glue steps (the `for scale in self.opt.scales` loop of M2/trainer.py:589-674 inside the
- * launch): dmh_smooth_fused_multi = dmh_smooth_fused of S scales in two launches (3-channel images);
- * dmh_disp_grad_multi = dmh_disp_grad of S scales in one launch (u_s = *g_total * inv_S + *g_scale_host[s]).
- * *_host arrays are host arrays of length S.  Outputs identical to the per-scale entry points.
- * dmh_disp_grad_multi returns DMH_ERR_UNSUPPORTED, with nothing launched, when a scale needs dmh_disp_grad's generic
- * kernel (non-integer factor, factor outside {1,2,4,8}, unaligned rows).                                            */
-int dmh_smooth_fused_multi(int S, const float* const* disp_host, const float* const* img_host, int B, const int* h_host,
-                           const int* w_host, float* const* ws_host, float* const* gN_host, dmh_stream_t stream);
-int dmh_disp_grad_multi(int S, const float* const* G_full_host, const float* const* gN_host,
-                        const float* const* img_scalars_host, const float* smooth_weight_host, const float* g_total,
-                        const float* const* g_scale_host, const float* g_smooth, float inv_S, int B, const int* h_host,
-                        const int* w_host, int H, int W, float* const* grad_disp_host, dmh_stream_t stream);
 
 /* ======================= stage 1: physical patch attack ======================= */
 

@@ -1,9 +1,9 @@
 #!/usr/bin/env python
-"""Same-box A/B of development switches: prints one JSON line with the stage-2 time (CUDA events), the whole step as a
+"""Same-box A/B of environment settings: prints one JSON line with the stage-2 time (CUDA events), the whole step as a
 two-stream CUDA-graph replay at per-GPU batch 32 (the bench headline) and at batch 4 (the shard of an 8-GPU
-strong-scaling run, no collective).  The switches are environment variables read by the library / bench.py
-(DMH_MS_PAIR, DMH_GLUE_MULTI, DMH_S1_PRIORITY, ...): run once per setting, e.g.
-    for p in 0 3 4 5; do DMH_MS_PAIR=$p python profiles/ab.py; done"""
+strong-scaling run, no collective).  The settings are environment variables read by the library / bench.py
+(DMH_MULTISCALE, DMH_MULTISOURCE, DMH_S1_PRIORITY): run once per setting, e.g.
+    for p in 0 1; do DMH_MULTISCALE=$p python profiles/ab.py; done"""
 import json
 import os
 import sys

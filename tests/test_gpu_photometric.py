@@ -505,54 +505,6 @@ def test_packed_source_gather_is_bit_identical(dev, hw, dhw):
     assert float(outs[0][1].abs().max()) > 0
 
 
-@pytest.mark.parametrize("hw,dhw", [((64, 96), (64, 96)), ((40, 72), (40, 72)), ((96, 160), (24, 40)), ((72, 200), (36, 100))])
-def test_split_path_is_bit_identical_to_fused(dev, hw, dhw):
-    """dmh_photo_scale_split (warp kernel without halo + TMA-fed loss kernel) against the fused single-source kernel:
-    loss partial sums, disparity gradient and argmin must agree bit for bit, incl. ragged tiles and up-sampled
-    disparities (W % 4 == 0: the split path needs TMA)."""
-    from depthmodelhardening_b200 import _lib, ops
-    from depthmodelhardening_b200._lib import check, ptr, ptr_array, stream
-    H, W = hw
-    h, w = dhw
-    B = 2
-    pb = synth.photo_batch(batch=B, height=H, width=W, frame_ids=(0, "s"), scales=(0,), seed=73).to(dev)
-    lib = _lib.load()
-    target, src = pb.color[(0, 0)].contiguous(), pb.color[("s", 0)].contiguous()
-    gen = torch.Generator().manual_seed(6)
-    disp = (0.05 + 0.4 * torch.rand(B, 1, h, w, generator=gen)).to(dev)
-    ident = torch.empty(B, 1, H, W, device=dev)
-    pk = torch.empty(B, H, W, 4, device=dev)
-    check(lib.dmh_identity_loss_pack(ptr(target), ptr(src), B, H, W, 0, ptr(ident), ptr(pk), stream()))
-    tiles = lib.dmh_photo_tiles(H, W)
-    K, iK, T = pb.K.contiguous(), pb.inv_K.contiguous(), pb.T["s"].contiguous()
-    nz = pb.noise[0][:, :1].contiguous()
-    outs = []
-    for split in (0, 1, 2):            # fused kernel; two kernels; persistent producer / consumer kernel
-        part = torch.zeros(B * tiles, device=dev)
-        g = torch.empty(B, 1, H, W, device=dev)
-        sel = torch.empty(B, H, W, device=dev, dtype=torch.uint8)
-        if split:
-            ws = torch.full((lib.dmh_photo_split_workspace_floats(B, H, W),), float("nan"), device=dev)
-            fl = ops.FLAG_SRC_PACKED | (ops.FLAG_PIPELINED if split == 2 else 0)
-            check(lib.dmh_photo_scale_split(ptr(target), ptr(pk), ptr(T), ptr(disp), h, w, ptr(K), ptr(iK), ptr(ident),
-                                            ptr(nz), B, H, W, 0.1, 100.0, fl, 1.0, ptr(ws), ptr(part),
-                                            ptr(g), ptr(sel), stream()), "photo_scale_split")
-        else:
-            check(lib.dmh_photo_scale(ptr(target), ptr_array([pk]), ptr_array([T]), 1, ptr(disp), h, w, ptr(K), ptr(iK),
-                                      ptr(ident), ptr(nz), B, H, W, 0.1, 100.0, ops.FLAG_SRC_PACKED, 1.0, ptr(part), ptr(g),
-                                      None, ptr(sel), None, stream()), "photo_scale")
-        outs.append((part, g, sel))
-    torch.cuda.synchronize()
-    nfast = B * ((H + 31) // 32) * ((W + 31) // 32)                # tiles of the 32 x 32 kernels (partials beyond: zero)
-    for alt in outs[1:]:
-        for i, (a, b_) in enumerate(zip(outs[0], alt)):
-            assert torch.isfinite(b_.float()).all()
-            if i == 0:     # per-tile loss sums: same pixels, the block reduction adds them in a different order
-                assert torch.allclose(a[:nfast], b_[:nfast], rtol=2e-6, atol=0.0)
-            else:
-                assert torch.equal(a, b_)
-
-
 # ----------------------------------------------------------------------------- all scales in one launch (photo_ms.cu)
 def _per_scale_vs_multiscale(dev, H, W, dsizes, B=2, seed=81, disp_fn=None, T=None, noise=True, automask=True):
     """S calls of dmh_photo_scale (packed source) against ONE dmh_photo_multiscale call on the same buffers."""
@@ -608,7 +560,7 @@ def _assert_same_bits(ref, got):
 
 @pytest.mark.parametrize("hw", [(64, 96), (40, 72), (96, 160), (72, 200), (192, 640)])
 def test_multiscale_kernel_is_bit_identical_to_per_scale(dev, hw):
-    """dmh_photo_multiscale (all scales in one launch, cp.async tap pipeline, branch-free exact reciprocals) against S
+    """dmh_photo_multiscale (all scales in one launch, register tap pipeline, branch-free exact reciprocals) against S
     launches of the per-scale kernel: loss partial sums, disparity gradients and argmin agree BIT FOR BIT, incl.
     ragged tiles, every up-sampling factor of the 4-scale pyramid and a non-integer factor."""
     H, W = hw
@@ -690,102 +642,6 @@ def test_objective_multiscale_switch_is_bit_identical(dev):
     assert torch.equal(res[0][0], res[1][0])
     for a, b_ in zip(res[0][1], res[1][1]):
         assert torch.equal(a, b_)
-
-
-# ---- glue steps of all scales in one launch each (csrc/objective_fused.cu: dmh_smooth_fused_multi, dmh_disp_grad_multi)
-@pytest.mark.parametrize("hw,B", [((320, 1024), 2), ((96, 160), 3), ((64, 96), 1)])
-def test_glue_multi_launches_are_bit_identical_to_per_scale(dev, hw, B):
-    """dmh_smooth_fused_multi (2 launches for S scales) and dmh_disp_grad_multi (1 launch) against S calls of
-    dmh_smooth_fused / dmh_disp_grad on the same buffers: workspaces (mean and block partial sums), gN and the final
-    disparity gradients agree BIT FOR BIT; a scale that needs the generic up-sampling kernel is refused untouched."""
-    import ctypes as C
-    from depthmodelhardening_b200 import _lib
-    from depthmodelhardening_b200._lib import check, ptr, ptr_array, stream
-    lib = _lib.load()
-    H, W = hw
-    S = 4
-    gen = torch.Generator().manual_seed(97)
-    sizes = [(H >> s, W >> s) for s in range(S)]
-    disps = [(0.05 + 0.4 * torch.rand(B, 1, h, w, generator=gen)).to(dev) for h, w in sizes]
-    imgs = [torch.rand(B, 3, h, w, generator=gen).to(dev) for h, w in sizes]
-    hs = (C.c_int * S)(*[h for h, _ in sizes])
-    ws_ = (C.c_int * S)(*[w for _, w in sizes])
-
-    def bufs():
-        return ([torch.full((lib.dmh_smooth_fused_workspace_floats(B, h, w),), float("nan"), device=dev) for h, w in sizes],
-                [torch.full((B, 1, h, w), float("nan"), device=dev) for h, w in sizes])
-    ws_a, gN_a = bufs()
-    for s, (h, w) in enumerate(sizes):
-        check(lib.dmh_smooth_fused(ptr(disps[s]), ptr(imgs[s]), B, 3, h, w, ptr(ws_a[s]), ptr(gN_a[s]), stream()))
-    ws_b, gN_b = bufs()
-    n0 = lib.dmh_launch_count()
-    check(lib.dmh_smooth_fused_multi(S, ptr_array(disps), ptr_array(imgs), B, hs, ws_, ptr_array(ws_b), ptr_array(gN_b),
-                                     stream()), "smooth_fused_multi")
-    assert lib.dmh_launch_count() - n0 == 2
-    torch.cuda.synchronize()
-    for s in range(S):
-        assert torch.isfinite(ws_b[s]).all() and torch.isfinite(gN_b[s]).all()
-        assert torch.equal(ws_a[s].view(torch.int32), ws_b[s].view(torch.int32)), "scale %d: partial sums differ" % s
-        assert torch.equal(gN_a[s].view(torch.int32), gN_b[s].view(torch.int32)), "scale %d: gN differs" % s
-    assert float(gN_b[0].abs().max()) > 0
-
-    # backward: full-resolution gradients of every scale -> (h, w), normalisation backward, upstream scalars
-    G = [torch.randn(B, 1, H, W, generator=gen).to(dev) for _ in range(S)]
-    img_scalars = (0.5 + torch.rand(S, B, 2, generator=gen)).to(dev)
-    g_total = torch.tensor([0.7], device=dev)
-    g_scales = torch.tensor([0.1, -0.2, 0.3, 0.05], device=dev)
-    smooth_w = [1e-3 / (2 ** s) for s in range(S)]
-    for use_scale in (True, False):
-        out_a = [torch.full((B, 1, h, w), float("nan"), device=dev) for h, w in sizes]
-        for s, (h, w) in enumerate(sizes):
-            check(lib.dmh_disp_grad(ptr(G[s]), ptr(gN_a[s]), ptr(img_scalars[s]), smooth_w[s], ptr(g_total),
-                                    ptr(g_scales[s:s + 1]) if use_scale else None, None, 1.0 / S, B, h, w, H, W,
-                                    ptr(out_a[s]), stream()), "disp_grad")
-        out_b = [torch.full((B, 1, h, w), float("nan"), device=dev) for h, w in sizes]
-        n0 = lib.dmh_launch_count()
-        check(lib.dmh_disp_grad_multi(S, ptr_array(G), ptr_array(gN_a), ptr_array([img_scalars[s] for s in range(S)]),
-                                      (C.c_float * S)(*smooth_w), ptr(g_total),
-                                      ptr_array([g_scales[s:s + 1] for s in range(S)]) if use_scale else None, None,
-                                      1.0 / S, B, hs, ws_, H, W, ptr_array(out_b), stream()), "disp_grad_multi")
-        assert lib.dmh_launch_count() - n0 == 1
-        torch.cuda.synchronize()
-        for s in range(S):
-            assert torch.isfinite(out_b[s]).all()
-            assert torch.equal(out_a[s].view(torch.int32), out_b[s].view(torch.int32)), "scale %d: gradients differ" % s
-    # a non-integer factor needs dmh_disp_grad's generic kernel: refused, nothing written
-    h2, w2 = H // 2 + 3, W // 2 + 5
-    untouched = torch.full((B, 1, h2, w2), float("nan"), device=dev)
-    rc = lib.dmh_disp_grad_multi(1, ptr_array([G[0]]), None, None, (C.c_float * 1)(0.0), ptr(g_total), None, None, 1.0, B,
-                                 (C.c_int * 1)(h2), (C.c_int * 1)(w2), H, W, ptr_array([untouched]), stream())
-    torch.cuda.synchronize()
-    assert rc == _lib.ERR_UNSUPPORTED and torch.isnan(untouched).all()
-
-
-@pytest.mark.parametrize("shape", [(2, 96, 160), (2, 320, 1024), (2, 50, 70)])
-def test_objective_glue_switch_is_bit_identical(dev, shape):
-    """ops.objective with the all-scales glue launches (DMH_SMOOTH_MULTI / DMH_DGRAD_MULTI) against the per-scale
-    launches: identical losses and disparity gradients through the public autograd path (the 50 x 70 case falls back
-    to per-scale backward launches)."""
-    from depthmodelhardening_b200 import objective, ops
-    B, H, W = shape
-    scales = (0, 1, 2, 3) if H % 8 == 0 and W % 8 == 0 else (0, 1)
-    g = synth.photo_batch(batch=B, height=H, width=W, frame_ids=(0, "s"), scales=scales, seed=95).to(dev)
-    res = []
-    for multi in (True, False):
-        old = (ops.SMOOTH_MULTI, ops.DGRAD_MULTI)
-        ops.SMOOTH_MULTI = ops.DGRAD_MULTI = multi
-        try:
-            disps = {s: g.disp[s].clone().requires_grad_(True) for s in g.scales}
-            losses, _ = objective.photometric_losses(g.color, disps, g.K, g.inv_K, g.T, g.frame_ids, g.scales, g.height,
-                                                     g.width, noise=g.noise)
-            losses["loss"].backward()
-            res.append((losses["loss"].detach().clone(), [disps[s].grad.clone() for s in g.scales]))
-        finally:
-            ops.SMOOTH_MULTI, ops.DGRAD_MULTI = old
-    torch.cuda.synchronize()
-    assert torch.equal(res[0][0], res[1][0])
-    for a, b_ in zip(res[0][1], res[1][1]):
-        assert torch.equal(a, b_) and torch.isfinite(a).all()
 
 
 # ---- the multi-source tile kernel (csrc/photo_mf.cu, dmh_photo_multisource)

@@ -142,3 +142,64 @@ def test_install_rebinds_every_patch_attack_class():
         dmh.uninstall()
     for m, c in names.items():
         assert getattr(mods[m], c) is originals[m], m
+
+
+# ---- stage 1: the span table of the patch kernels (csrc/patch.cu aa_table_kernel / aa_span3) against the per-pixel
+# weight function the backward used before (aa_weight_of), restated op by op in IEEE float32
+f32 = np.float32
+
+
+def _aa_filter(x):
+    x = abs(x)
+    return f32(1.0) - x if x < f32(1.0) else f32(0.0)
+
+
+def _span3(i, in_size, scale):
+    """aa_span3: (lo, w0, w1, w2) of output index i."""
+    support = scale if scale >= f32(1.0) else f32(1.0)
+    invscale = f32(1.0) / scale if scale >= f32(1.0) else f32(1.0)
+    center = f32(scale * f32(f32(i) + f32(0.5)))
+    lo = max(int(f32(f32(center - support) + f32(0.5))), 0)
+    n = min(min(int(f32(f32(center + support) + f32(0.5))), in_size) - lo, 3)
+    w, total = [], f32(0.0)
+    for j in range(3):
+        wj = _aa_filter(f32(f32(f32(f32(j) + f32(f32(lo) - center)) + f32(0.5)) * invscale)) if j < n else f32(0.0)
+        w.append(wj)
+        total = f32(total + wj)
+    if total != 0:
+        w = [f32(x / total) for x in w]
+    return lo, w
+
+
+def _weight_of(o, in_size, scale, ci, maxt=8):
+    """aa_weight_of: weight with which output index o reads input index ci."""
+    support = scale if scale >= f32(1.0) else f32(1.0)
+    invscale = f32(1.0) / scale if scale >= f32(1.0) else f32(1.0)
+    center = f32(scale * f32(f32(o) + f32(0.5)))
+    lo = max(int(f32(f32(center - support) + f32(0.5))), 0)
+    n = min(min(int(f32(f32(center + support) + f32(0.5))), in_size) - lo, maxt)
+    if ci < lo or ci >= lo + n:
+        return f32(0.0)
+    total, mine = f32(0.0), f32(0.0)
+    for j in range(n):
+        w = _aa_filter(f32(f32(f32(f32(j) + f32(f32(lo) - center)) + f32(0.5)) * invscale))
+        total = f32(total + w)
+        if lo + j == ci:
+            mine = w
+    return f32(mine / total) if total != 0 else mine
+
+
+@pytest.mark.parametrize("in_size,out_size", [(1242, 1024), (375, 320), (100, 81), (64, 64), (97, 70)])
+def test_span_table_equals_the_per_pixel_weight_function(in_size, out_size):
+    """Every (output index, input index) pair: the table entry the patch kernels read == aa_weight_of, bit for bit, for
+    scale factors below 1.5 (3-tap spans); the weights of a span sum to 1 within rounding."""
+    scale = f32(f32(in_size) / f32(out_size))
+    assert scale < 1.5
+    for o in range(out_size):
+        lo, w = _span3(o, in_size, scale)
+        assert abs(float(sum(w, f32(0.0))) - 1.0) < 1e-6
+        for ci in range(max(lo - 2, 0), min(lo + 5, in_size)):
+            d = ci - lo
+            tab = w[d] if 0 <= d < 3 else f32(0.0)
+            ref = _weight_of(o, in_size, scale, ci)
+            assert tab.tobytes() == ref.tobytes(), (o, ci, float(tab), float(ref))
