@@ -35,7 +35,7 @@ __global__ void const_div_check_kernel(float c, float rc) {
         atomicAdd(&g_const_div_bad, 1u);
 }
 
-bool const_div_exact(int c, float* rc_out) {
+bool const_div_exact(int c, float* rc_out, cudaStream_t caller) {
     static std::mutex mu;
     static std::map<std::pair<int, int>, bool> cache;               // (device, c) -> verified
     static std::map<int, cudaStream_t> check_stream;                // one private non-blocking stream per device
@@ -47,11 +47,18 @@ bool const_div_exact(int c, float* rc_out) {
     std::lock_guard<std::mutex> lock(mu);
     auto it = cache.find({dev, c});
     if (it != cache.end()) return it->second;
+    // The check waits for its result, and a synchronisation while the caller's stream is being captured is refused and
+    // invalidates the capture (global capture mode, PyTorch's default).  So while the caller's stream captures, the
+    // constant is reported as NOT verified and NOT cached, without any call that synchronises: the caller takes the
+    // generic IEEE division (same bits), and the first call outside a capture verifies it.
+    cudaStreamCaptureStatus capture = cudaStreamCaptureStatusNone;
+    if (cudaStreamIsCapturing(caller, &capture) != cudaSuccess || capture != cudaStreamCaptureStatusNone) {
+        cudaGetLastError();
+        return false;
+    }
     // First use of this constant on this device: one small launch + a 4-byte read-back, on a PRIVATE non-blocking
-    // stream with asynchronous copies (never the legacy stream: no device-wide synchronisation, nothing joins a
-    // stream capture that may be in progress on the caller's stream).  If the check cannot run -- e.g. this thread
-    // is inside a capture whose mode forbids the synchronisation -- the constant is reported as NOT verified and
-    // NOT cached: the caller then takes the generic IEEE division (same bits), and a later call verifies it.
+    // stream with asynchronous copies (never the legacy stream: no device-wide synchronisation).  If the check cannot
+    // run, the constant is likewise reported as not verified and not cached.
     cudaStream_t& cs = check_stream[dev];
     bool ran = true;
     if (!cs) ran = cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking) == cudaSuccess;
@@ -102,7 +109,7 @@ int dmh_version(void) { return 1; }
 int dmh_build_arch(void) { return 100; }
 int dmh_const_div_exact(int c) {
     float rc;
-    return dmh::const_div_exact(c, &rc) ? 1 : 0;
+    return dmh::const_div_exact(c, &rc, cudaStreamPerThread) ? 1 : 0;
 }
 int dmh_unpack_u8(const uint8_t* in, long long n, float* out, dmh_stream_t stream) {
     DMH_REQUIRE(in && out, "dmh_unpack_u8: null pointer");

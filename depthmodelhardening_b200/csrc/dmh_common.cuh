@@ -13,8 +13,9 @@ namespace dmh {
 void set_error(const char* fmt, ...);
 void count_launches(int n);   // bookkeeping for dmh_launch_count()
 // true iff div_const(a, c, *rc_out) == a / c bit for bit for every float a (verified exhaustively on the current
-// device the first time a constant is seen: one small launch + a synchronous 4-byte read-back; cached)
-bool const_div_exact(int c, float* rc_out);
+// device the first time a constant is seen: one small launch + a synchronous 4-byte read-back; cached).  While
+// `caller` (the stream the kernel will be launched on) is being captured, an unseen constant reports false.
+bool const_div_exact(int c, float* rc_out, cudaStream_t caller);
 
 #define DMH_REQUIRE(cond, ...)                    \
     do {                                          \

@@ -508,7 +508,7 @@ int launch_photo_fast(const float* target, const float* src, const float* T, con
         use_tma = (r == CUDA_SUCCESS);
     }
     // division by W-1 / H-1 in the coordinate chain: the 3-instruction form where it is proven bit-exact
-    const bool fastdiv = W > 1 && H > 1 && const_div_exact(W - 1, &p.rcw) && const_div_exact(H - 1, &p.rch);
+    const bool fastdiv = W > 1 && H > 1 && const_div_exact(W - 1, &p.rcw, st) && const_div_exact(H - 1, &p.rch, st);
     const bool packed = (flags & DMH_PHOTO_SRC_PACKED) != 0;
     const bool up = !(disp_h == H && disp_w == W);
 #define DMH_FAST_GO(T_, D_, P_, U_)                                                                           \

@@ -822,7 +822,8 @@ extern "C" int dmh_photo_multisource(const float* target, const float* const* sr
             return DMH_ERR_UNSUPPORTED;
         }
     }
-    const bool fastdiv = const_div_exact(W - 1, &p.rcw) && const_div_exact(H - 1, &p.rch);
+    const bool fastdiv = const_div_exact(W - 1, &p.rcw, (cudaStream_t)stream) &&
+                         const_div_exact(H - 1, &p.rch, (cudaStream_t)stream);
     p.gx = ceil_div(W, FT_T); p.gy = ceil_div(H, FT_T);
     cudaStream_t st = (cudaStream_t)stream;
     {

@@ -427,15 +427,16 @@ def test_general_kernel_full_size_properties(dev, hw):
 def test_constant_division_is_verified_exact(dev):
     """The fused kernel divides by W-1 / H-1 with q0 = a*rc; q = fma(fma(-q0, c, a), rc, q0) only for constants
     the library has verified exhaustively (2^24 significands x both signs) to match IEEE division bit for bit;
-    the benchmark / reference sizes must be among them (otherwise the kernel silently keeps IEEE division)."""
+    the benchmark / reference sizes must be among them (otherwise the kernel silently keeps IEEE division).
+    No constant from 1 to 4100 fails the check, so the IEEE-division builds run only for H = 1 or W = 1 (constant 0,
+    refused) and for a size first seen while the launching stream is captured (tests/test_gpu_objective_glue.py)."""
     from depthmodelhardening_b200 import _lib
     lib = _lib.load()
     for c in (1023, 319, 639, 191, 2047):
         assert lib.dmh_const_div_exact(c) == 1, c
     assert lib.dmh_const_div_exact(0) == 0
-    # and the check is not vacuous: some constants do fail it (they take IEEE division)
-    fails = [c for c in range(3, 400, 2) if lib.dmh_const_div_exact(c) == 0]
-    print("constants failing the 3-instruction division:", fails[:10], len(fails))
+    fails = [c for c in range(1, 4101) if lib.dmh_const_div_exact(c) == 0]
+    assert fails == [], "constants failing the 3-instruction division: %s" % fails[:20]
 
 
 def test_cuda_graph_replay_matches_eager(dev):
