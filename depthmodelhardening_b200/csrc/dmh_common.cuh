@@ -65,18 +65,6 @@ __device__ __forceinline__ float block_sum(float v, float* red) {
     return v;
 }
 
-__device__ __forceinline__ float ldg(const float* p) { return __ldg(p); }
-
-// streaming 128-bit load that does not allocate in L1 (data read once)
-__device__ __forceinline__ float4 ld_stream4(const float* p) {
-    float4 v;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];"
-                 : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w)
-                 : "l"(p));
-    return v;
-}
-
-
 // ATen upsample_bilinear2d (align_corners=False) source taps: src = max(scale*(dst+0.5)-0.5, 0)
 struct UpTap { int i0, i1; float l0, l1; };
 __device__ __forceinline__ UpTap up_tap(int dst, float scale, int in_size) {
@@ -104,13 +92,13 @@ __device__ __forceinline__ float load_disp(const DispSrc& d, int b, int iy, int 
            ty.l1 * (tx.l0 * __ldg(p + ty.i1 * d.w + tx.i0) + tx.l1 * __ldg(p + ty.i1 * d.w + tx.i1));
 }
 
-// depth-hints arguments of the single-source fast kernel (photo_fast.cu), handed over by dmh_photo_scale_dh
+// depth-hints arguments of dmh_photo_scale_dh, for the single-source fast kernel (photo_fast.cu) and the general one
 struct FastDhArgs {
     const float* hint_reproj;
     const float* hint_depth;
     const float* hint_valid;
     float* grad_hint;
-    int nblk;              // stride between the four partial-sum arrays
+    int nblk;              // stride between the four partial-sum arrays (set by the launcher of the fast kernel)
 };
 
 }  // namespace dmh

@@ -35,13 +35,8 @@
 // phase; the 1-px reflection (ReflectionPad2d) of border tiles is patched in
 // shared memory afterwards.  Rows that are not 16-byte aligned (W % 4 != 0 or a
 // misaligned base) take the plain-load instantiation of the same kernel.
-#include <cuda.h>
-#include <string.h>
-
-#include "../../include/dmh_b200.h"
-#include "dmh_common.cuh"
-
-using namespace dmh;
+#include <array>
+#include <utility>
 
 #include "photo_tile.cuh"
 
@@ -437,7 +432,13 @@ ident_bf16_kernel(const IdentParams p, const uint16_t* __restrict__ tgt16, const
     ident_tile_tail(p, xs, ys, tid, b, 0, x0, y0, tgt_f32);
 }
 
-size_t fast_smem_bytes() { return sizeof(float) * (3 * FT_NT + 3 * FT_N2 + 9 * FT_N1 + 24 + 32) + FT_N1; }
+using FastKernel = void (*)(const FastParams, const CUtensorMap);
+
+// every instantiation of photo_fast_kernel, at index TMA + 2 FASTDIV + 4 PK + 8 UP + 16 DH
+template <int... I>
+std::array<FastKernel, sizeof...(I)> fast_kernel_table(std::integer_sequence<int, I...>) {
+    return {photo_fast_kernel<(I & 1) != 0, (I & 2) != 0, (I & 4) != 0, (I & 8) != 0, (I & 16) != 0>...};
+}
 
 }  // namespace
 
@@ -445,7 +446,7 @@ namespace dmh {
 
 int photo_fast_tiles(int H, int W) { return ceil_div(W, FT_T) * ceil_div(H, FT_T); }
 
-// Called by dmh_photo_scale when F == 1 and no pose gradient is requested.
+// Called by dmh_photo_scale and dmh_photo_scale_dh when F == 1 and no pose gradient is requested.
 int launch_photo_fast(const float* target, const float* src, const float* T, const float* disp, int disp_h,
                       int disp_w, const float* K, const float* inv_K, const float* ident, const float* noise, int B, int H, int W, float min_depth,
                       float max_depth, int flags, float grad_scale, float* loss_partial, float* grad_disp,
@@ -455,80 +456,24 @@ int launch_photo_fast(const float* target, const float* src, const float* T, con
     p.disp.ptr = disp; p.disp.h = disp_h; p.disp.w = disp_w; p.disp.sh = (float)disp_h / (float)H; p.disp.sw = (float)disp_w / (float)W; p.inv_K = inv_K; p.ident = ident;
     p.noise = noise; p.loss_partial = loss_partial; p.grad_disp = grad_disp; p.sel = sel; p.warped = warped;
     p.B = B; p.H = H; p.W = W; p.flags = flags;
-    const bool is_depth = (flags & DMH_PHOTO_INPUT_IS_DEPTH) != 0;
-    p.ds.min_disp = is_depth ? 0.f : (float)(1.0 / (double)max_depth);
-    p.ds.range = is_depth ? 0.f : (float)(1.0 / (double)min_depth - 1.0 / (double)max_depth);
+    p.ds = depth_scale(min_depth, max_depth, (flags & DMH_PHOTO_INPUT_IS_DEPTH) != 0);
     p.grad_scale = grad_scale;
     p.hint_reproj = dh ? dh->hint_reproj : nullptr; p.hint_depth = dh ? dh->hint_depth : nullptr;
     p.hint_valid = dh ? dh->hint_valid : nullptr; p.grad_hint = dh ? dh->grad_hint : nullptr;
     p.dh_nblk = dh ? dh->nblk : 0;
-    const size_t smem = fast_smem_bytes();
-    static bool configured_dev[64] = {false};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!configured_dev[dev & 63]) {
-        cudaError_t e = cudaSuccess;
-#define DMH_FAST_FN(T_, D_, P_, U_) (const void*)photo_fast_kernel<T_, D_, P_, U_>
-#define DMH_FAST_FN4(P_, U_) DMH_FAST_FN(false, false, P_, U_), DMH_FAST_FN(false, true, P_, U_), \
-                             DMH_FAST_FN(true, false, P_, U_), DMH_FAST_FN(true, true, P_, U_)
-        const void* fns[16] = {DMH_FAST_FN4(false, false), DMH_FAST_FN4(false, true), DMH_FAST_FN4(true, false),
-                               DMH_FAST_FN4(true, true)};
-#undef DMH_FAST_FN4
-#undef DMH_FAST_FN
-        for (int i = 0; i < 16 && e == cudaSuccess; ++i)
-            e = cudaFuncSetAttribute(fns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-#define DMH_DH_FN(T_, D_, P_, U_) (const void*)photo_fast_kernel<T_, D_, P_, U_, true>
-#define DMH_DH_FN4(P_, U_) DMH_DH_FN(false, false, P_, U_), DMH_DH_FN(false, true, P_, U_), \
-                           DMH_DH_FN(true, false, P_, U_), DMH_DH_FN(true, true, P_, U_)
-        const void* dfns[16] = {DMH_DH_FN4(false, false), DMH_DH_FN4(false, true), DMH_DH_FN4(true, false),
-                                DMH_DH_FN4(true, true)};
-#undef DMH_DH_FN4
-#undef DMH_DH_FN
-        for (int i = 0; i < 16 && e == cudaSuccess; ++i)
-            e = cudaFuncSetAttribute(dfns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) {
-            set_error("dmh_photo_scale(fast): cudaFuncSetAttribute failed: %s", cudaGetErrorString(e));
-            return DMH_ERR_CUDA;
-        }
-        configured_dev[dev & 63] = true;
-    }
+    const size_t smem = tile_smem_bytes();
+    static const std::array<FastKernel, 32> kernels = fast_kernel_table(std::make_integer_sequence<int, 32>());
+    static KernelSetup setup;
+    if (setup.sms("dmh_photo_scale(fast)", kernels.data(), (int)kernels.size(), smem) == 0) return DMH_ERR_CUDA;
     dim3 grid(ceil_div(W, FT_T), ceil_div(H, FT_T), B);
-    // TMA descriptor of the target frames viewed as a (W, H, 3, B) fp32 tensor; needs 16-byte aligned rows
     CUtensorMap map;
-    memset(&map, 0, sizeof(map));
-    bool use_tma = (W % 4 == 0) && ((uintptr_t)target % 16 == 0) && tma_encoder() != nullptr;
-    if (use_tma) {
-        const cuuint64_t gdim[4] = {(cuuint64_t)W, (cuuint64_t)H, 3, (cuuint64_t)B};
-        const cuuint64_t gstr[3] = {(cuuint64_t)W * 4, (cuuint64_t)W * H * 4, (cuuint64_t)W * H * 12};
-        const cuuint32_t box[4] = {FT_TP, FT_R2, 3, 1};
-        const cuuint32_t estr[4] = {1, 1, 1, 1};
-        const CUresult r = tma_encoder()(&map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(target), gdim, gstr,
-                                         box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        use_tma = (r == CUDA_SUCCESS);
-    }
+    const bool use_tma = encode_frames_map(&map, target, B, H, W, FT_TP, FT_R2);
     // division by W-1 / H-1 in the coordinate chain: the 3-instruction form where it is proven bit-exact
     const bool fastdiv = W > 1 && H > 1 && const_div_exact(W - 1, &p.rcw, st) && const_div_exact(H - 1, &p.rch, st);
     const bool packed = (flags & DMH_PHOTO_SRC_PACKED) != 0;
     const bool up = !(disp_h == H && disp_w == W);
-#define DMH_FAST_GO(T_, D_, P_, U_)                                                                           \
-    do {                                                                                                      \
-        if (dh) DMH_LAUNCH((photo_fast_kernel<T_, D_, P_, U_, true>), grid, FT_THREADS, smem, st)(p, map); \
-        else DMH_LAUNCH((photo_fast_kernel<T_, D_, P_, U_>), grid, FT_THREADS, smem, st)(p, map);         \
-    } while (0)
-#define DMH_FAST_GO2(P_, U_)                                           \
-    do {                                                               \
-        if (use_tma && fastdiv) DMH_FAST_GO(true, true, P_, U_);       \
-        else if (use_tma) DMH_FAST_GO(true, false, P_, U_);            \
-        else if (fastdiv) DMH_FAST_GO(false, true, P_, U_);            \
-        else DMH_FAST_GO(false, false, P_, U_);                        \
-    } while (0)
-    if (packed && up) DMH_FAST_GO2(true, true);
-    else if (packed) DMH_FAST_GO2(true, false);
-    else if (up) DMH_FAST_GO2(false, true);
-    else DMH_FAST_GO2(false, false);
-#undef DMH_FAST_GO2
-#undef DMH_FAST_GO
+    const FastKernel kernel = kernels[use_tma + 2 * fastdiv + 4 * packed + 8 * up + 16 * (dh != nullptr)];
+    DMH_LAUNCH(kernel, grid, FT_THREADS, smem, st)(p, map);
     return DMH_OK;
 }
 
@@ -541,24 +486,10 @@ int launch_ident_fast(const float* target, const float* const* src_host, int F, 
     for (int f = 0; f < DMH_PHOTO_MAX_FRAMES; ++f) p.src[f] = f < F ? src_host[f] : nullptr;
     p.out = out; p.B = B; p.F = F; p.H = H; p.W = W; p.no_ssim = no_ssim;
     dim3 grid(ceil_div(W, FT_T), ceil_div(H, FT_T), B * F);
-    // TMA descriptors of the frames viewed as (W, H, 3, B) fp32 tensors; rows must be 16-byte aligned
     IdentMaps maps;
     memset(&maps, 0, sizeof(maps));
-    bool use_tma = (W % 4 == 0) && ((uintptr_t)target % 16 == 0) && tma_encoder() != nullptr;
-    for (int f = 0; f < F && use_tma; ++f) use_tma = (uintptr_t)src_host[f] % 16 == 0;
-    if (use_tma) {
-        const cuuint64_t gdim[4] = {(cuuint64_t)W, (cuuint64_t)H, 3, (cuuint64_t)B};
-        const cuuint64_t gstr[3] = {(cuuint64_t)W * 4, (cuuint64_t)W * H * 4, (cuuint64_t)W * H * 12};
-        const cuuint32_t box[4] = {ID_P, ID_R, 3, 1};
-        const cuuint32_t estr[4] = {1, 1, 1, 1};
-        for (int f = -1; f < F && use_tma; ++f) {
-            const float* base = f < 0 ? target : src_host[f];
-            use_tma = tma_encoder()(f < 0 ? &maps.tgt : &maps.src[f], CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4,
-                                    const_cast<float*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                                    CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-        }
-    }
+    bool use_tma = encode_frames_map(&maps.tgt, target, B, H, W, ID_P, ID_R);
+    for (int f = 0; f < F && use_tma; ++f) use_tma = encode_frames_map(&maps.src[f], src_host[f], B, H, W, ID_P, ID_R);
     if (use_tma) DMH_LAUNCH(ident_fast_kernel<true>, grid, 256, 0, st)(p, maps);
     else DMH_LAUNCH(ident_fast_kernel<false>, grid, 256, 0, st)(p, maps);
     return DMH_OK;

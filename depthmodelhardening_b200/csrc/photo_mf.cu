@@ -755,7 +755,8 @@ extern "C" int dmh_photo_multisource(const float* target, const float* const* sr
     DMH_REQUIRE((long long)H * W < (1ll << 27), "dmh_photo_multisource: frame too large for 32-bit tap offsets");
     DMH_REQUIRE(min_depth > 0.f && max_depth > min_depth, "dmh_photo_multisource: bad depth range");
     DMH_REQUIRE((uintptr_t)workspace % 16 == 0, "dmh_photo_multisource: workspace must be 16-byte aligned");
-    if (W % 4 != 0 || (uintptr_t)target % 16 != 0 || tma_encoder() == nullptr) {
+    CUtensorMap map;
+    if (!encode_frames_map(&map, target, B, H, W, FT_TP, FT_R2)) {
         set_error("dmh_photo_multisource: needs W %% 4 == 0 and 16-byte aligned frames (TMA); use dmh_photo_scale");
         return DMH_ERR_UNSUPPORTED;
     }
@@ -773,8 +774,7 @@ extern "C" int dmh_photo_multisource(const float* target, const float* const* sr
     DMH_REQUIRE(!any_ident || all_ident, "dmh_photo_multisource: identity losses for some sources only");
     p.K = K; p.inv_K = inv_K; p.next_item = reinterpret_cast<int*>(workspace); p.scratch = workspace + 4;
     p.F = F; p.S = S; p.B = B; p.H = H; p.W = W;
-    p.ds.min_disp = (float)(1.0 / (double)max_depth);
-    p.ds.range = (float)(1.0 / (double)min_depth - 1.0 / (double)max_depth);
+    p.ds = depth_scale(min_depth, max_depth, false);
     p.grad_scale = grad_scale;
     bool pose = false;
     for (int s = 0; s < S; ++s) {
@@ -790,38 +790,11 @@ extern "C" int dmh_photo_multisource(const float* target, const float* const* sr
         pose = pose || p.sc[s].grad_P;
     }
     const size_t smem = sizeof(float) * (3 * FT_NT + 3 * FT_N2 + 9 * FT_N1 + MF_MAXF * 24 + 8 + 96) + FT_N1;
-    static bool configured_dev[64] = {false};
-    static int mf_sms[64] = {0};
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (!configured_dev[dev & 63]) {
-        const void* fns[4] = {(const void*)photo_mf_kernel<true, false>, (const void*)photo_mf_kernel<true, true>,
+    static KernelSetup setup;
+    const void* kernels[4] = {(const void*)photo_mf_kernel<true, false>, (const void*)photo_mf_kernel<true, true>,
                               (const void*)photo_mf_kernel<false, false>, (const void*)photo_mf_kernel<false, true>};
-        cudaError_t e = cudaSuccess;
-        for (int i = 0; i < 4 && e == cudaSuccess; ++i)
-            e = cudaFuncSetAttribute(fns[i], cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e == cudaSuccess) e = cudaDeviceGetAttribute(&mf_sms[dev & 63], cudaDevAttrMultiProcessorCount, dev);
-        if (e != cudaSuccess) {
-            set_error("dmh_photo_multisource: cudaFuncSetAttribute failed: %s", cudaGetErrorString(e));
-            return DMH_ERR_CUDA;
-        }
-        configured_dev[dev & 63] = true;
-    }
-    CUtensorMap map;
-    memset(&map, 0, sizeof(map));
-    {
-        const cuuint64_t gdim[4] = {(cuuint64_t)W, (cuuint64_t)H, 3, (cuuint64_t)B};
-        const cuuint64_t gstr[3] = {(cuuint64_t)W * 4, (cuuint64_t)W * H * 4, (cuuint64_t)W * H * 12};
-        const cuuint32_t box[4] = {FT_TP, FT_R2, 3, 1};
-        const cuuint32_t estr[4] = {1, 1, 1, 1};
-        const CUresult r = tma_encoder()(&map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(target), gdim, gstr,
-                                         box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE,
-                                         CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) {
-            set_error("dmh_photo_multisource: cuTensorMapEncodeTiled failed (%d); use dmh_photo_scale", (int)r);
-            return DMH_ERR_UNSUPPORTED;
-        }
-    }
+    const int sms = setup.sms("dmh_photo_multisource", kernels, 4, smem);
+    if (sms == 0) return DMH_ERR_CUDA;
     const bool fastdiv = const_div_exact(W - 1, &p.rcw, (cudaStream_t)stream) &&
                          const_div_exact(H - 1, &p.rch, (cudaStream_t)stream);
     p.gx = ceil_div(W, FT_T); p.gy = ceil_div(H, FT_T);
@@ -839,12 +812,8 @@ extern "C" int dmh_photo_multisource(const float* target, const float* const* sr
         }
     }
     // persistent grid of 2 CTAs per SM; the tiles of the partial last round become S single-scale items each
-    const int slots = 2 * mf_sms[dev & 63], n_tiles = p.gx * p.gy * B;
-    p.n_full = n_tiles;
-    if (S > 1 && n_tiles > slots) {
-        const int tail = n_tiles % slots;
-        if (tail > 0 && (tail * S + slots - 1) / slots < S) p.n_full = n_tiles - tail;
-    }
+    const int slots = 2 * sms, n_tiles = p.gx * p.gy * B;
+    p.n_full = split_last_wave(n_tiles, S, slots);
     p.n_items = p.n_full + (n_tiles - p.n_full) * S;
     const int n_ctas = p.n_items < slots ? p.n_items : slots;
     {

@@ -15,10 +15,7 @@
 //   read  12 (target) + 12 F (sources, gathered via L2) + 4 (disp) + 4 Fi (ident)
 //         + 4 Fi (noise);  write 4 (grad_disp)  [+1 sel]
 // Shared memory per CTA: (3 + 1 + 3F) * 720 + 9 * 612 + 612 floats (~43 KB, F=1).
-#include "../../include/dmh_b200.h"
-#include "dmh_common.cuh"
-
-using namespace dmh;
+#include "photo_launch.cuh"
 
 namespace {
 
@@ -456,19 +453,9 @@ size_t photo_smem_bytes(int F) {
 template <int F>
 int launch_photo(const PhotoParams& p, dim3 grid, cudaStream_t st) {
     const size_t smem = photo_smem_bytes(F);
-    static bool configured_dev[64] = {false};   // idempotent attribute; racing writers set the same value
-    int dev = 0;
-    cudaGetDevice(&dev);
-    bool& configured = configured_dev[dev & 63];
-    if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(photo_scale_kernel<F>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)smem);
-        if (e != cudaSuccess) {
-            set_error("dmh_photo_scale: cudaFuncSetAttribute failed: %s", cudaGetErrorString(e));
-            return DMH_ERR_CUDA;
-        }
-        configured = true;
-    }
+    static KernelSetup setup;
+    const void* kernel = (const void*)photo_scale_kernel<F>;
+    if (setup.sms("dmh_photo_scale", &kernel, 1, smem) == 0) return DMH_ERR_CUDA;
     DMH_LAUNCH(photo_scale_kernel<F>, grid, PH_THREADS, smem, st)(p);
     return DMH_OK;
 }
@@ -486,6 +473,84 @@ int launch_ident_bf16(const uint16_t* target, const uint16_t* src, int B, int H,
 int launch_ident_fast(const float* target, const float* const* src_host, int F, int B, int H, int W, int no_ssim,
                       float* out, float* packed, cudaStream_t st);
 }  // namespace dmh
+
+namespace {
+
+// dmh_photo_scale (dh == nullptr) and dmh_photo_scale_dh: argument checks, then the single-source fast kernel or the
+// general one.  With depth hints, loss_partial holds the four [B * dmh_photo_tiles] arrays of the depth-hints sums
+// and the fast path also excludes DMH_PHOTO_AVG_REPROJECTION.  `name` is the public entry point, for the errors.
+int photo_scale_launch(const char* name, const float* target, const float* const* src_host, const float* const* T_host,
+                       int F, const float* disp, int disp_h, int disp_w, const float* K, const float* inv_K,
+                       const float* ident, const float* noise, int B, int H, int W, float min_depth, float max_depth,
+                       int flags, float grad_scale, float* loss_partial, float* grad_disp, float* grad_P_partial,
+                       uint8_t* sel, float* const* warped_host, const FastDhArgs* dh, cudaStream_t st) {
+    DMH_REQUIRE(target && src_host && T_host && disp && K && inv_K && loss_partial && grad_disp, "%s: null pointer", name);
+    DMH_REQUIRE(F >= 1 && F <= PH_MAXF, "%s: F=%d outside [1,%d]", name, F, PH_MAXF);
+    DMH_REQUIRE(B > 0 && B <= 65535 && H >= 2 && W >= 2, "%s: bad shape B=%d H=%d W=%d", name, B, H, W);
+    DMH_REQUIRE(disp_h >= 1 && disp_w >= 1 && disp_h <= H && disp_w <= W, "%s: bad disparity size %dx%d", name, disp_h,
+                disp_w);
+    const bool is_depth = (flags & DMH_PHOTO_INPUT_IS_DEPTH) != 0;
+    DMH_REQUIRE(is_depth || (min_depth > 0.f && max_depth > min_depth), "%s: bad depth range", name);
+    DMH_REQUIRE(!(flags & DMH_PHOTO_SRC_PACKED) || (uintptr_t)src_host[0] % 16 == 0,
+                "%s: DMH_PHOTO_SRC_PACKED needs a 16-byte aligned source", name);
+    const int fast_excl = DMH_PHOTO_NO_SSIM | DMH_PHOTO_INPUT_IS_DEPTH | (dh ? DMH_PHOTO_AVG_REPROJECTION : 0);
+    const bool fast_ok = F == 1 && !grad_P_partial && !(warped_host && warped_host[0]) && !(flags & fast_excl) &&
+                         H * (long long)W < (1ll << 28);
+    DMH_REQUIRE(!(flags & DMH_PHOTO_SRC_PACKED) || fast_ok,
+                "%s: DMH_PHOTO_SRC_PACKED needs the single-source fast path (F == 1, SSIM on, disparity input, no pose "
+                "gradient, no warped output)", name);
+    const int nblk = B * dmh_photo_tiles(H, W);
+    if (fast_ok) {
+        // single source frame, no pose gradient: the 32x32-tile fast kernel (photo_fast.cu).  It writes fewer partial
+        // sums than dmh_photo_tiles() promises (at the head of each array); zero the rest so the caller's reduction is
+        // exact.
+        DMH_REQUIRE(src_host[0] && T_host[0], "%s: null src/T for frame 0", name);
+        const int used = B * photo_fast_tiles(H, W);
+        cudaError_t e = cudaSuccess;
+        if (dh) e = cudaMemsetAsync(loss_partial, 0, sizeof(float) * 4 * (size_t)nblk, st);
+        else if (nblk > used) e = cudaMemsetAsync(loss_partial + used, 0, sizeof(float) * (size_t)(nblk - used), st);
+        if (e != cudaSuccess) { set_error("%s: memset failed: %s", name, cudaGetErrorString(e)); return DMH_ERR_CUDA; }
+        FastDhArgs a = {};
+        if (dh) { a = *dh; a.nblk = nblk; }
+        const int rc = launch_photo_fast(target, src_host[0], T_host[0], disp, disp_h, disp_w, K, inv_K, ident, noise, B, H,
+                                         W, min_depth, max_depth, flags, grad_scale, loss_partial, grad_disp, sel,
+                                         warped_host ? warped_host[0] : nullptr, dh ? &a : nullptr, st);
+        if (rc != DMH_OK) return rc;
+        DMH_CHECK_LAUNCH(name);
+        return DMH_OK;
+    }
+    PhotoParams p;
+    p.target = target;
+    for (int f = 0; f < PH_MAXF; ++f) {
+        p.src[f] = f < F ? src_host[f] : nullptr;
+        p.T[f] = f < F ? T_host[f] : nullptr;
+        p.warped[f] = (warped_host && f < F) ? warped_host[f] : nullptr;
+        DMH_REQUIRE(f >= F || (p.src[f] && p.T[f]), "%s: null src/T for frame %d", name, f);
+    }
+    p.disp.ptr = disp; p.disp.h = disp_h; p.disp.w = disp_w;
+    p.disp.sh = (float)disp_h / (float)H; p.disp.sw = (float)disp_w / (float)W;
+    p.K = K; p.inv_K = inv_K; p.ident = ident; p.noise = noise;
+    p.loss_partial = loss_partial; p.grad_disp = grad_disp; p.grad_P_partial = grad_P_partial; p.sel = sel;
+    p.B = B; p.H = H; p.W = W; p.F = F; p.flags = flags;
+    p.ds = depth_scale(min_depth, max_depth, is_depth);
+    p.grad_scale = grad_scale;
+    p.dh = dh != nullptr;
+    p.hint_reproj = dh ? dh->hint_reproj : nullptr; p.hint_depth = dh ? dh->hint_depth : nullptr;
+    p.hint_valid = dh ? dh->hint_valid : nullptr; p.grad_hint = dh ? dh->grad_hint : nullptr;
+    dim3 grid(ceil_div(W, PH_TW), ceil_div(H, PH_TH), B);
+    int rc = DMH_OK;
+    switch (F) {
+        case 1: rc = launch_photo<1>(p, grid, st); break;
+        case 2: rc = launch_photo<2>(p, grid, st); break;
+        case 3: rc = launch_photo<3>(p, grid, st); break;
+        default: rc = launch_photo<4>(p, grid, st); break;
+    }
+    if (rc != DMH_OK) return rc;
+    DMH_CHECK_LAUNCH(name);
+    return DMH_OK;
+}
+
+}  // namespace
 
 extern "C" {
 
@@ -529,15 +594,15 @@ int dmh_identity_loss_pack_bf16(const uint16_t* target_bf16, const uint16_t* src
 
 int dmh_photo_tiles(int H, int W) { return ceil_div(W, PH_TW) * ceil_div(H, PH_TH); }
 
-// depth-hints arguments handed from dmh_photo_scale_dh to the shared launcher below (same thread, same call)
-struct DhNext { bool armed; const float *hint_reproj, *hint_depth, *hint_valid; float* grad_hint; };
-static thread_local DhNext g_dh_next = {false, nullptr, nullptr, nullptr, nullptr};
-
 int dmh_photo_scale(const float* target, const float* const* src_host, const float* const* T_host, int F,
                     const float* disp, int disp_h, int disp_w, const float* K, const float* inv_K, const float* ident,
                     const float* noise, int B, int H, int W, float min_depth, float max_depth, int flags, float grad_scale,
                     float* loss_partial, float* grad_disp, float* grad_P_partial, uint8_t* sel,
-                    float* const* warped_host, dmh_stream_t stream);
+                    float* const* warped_host, dmh_stream_t stream) {
+    return photo_scale_launch("dmh_photo_scale", target, src_host, T_host, F, disp, disp_h, disp_w, K, inv_K, ident,
+                              noise, B, H, W, min_depth, max_depth, flags, grad_scale, loss_partial, grad_disp,
+                              grad_P_partial, sel, warped_host, nullptr, (cudaStream_t)stream);
+}
 
 int dmh_photo_scale_dh(const float* target, const float* const* src_host, const float* const* T_host, int F,
                        const float* disp, int disp_h, int disp_w, const float* K, const float* inv_K,
@@ -548,113 +613,10 @@ int dmh_photo_scale_dh(const float* target, const float* const* src_host, const 
     DMH_REQUIRE(!hint_reproj || (hint_depth && hint_valid && grad_disp_hint),
                 "dmh_photo_scale_dh: depth hints need hint_depth, hint_valid and grad_disp_hint");
     DMH_REQUIRE(!noise || ident, "dmh_photo_scale_dh: noise without identity losses");
-    // single source, no pose gradient (the stereo-only depth-hints configuration): the 32x32-tile fast kernel
-    // with the depth-hints decision; same contract (its fewer per-CTA partials sit at the head of each array)
-    if (F == 1 && !grad_P_partial && !(flags & (DMH_PHOTO_FORCE_GENERIC | DMH_PHOTO_NO_SSIM | DMH_PHOTO_INPUT_IS_DEPTH |
-                                                DMH_PHOTO_AVG_REPROJECTION)) &&
-        H * (long long)W < (1ll << 28)) {
-        DMH_REQUIRE(target && src_host && src_host[0] && T_host && T_host[0] && disp && K && inv_K && sums_partial && grad_disp,
-                    "dmh_photo_scale_dh: null pointer");
-        DMH_REQUIRE(B > 0 && B <= 65535 && H >= 2 && W >= 2 && disp_h >= 1 && disp_w >= 1 && disp_h <= H && disp_w <= W,
-                    "dmh_photo_scale_dh: bad shape");
-        DMH_REQUIRE(min_depth > 0.f && max_depth > min_depth, "dmh_photo_scale_dh: bad depth range");
-        DMH_REQUIRE(!(flags & DMH_PHOTO_SRC_PACKED) || (uintptr_t)src_host[0] % 16 == 0,
-                    "dmh_photo_scale_dh: DMH_PHOTO_SRC_PACKED needs a 16-byte aligned source");
-        const int nblk = B * dmh_photo_tiles(H, W);
-        cudaError_t e = cudaMemsetAsync(sums_partial, 0, sizeof(float) * 4 * (size_t)nblk, (cudaStream_t)stream);
-        if (e != cudaSuccess) { set_error("dmh_photo_scale_dh: memset failed: %s", cudaGetErrorString(e)); return DMH_ERR_CUDA; }
-        FastDhArgs a;
-        a.hint_reproj = hint_reproj; a.hint_depth = hint_depth; a.hint_valid = hint_valid; a.grad_hint = grad_disp_hint;
-        a.nblk = nblk;
-        const int rc = launch_photo_fast(target, src_host[0], T_host[0], disp, disp_h, disp_w, K, inv_K, ident, noise, B, H, W,
-                                         min_depth, max_depth, flags, 1.0f, sums_partial, grad_disp, sel, nullptr, &a,
-                                         (cudaStream_t)stream);
-        if (rc != DMH_OK) return rc;
-        DMH_CHECK_LAUNCH("dmh_photo_scale_dh(fast)");
-        return DMH_OK;
-    }
-    DMH_REQUIRE(!(flags & DMH_PHOTO_SRC_PACKED), "dmh_photo_scale_dh: DMH_PHOTO_SRC_PACKED needs the single-source fast path");
-    g_dh_next.armed = true;
-    g_dh_next.hint_reproj = hint_reproj; g_dh_next.hint_depth = hint_depth; g_dh_next.hint_valid = hint_valid;
-    g_dh_next.grad_hint = grad_disp_hint;
-    const int rc = dmh_photo_scale(target, src_host, T_host, F, disp, disp_h, disp_w, K, inv_K, ident, noise, B, H, W,
-                                   min_depth, max_depth, flags | DMH_PHOTO_FORCE_GENERIC, 1.0f, sums_partial, grad_disp,
-                                   grad_P_partial, sel, nullptr, stream);
-    g_dh_next.armed = false;
-    return rc;
-}
-
-int dmh_photo_scale(const float* target, const float* const* src_host, const float* const* T_host, int F,
-                    const float* disp, int disp_h, int disp_w, const float* K, const float* inv_K, const float* ident,
-                    const float* noise, int B, int H, int W, float min_depth, float max_depth, int flags, float grad_scale,
-                    float* loss_partial, float* grad_disp, float* grad_P_partial, uint8_t* sel,
-                    float* const* warped_host, dmh_stream_t stream) {
-    DMH_REQUIRE(target && src_host && T_host && disp && K && inv_K && loss_partial && grad_disp,
-                "dmh_photo_scale: null pointer");
-    DMH_REQUIRE(F >= 1 && F <= PH_MAXF, "dmh_photo_scale: F=%d outside [1,%d]", F, PH_MAXF);
-    DMH_REQUIRE(B > 0 && B <= 65535 && H >= 2 && W >= 2, "dmh_photo_scale: bad shape B=%d H=%d W=%d", B, H, W);
-    DMH_REQUIRE(disp_h >= 1 && disp_w >= 1 && disp_h <= H && disp_w <= W, "dmh_photo_scale: bad disparity size %dx%d", disp_h, disp_w);
-    const bool is_depth = (flags & DMH_PHOTO_INPUT_IS_DEPTH) != 0;
-    DMH_REQUIRE(is_depth || (min_depth > 0.f && max_depth > min_depth), "dmh_photo_scale: bad depth range");
-    DMH_REQUIRE(!(flags & DMH_PHOTO_SRC_PACKED) || (uintptr_t)src_host[0] % 16 == 0,
-                "dmh_photo_scale: DMH_PHOTO_SRC_PACKED needs a 16-byte aligned source");
-    const bool fast_ok = F == 1 && !grad_P_partial && !(warped_host && warped_host[0]) &&
-                         !(flags & (DMH_PHOTO_FORCE_GENERIC | DMH_PHOTO_NO_SSIM | DMH_PHOTO_INPUT_IS_DEPTH)) &&
-                         H * (long long)W < (1ll << 28);
-    DMH_REQUIRE(!(flags & DMH_PHOTO_SRC_PACKED) || fast_ok,
-                "dmh_photo_scale: DMH_PHOTO_SRC_PACKED needs the single-source fast path (F == 1, SSIM on, disparity "
-                "input, no pose gradient, no warped output)");
-    if (fast_ok) {
-        // single source frame, no pose gradient: the 32x32-tile fast kernel (photo_fast.cu).  It writes
-        // fewer partial sums than dmh_photo_tiles() promises; zero the tail so the caller's reduction is exact.
-        DMH_REQUIRE(src_host[0] && T_host[0], "dmh_photo_scale: null src/T for frame 0");
-        const int used = B * photo_fast_tiles(H, W), total = B * dmh_photo_tiles(H, W);
-        if (total > used) {
-            cudaError_t e = cudaMemsetAsync(loss_partial + used, 0, sizeof(float) * (size_t)(total - used),
-                                            (cudaStream_t)stream);
-            if (e != cudaSuccess) { set_error("dmh_photo_scale: memset failed: %s", cudaGetErrorString(e)); return DMH_ERR_CUDA; }
-        }
-        const int rc = launch_photo_fast(target, src_host[0], T_host[0], disp, disp_h, disp_w, K, inv_K, ident, noise, B, H, W, min_depth,
-                                         max_depth, flags, grad_scale, loss_partial, grad_disp, sel,
-                                         warped_host ? warped_host[0] : nullptr, nullptr, (cudaStream_t)stream);
-        if (rc != DMH_OK) return rc;
-        DMH_CHECK_LAUNCH("dmh_photo_scale(fast)");
-        return DMH_OK;
-    }
-    PhotoParams p;
-    p.target = target;
-    for (int f = 0; f < PH_MAXF; ++f) {
-        p.src[f] = f < F ? src_host[f] : nullptr;
-        p.T[f] = f < F ? T_host[f] : nullptr;
-        p.warped[f] = (warped_host && f < F) ? warped_host[f] : nullptr;
-        DMH_REQUIRE(f >= F || (p.src[f] && p.T[f]), "dmh_photo_scale: null src/T for frame %d", f);
-    }
-    p.disp.ptr = disp; p.disp.h = disp_h; p.disp.w = disp_w;
-    p.disp.sh = (float)disp_h / (float)H; p.disp.sw = (float)disp_w / (float)W;
-    p.K = K; p.inv_K = inv_K; p.ident = ident; p.noise = noise;
-    p.loss_partial = loss_partial; p.grad_disp = grad_disp; p.grad_P_partial = grad_P_partial; p.sel = sel;
-    p.B = B; p.H = H; p.W = W; p.F = F; p.flags = flags;
-    p.ds.min_disp = is_depth ? 0.f : (float)(1.0 / (double)max_depth);
-    p.ds.range = is_depth ? 0.f : (float)(1.0 / (double)min_depth - 1.0 / (double)max_depth);
-    p.grad_scale = grad_scale;
-    p.dh = 0; p.hint_reproj = nullptr; p.hint_depth = nullptr; p.hint_valid = nullptr; p.grad_hint = nullptr;
-    if (g_dh_next.armed) {       // set by dmh_photo_scale_dh on this thread for the call it forwards
-        p.dh = 1; p.hint_reproj = g_dh_next.hint_reproj; p.hint_depth = g_dh_next.hint_depth;
-        p.hint_valid = g_dh_next.hint_valid; p.grad_hint = g_dh_next.grad_hint;
-        g_dh_next.armed = false;
-    }
-    dim3 grid(ceil_div(W, PH_TW), ceil_div(H, PH_TH), B);
-    cudaStream_t st = (cudaStream_t)stream;
-    int rc = DMH_OK;
-    switch (F) {
-        case 1: rc = launch_photo<1>(p, grid, st); break;
-        case 2: rc = launch_photo<2>(p, grid, st); break;
-        case 3: rc = launch_photo<3>(p, grid, st); break;
-        default: rc = launch_photo<4>(p, grid, st); break;
-    }
-    if (rc != DMH_OK) return rc;
-    DMH_CHECK_LAUNCH("dmh_photo_scale");
-    return DMH_OK;
+    const FastDhArgs dh = {hint_reproj, hint_depth, hint_valid, grad_disp_hint, 0};
+    return photo_scale_launch("dmh_photo_scale_dh", target, src_host, T_host, F, disp, disp_h, disp_w, K, inv_K, ident,
+                              noise, B, H, W, min_depth, max_depth, flags, 1.0f, sums_partial, grad_disp, grad_P_partial,
+                              sel, nullptr, &dh, (cudaStream_t)stream);
 }
 
 }  // extern "C"

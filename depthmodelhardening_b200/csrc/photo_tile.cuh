@@ -3,13 +3,7 @@
 // phase B (sliding-window SSIM + decision + gated coefficients) and phase C (box sums -> gradient).
 // Everything sits in an anonymous namespace: each translation unit gets its own copy.
 #pragma once
-#include <cuda.h>
-#include <string.h>
-
-#include "../../include/dmh_b200.h"
-#include "dmh_common.cuh"
-
-using namespace dmh;
+#include "photo_launch.cuh"
 
 namespace {
 
@@ -56,6 +50,10 @@ __device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, u
 #define FT_THREADS 256
 #define FT_STRIPS 7
 #define FT_ROWS 5                // 7 strips x 5 rows >= 34 ring rows
+
+// dynamic shared memory of photo_fast_kernel and photo_ms_kernel: target tile, warped tile, the 9 coefficient planes,
+// camera (24 floats), reduction slots (32 floats) and the gate bytes
+size_t tile_smem_bytes() { return sizeof(float) * (3 * FT_NT + 3 * FT_N2 + 9 * FT_N1 + 24 + 32) + FT_N1; }
 
 struct FastParams {
     const float* target;
@@ -438,22 +436,6 @@ __device__ __forceinline__ void phase_c(const P& p, const TileSmem& sm, int tid,
             hprevC[0] = hprevC[1]; hprevC[1] = hcC;
         }
     }
-}
-
-// cuTensorMapEncodeTiled through the runtime's driver entry point lookup (no link-time libcuda dependency)
-typedef CUresult (*TmaEncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-TmaEncodeFn tma_encoder() {
-    static TmaEncodeFn fn = [] {
-        void* f = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &f, cudaEnableDefault, &q) != cudaSuccess ||
-            q != cudaDriverEntryPointSuccess)
-            f = nullptr;
-        return reinterpret_cast<TmaEncodeFn>(f);
-    }();
-    return fn;
 }
 
 }  // namespace

@@ -284,11 +284,7 @@ class _ObjectiveDH(torch.autograd.Function):
         if need_T:
             for f in range(n_src):
                 if ctx.needs_input_grad[base + f]:
-                    acc = None
-                    for s in range(S):
-                        t = gPs[s][f].sum(1) * u_r[s]
-                        acc = t if acc is None else acc + t
-                    _, g_T[f] = ops._grad_KT_from_P(acc.view(-1, 3, 4), k, Ts[f], False, True)
+                    g_T[f] = ops._pose_grad_T(gPs, u_r, f, k, Ts[f])
         return (None,) * 7 + (None,) * S + (None,) * n_src + tuple(g_T) + tuple(grads_disp) + \
             ((None,) * S if has_noise else ())
 

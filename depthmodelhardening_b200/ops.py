@@ -151,6 +151,16 @@ def _grad_KT_from_P(gP, K, T, need_K, need_T):
     return gK, gT
 
 
+def _pose_grad_T(gPs, u, f, K, T):
+    """d(loss)/d(T) of source f from the per-scale pose-gradient partials gPs[s] (F,B,tiles,12): summed over the tiles,
+    weighted by the upstream u[s] and added in scale order."""
+    acc = None
+    for s, gP in enumerate(gPs):
+        t = gP[f].sum(1) * u[s]
+        acc = t if acc is None else acc + t
+    return _grad_KT_from_P(acc.view(-1, 3, 4), K, T, False, True)[1]
+
+
 # ----------------------------------------------------------------------------- A12
 class _GridSample(torch.autograd.Function):
     @staticmethod
@@ -520,7 +530,7 @@ class _Objective(torch.autograd.Function):
             check(lib.dmh_identity_loss(ptr(target), src_arr, n_src, B, H, W, no_ssim, ptr(ident), stream()),
                   "identity_loss")
         tiles = lib.dmh_photo_tiles(H, W)
-        G, gN, wss, parts, gPs, sels = [], [], [], [], [], []
+        gN, wss = [], []
         T_arr = ptr_array(Ts)
         inv_den = 1.0 / float(B * H * W)
         # the smoothness term (memory-bound, 8 small launches) is independent of the photometric kernels
@@ -542,18 +552,21 @@ class _Objective(torch.autograd.Function):
         # tail of one launch (10240 CTAs = 23.06 waves of 444) overlaps the head of the next
         multiscale = (packed and MULTISCALE and S <= 4 and W % 4 == 0 and target.data_ptr() % 16 == 0
                       and H * W < (1 << 27))
-        if multisrc:
+        parts = [torch.empty(B * tiles, device=dev, dtype=torch.float32) for _ in range(S)]
+        G = [torch.empty(B, 1, H, W, device=dev, dtype=torch.float32) for _ in range(S)]
+        sels = [torch.empty(B, H, W, device=dev, dtype=torch.uint8) if want_sel else None for _ in range(S)]
+        if multisrc and need_T:
             tiles32 = ((H + 31) // 32) * ((W + 31) // 32)
             # one buffer for the pose-gradient partials of every scale: the backward reduces it with one einsum
-            gP_all = torch.empty(S, n_src, B, tiles32, 12, device=dev, dtype=torch.float32) if need_T else None
-            for s in range(S):
-                parts.append(torch.empty(B * tiles, device=dev, dtype=torch.float32))
-                G.append(torch.empty(B, 1, H, W, device=dev, dtype=torch.float32))
-                gPs.append(gP_all[s] if need_T else None)
-                sels.append(torch.empty(B, H, W, device=dev, dtype=torch.uint8) if want_sel else None)
+            gP_all = torch.empty(S, n_src, B, tiles32, 12, device=dev, dtype=torch.float32)
+            gPs = list(gP_all)
+        else:
+            gPs = [torch.empty(n_src, B, tiles, 12, device=dev, dtype=torch.float32) if need_T else None
+                   for _ in range(S)]
+        dh_ = (_C.c_int * S)(*[d.shape[2] for d in disps])
+        dw_ = (_C.c_int * S)(*[d.shape[3] for d in disps])
+        if multisrc:
             mf_ws = torch.empty(lib.dmh_photo_multisource_workspace_floats(n_src), device=dev, dtype=torch.float32)
-            dh_ = (_C.c_int * S)(*[d.shape[2] for d in disps])
-            dw_ = (_C.c_int * S)(*[d.shape[3] for d in disps])
             with _timed("photo_mf"):
                 check(lib.dmh_photo_multisource(ptr(target), ptr_array(src_pks), ptr_array(Ts), n_src, S, ptr_array(disps),
                                                 dh_, dw_, ptr(k), ptr(ik), ptr_array(idents) if automask else None,
@@ -564,13 +577,6 @@ class _Objective(torch.autograd.Function):
         if multiscale:
             # ONE launch for all scales (csrc/photo_ms.cu): the scale loop of generate_images_pred / compute_losses
             # runs inside the kernel; same bits as the per-scale launches below
-            for s in range(S):
-                parts.append(torch.empty(B * tiles, device=dev, dtype=torch.float32))
-                G.append(torch.empty(B, 1, H, W, device=dev, dtype=torch.float32))
-                gPs.append(None)
-                sels.append(torch.empty(B, H, W, device=dev, dtype=torch.uint8) if want_sel else None)
-            dh_ = (_C.c_int * S)(*[d.shape[2] for d in disps])
-            dw_ = (_C.c_int * S)(*[d.shape[3] for d in disps])
             with _timed("photo_ms"):
                 check(lib.dmh_photo_multiscale(ptr(target), ptr(src_pk), ptr(Ts[0]), S, ptr_array(disps), dh_, dw_, ptr(k),
                                                ptr(ik), ptr(ident), ptr_array(noises) if has_noise else None, B, H, W,
@@ -579,28 +585,20 @@ class _Objective(torch.autograd.Function):
         alt = _side_stream(dev, 1)
         alt.wait_stream(cur)
         for s in range(S if not (multiscale or multisrc) else 0):
-            d = disps[s]
-            h, w = d.shape[2], d.shape[3]
-            part = torch.empty(B * tiles, device=dev, dtype=torch.float32)
-            g_full = torch.empty(B, 1, H, W, device=dev, dtype=torch.float32)
-            gP = torch.empty(n_src, B, tiles, 12, device=dev, dtype=torch.float32) if need_T else None
-            sel = torch.empty(B, H, W, device=dev, dtype=torch.uint8) if want_sel else None
             with torch.cuda.stream(alt if (s & 1) else cur):
                 with _timed("photo_scale"):
-                    check(lib.dmh_photo_scale(ptr(target), src_arr, T_arr, n_src, ptr(d), h, w, ptr(k), ptr(ik),
-                                              ptr(ident), ptr(noises[s]), B, H, W, min_depth, max_depth, flags, inv_den,
-                                              ptr(part), ptr(g_full), ptr(gP), ptr(sel), None, stream()), "photo_scale")
-            G.append(g_full); parts.append(part); gPs.append(gP); sels.append(sel)
+                    check(lib.dmh_photo_scale(ptr(target), src_arr, T_arr, n_src, ptr(disps[s]), dh_[s], dw_[s], ptr(k),
+                                              ptr(ik), ptr(ident), ptr(noises[s]), B, H, W, min_depth, max_depth, flags,
+                                              inv_den, ptr(parts[s]), ptr(G[s]), ptr(gPs[s]), ptr(sels[s]), None,
+                                              stream()), "photo_scale")
         cur.wait_stream(alt)
         cur.wait_stream(side)
         img_scalars = torch.empty(S, B, 2, device=dev, dtype=torch.float32)
         losses = torch.empty(S + 1, device=dev, dtype=torch.float32)
-        hs = (_C.c_int * S)(*[d.shape[2] for d in disps])
-        wsz = (_C.c_int * S)(*[d.shape[3] for d in disps])
         pn = (_C.c_int * S)(*[p_.numel() for p_ in parts])
         sw = (_C.c_float * S)(*[float(x) for x in smooth_w])
         fin_ws = torch.empty(lib.dmh_objective_finish_workspace_bytes(S, B), device=dev, dtype=torch.uint8)
-        check(lib.dmh_objective_finish(S, B, ptr_array(wss), hs, wsz, ptr_array(parts), pn, sw, float(B * H * W),
+        check(lib.dmh_objective_finish(S, B, ptr_array(wss), dh_, dw_, ptr_array(parts), pn, sw, float(B * H * W),
                                        ptr(fin_ws), ptr(img_scalars), ptr(losses), stream()), "objective_finish")
         ctx.cfg = (S, n_src, B, H, W, tuple(float(x) for x in smooth_w), need_T, [tuple(d.shape) for d in disps],
                    has_noise)
@@ -661,11 +659,7 @@ class _Objective(torch.autograd.Function):
             u = [(gt[0] / S if gt is not None else 0.0) + (gs[s] if gs is not None else 0.0) for s in range(S)]
             for f in range(n_src):
                 if ctx.needs_input_grad[base + f]:
-                    acc = None
-                    for s in range(S):
-                        t = gPs[s][f].sum(1) * u[s]
-                        acc = t if acc is None else acc + t
-                    _, g_T[f] = _grad_KT_from_P(acc.view(-1, 3, 4), k, Ts[f], False, True)
+                    g_T[f] = _pose_grad_T(gPs, u, f, k, Ts[f])
         return (None, None, None) + (None,) * S + (None,) * n_src + tuple(g_T) + tuple(grads_disp) + \
             ((None,) * S if has_noise else ())
 

@@ -166,7 +166,6 @@ int dmh_identity_loss_pack_bf16(const uint16_t* target_bf16, const uint16_t* src
 #define DMH_PHOTO_NO_SSIM 1
 #define DMH_PHOTO_AVG_REPROJECTION 2
 #define DMH_PHOTO_INPUT_IS_DEPTH 4
-#define DMH_PHOTO_FORCE_GENERIC 8 /* testing: never take the single-source fast kernel */
 #define DMH_PHOTO_SRC_PACKED 16 /* src_host[0] is the (B,H,W,4) layout of dmh_identity_loss_pack; F == 1, no pose grad */
 #define DMH_PHOTO_MAX_FRAMES 4
 int dmh_photo_tiles(int H, int W);           /* CTAs per batch item */
