@@ -65,6 +65,19 @@ __device__ __forceinline__ float block_sum(float v, float* red) {
     return v;
 }
 
+// Scatter `val` for the west/east tap pair of one source row with warp
+// aggregation: when lane+1's west tap is this lane's east tap (the common case
+// for a smooth disparity) the two contributions are summed in registers and a
+// single RED is issued.
+__device__ __forceinline__ void scatter_row(float* __restrict__ gp, long long o_w, bool w_in, bool e_in, float v_w,
+                                            float v_e, bool merge_e, bool recv_w, unsigned lane) {
+    const float send = (merge_e && e_in) ? v_e : 0.0f;
+    const float got = __shfl_up_sync(0xffffffffu, send, 1);
+    if (recv_w && lane > 0) v_w += got;
+    if (w_in && (v_w != 0.0f)) atomicAdd(gp + o_w, v_w);
+    if (e_in && !merge_e && (v_e != 0.0f)) atomicAdd(gp + o_w + 1, v_e);
+}
+
 // ATen upsample_bilinear2d (align_corners=False) source taps: src = max(scale*(dst+0.5)-0.5, 0)
 struct UpTap { int i0, i1; float l0, l1; };
 __device__ __forceinline__ UpTap up_tap(int dst, float scale, int in_size) {

@@ -279,6 +279,68 @@ DMH_HD SsimCoef ssim_coef(const SsimStats& s) {
 // reflect index for ReflectionPad2d(1): -1 -> 1, n -> n-2 (n >= 2)
 DMH_HD int reflect1(int i, int n) { return i < 0 ? -i : (i >= n ? 2 * n - 2 - i : i); }
 
+// image index of a position of a tile's 2-px halo: the 1-px reflection ring, clamped beyond it
+DMH_HD int ext_to_img(int e, int n) {
+    e = e < -1 ? -1 : (e > n ? n : e);
+    return reflect1(e, n);
+}
+// multiplicity with which window centre q (valid pixel) touches pixel p along one axis
+DMH_HD float reflect_mult(int p, int q, int n) {
+    float m = 1.0f;
+    if (p == 1 && q == 0) m += 1.0f;
+    if (p == n - 2 && q == n - 1) m += 1.0f;
+    return m;
+}
+
+// The in-image taps of one border-clamped bilinear sample (the others contribute nothing)
+struct Taps {
+    long long o00;
+    bool nw, ne, sw, se;
+};
+DMH_HD Taps make_taps(const Bilinear& bl, int H, int W) {
+    Taps t;
+    const bool x0in = bl.x0 >= 0 && bl.x0 < W, x1in = bl.x0 + 1 >= 0 && bl.x0 + 1 < W;
+    const bool y0in = bl.y0 >= 0 && bl.y0 < H, y1in = bl.y0 + 1 >= 0 && bl.y0 + 1 < H;
+    t.o00 = (long long)bl.y0 * W + bl.x0;
+    t.nw = y0in && x0in; t.ne = y0in && x1in; t.sw = y1in && x0in; t.se = y1in && x1in;
+    return t;
+}
+
+// ---------------------------------------------------------------------------
+// Colour-frame gradients of the min-reprojection objective.  `sel` is the candidate the forward picked, in the
+// reference's cat order: n_ident identity candidates (F, 1 under avg_reprojection, 0 without automask), then the
+// reprojections (F, or 1 under avg_reprojection).  Each returns the share of d(loss)/d(candidate) that source
+// frame f's reprojection / identity candidate receives at that pixel.
+DMH_HD float reproj_gate(int sel, int f, int n_ident, int F, bool avg) {
+    if (avg) return sel == n_ident ? 1.0f / (float)F : 0.0f;
+    return sel == n_ident + f ? 1.0f : 0.0f;
+}
+DMH_HD float ident_gate(int sel, int f, int n_ident, int F, bool avg) {
+    if (n_ident == 0) return 0.0f;
+    if (avg) return sel == 0 ? 1.0f / (float)F : 0.0f;
+    return sel == f ? 1.0f : 0.0f;
+}
+
+// d(gated loss)/d(x_p) and d/d(y_p) for one channel of R(x, y) = w_ssim*SSIM + w_l1*|y - x| at pixel p, from the
+// window sums over every centre q whose window reaches p (reflection multiplicities included) of the gated
+// coefficients: sa = sum ax, sd = sum ay, sb = sum b, sc = sum c (see SsimCoef), and the gate times w_l1 at p.
+// The sign of x - y is 0 at a tie, as torch's abs backward.
+DMH_HD void reproj_pixel_grad(float sa, float sb, float sc, float sd, float x, float y, float gl1, float& gx,
+                              float& gy) {
+    const float d = x - y;
+    const float sg = d > 0.f ? gl1 : (d < 0.f ? -gl1 : 0.f);
+    gx = sa + sb * x + sc * y + sg;
+    gy = sd + sb * y + sc * x - sg;
+}
+
+// d/d(I_c(a)) of |dn_a - dn_b| * exp(-mean_c |I_c(a) - I_c(b)|) for one edge (a, b) of the smoothness term,
+// given the edge's |dn_a - dn_b| * exp(...) = de and the channel count C; d/d(I_c(b)) is its negative.
+DMH_HD float smooth_edge_img_grad(float de, float ia, float ib, int C) {
+    const float d = ia - ib;
+    const float sg = d > 0.f ? 1.f : (d < 0.f ? -1.f : 0.f);
+    return -de * sg / (float)C;
+}
+
 
 // ---------------------------------------------------------------------------
 // Fast-path SSIM used by the fused kernels (photo_fast.cu, photo_objective.cu, identity loss): separable

@@ -55,30 +55,6 @@ struct PhotoParams {
     float* grad_hint;              // (B,1,H,W) d(sum proxy*mask_h)/d(up-sampled disp)
 };
 
-__device__ __forceinline__ int ext_to_img(int e, int n) {
-    e = e < -1 ? -1 : (e > n ? n : e);
-    return reflect1(e, n);
-}
-__device__ __forceinline__ float reflect_mult(int p, int q, int n) {
-    float m = 1.0f;
-    if (p == 1 && q == 0) m += 1.0f;
-    if (p == n - 2 && q == n - 1) m += 1.0f;
-    return m;
-}
-
-struct Taps {
-    long long o00;
-    bool nw, ne, sw, se;
-};
-__device__ __forceinline__ Taps make_taps(const Bilinear& bl, int H, int W) {
-    Taps t;
-    const bool x0in = bl.x0 >= 0 && bl.x0 < W, x1in = bl.x0 + 1 >= 0 && bl.x0 + 1 < W;
-    const bool y0in = bl.y0 >= 0 && bl.y0 < H, y1in = bl.y0 + 1 >= 0 && bl.y0 + 1 < H;
-    t.o00 = (long long)bl.y0 * W + bl.x0;
-    t.nw = y0in && x0in; t.ne = y0in && x1in; t.sw = y1in && x0in; t.se = y1in && x1in;
-    return t;
-}
-
 // 3x3 window statistics for one channel plane in shared memory around R2 position (r+1, c+1).
 // Same arithmetic as the single-source fast kernel and the identity-loss kernel (row sums of 3, then 3 rows,
 // mean = sum * (1/9)) so that the automask compares like with like.

@@ -80,11 +80,6 @@ struct FastParams {
     float rcw, rch;              // 1/(W-1), 1/(H-1) for the verified 3-instruction division
 };
 
-__device__ __forceinline__ int ext_to_img(int e, int n) {
-    e = e < -1 ? -1 : (e > n ? n : e);
-    return reflect1(e, n);
-}
-
 struct Gathered { float v[3]; float dix[3], diy[3]; };
 
 // The four bilinear taps of one sampling position.  With border padding the clipped coordinate lies in

@@ -328,18 +328,6 @@ __global__ void reproj_loss_fwd_kernel(const float* __restrict__ pred, const flo
 #define ST_R1H (ST_TH + 2)
 #define ST_THREADS 256
 
-__device__ __forceinline__ int ext_to_img(int e, int n) {
-    e = e < -1 ? -1 : (e > n ? n : e);
-    return reflect1(e, n);
-}
-// multiplicity with which window centre q (valid pixel) touches pixel p along one axis
-__device__ __forceinline__ float reflect_mult(int p, int q, int n) {
-    float m = 1.0f;
-    if (p == 1 && q == 0) m += 1.0f;
-    if (p == n - 2 && q == n - 1) m += 1.0f;
-    return m;
-}
-
 // mode 0: SSIM op   (grad_out is (B,C,H,W), weight 1)
 // mode 1: reprojection loss (grad_out is (B,1,H,W); SSIM weight 0.85/C, L1 weight 0.15/C; no_ssim: L1 weight 1/C)
 __global__ void __launch_bounds__(ST_THREADS)

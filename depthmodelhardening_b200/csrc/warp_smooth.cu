@@ -83,19 +83,6 @@ warp_fwd_kernel(const float* __restrict__ disp, int input_is_depth, DepthScale d
     }
 }
 
-// Scatter `val` for the west/east tap pair of one source row with warp
-// aggregation: when lane+1's west tap is this lane's east tap (the common case
-// for a smooth disparity) the two contributions are summed in registers and a
-// single RED is issued.
-__device__ __forceinline__ void scatter_row(float* __restrict__ gp, long long o_w, bool w_in, bool e_in, float v_w,
-                                            float v_e, bool merge_e, bool recv_w, unsigned lane) {
-    const float send = (merge_e && e_in) ? v_e : 0.0f;
-    const float got = __shfl_up_sync(0xffffffffu, send, 1);
-    if (recv_w && lane > 0) v_w += got;
-    if (w_in && (v_w != 0.0f)) atomicAdd(gp + o_w, v_w);
-    if (e_in && !merge_e && (v_e != 0.0f)) atomicAdd(gp + o_w + 1, v_e);
-}
-
 template <int C>
 __global__ void __launch_bounds__(WARP_THREADS)
 warp_bwd_kernel(const float* __restrict__ gwarped, const float* __restrict__ disp, int input_is_depth, DepthScale ds,

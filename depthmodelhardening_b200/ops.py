@@ -495,6 +495,9 @@ class _Objective(torch.autograd.Function):
         # disp grads are needed iff any disparity requires grad; pose grads iff any T does
         base = 3 + S + n_src
         need_T = any(ctx.needs_input_grad[base + i] for i in range(n_src))
+        # gradients for the colour frames (target, pyramid, sources): the backward recomputes them from the frames,
+        # the disparities and every scale's selection, so `sel` is requested internally
+        colour_grad = any(ctx.needs_input_grad[3 + i] for i in range(S + n_src))
         # single source, no pose gradient: the per-scale kernel gathers from a pixel-packed (B,H,W,4) copy of the
         # source (one 128-bit load per bilinear tap), written once by the identity-loss kernel
         packed = n_src == 1 and not need_T and not no_ssim and H * W < (1 << 28)
@@ -554,7 +557,8 @@ class _Objective(torch.autograd.Function):
                       and H * W < (1 << 27))
         parts = [torch.empty(B * tiles, device=dev, dtype=torch.float32) for _ in range(S)]
         G = [torch.empty(B, 1, H, W, device=dev, dtype=torch.float32) for _ in range(S)]
-        sels = [torch.empty(B, H, W, device=dev, dtype=torch.uint8) if want_sel else None for _ in range(S)]
+        want_sels = want_sel or colour_grad
+        sels = [torch.empty(B, H, W, device=dev, dtype=torch.uint8) if want_sels else None for _ in range(S)]
         if multisrc and need_T:
             tiles32 = ((H + 31) // 32) * ((W + 31) // 32)
             # one buffer for the pose-gradient partials of every scale: the backward reduces it with one einsum
@@ -573,7 +577,7 @@ class _Objective(torch.autograd.Function):
                                                 ptr_array(noises) if has_noise else None, B, H, W, min_depth, max_depth,
                                                 inv_den, ptr(mf_ws), ptr_array(parts), ptr_array(G),
                                                 ptr_array(gPs) if need_T else None,
-                                                ptr_array(sels) if want_sel else None, stream()), "photo_multisource")
+                                                ptr_array(sels) if want_sels else None, stream()), "photo_multisource")
         if multiscale:
             # ONE launch for all scales (csrc/photo_ms.cu): the scale loop of generate_images_pred / compute_losses
             # runs inside the kernel; same bits as the per-scale launches below
@@ -581,7 +585,7 @@ class _Objective(torch.autograd.Function):
                 check(lib.dmh_photo_multiscale(ptr(target), ptr(src_pk), ptr(Ts[0]), S, ptr_array(disps), dh_, dw_, ptr(k),
                                                ptr(ik), ptr(ident), ptr_array(noises) if has_noise else None, B, H, W,
                                                min_depth, max_depth, inv_den, ptr_array(parts), ptr_array(G),
-                                               ptr_array(sels) if want_sel else None, stream()), "photo_multiscale")
+                                               ptr_array(sels) if want_sels else None, stream()), "photo_multiscale")
         alt = _side_stream(dev, 1)
         alt.wait_stream(cur)
         for s in range(S if not (multiscale or multisrc) else 0):
@@ -605,7 +609,17 @@ class _Objective(torch.autograd.Function):
         if multisrc and need_T:
             gPs = [gP_all]                                   # (S, F, B, tiles, 12) as ONE saved tensor
         ctx.gp_stacked = bool(multisrc and need_T)
-        ctx.save_for_backward(img_scalars, k, *G, *gN, *[t for t in Ts], *[g for g in gPs if g is not None])
+        gPs = [g for g in gPs if g is not None]
+        ctx.n_gP = len(gPs)
+        ctx.colour = None
+        colour_saved = []
+        if colour_grad:
+            # the frames as the kernels read them (fp32; a bf16 source is widened in the backward), the disparities
+            # and the selections
+            ctx.colour = (float(min_depth), float(max_depth), flags & (FLAG_NO_SSIM | FLAG_AVG_REPROJECTION),
+                          bool(automask), [c.dtype for c in colors_in], [t.dtype for t in srcs_in])
+            colour_saved = [ik, *colors, *srcs, *disps, *sels]
+        ctx.save_for_backward(img_scalars, k, *G, *gN, *[t for t in Ts], *gPs, *colour_saved)
         out_sels = tuple(sels) if want_sel else ()
         for t in out_sels:
             ctx.mark_non_differentiable(t)
@@ -619,7 +633,7 @@ class _Objective(torch.autograd.Function):
         G = saved[2:2 + S]
         gN = saved[2 + S:2 + 2 * S]
         Ts = saved[2 + 2 * S:2 + 2 * S + n_src]
-        gPs = saved[2 + 2 * S + n_src:]
+        gPs = saved[2 + 2 * S + n_src:2 + 2 * S + n_src + ctx.n_gP]
         lib = _lib_()
         gt = f32c(g_total).reshape(1) if g_total is not None else None
         gs = f32c(g_scales) if g_scales is not None else None
@@ -660,8 +674,59 @@ class _Objective(torch.autograd.Function):
             for f in range(n_src):
                 if ctx.needs_input_grad[base + f]:
                     g_T[f] = _pose_grad_T(gPs, u, f, k, Ts[f])
-        return (None, None, None) + (None,) * S + (None,) * n_src + tuple(g_T) + tuple(grads_disp) + \
+        g_col, g_src = [None] * S, [None] * n_src
+        if ctx.colour is not None:
+            g_col, g_src = _Objective._colour_grads(ctx, saved[2 + 2 * S + n_src + ctx.n_gP:], img_scalars, k, Ts, gt,
+                                                    gs)
+        return (None, None, None) + tuple(g_col) + tuple(g_src) + tuple(g_T) + tuple(grads_disp) + \
             ((None,) * S if has_noise else ())
+
+    @staticmethod
+    def _colour_grads(ctx, saved, img_scalars, k, Ts, gt, gs):
+        """d(loss)/d(colour(0, s)) and d(loss)/d(source f) for the inputs that require them (None for the rest):
+        the identity candidates' terms (one launch, initialises the target and source gradients), the reprojection
+        terms (one launch per scale) and the smoothness terms (one launch per scale; scale 0 adds into the target's).
+        Computed on the fp32 frames; returned in each input's dtype."""
+        S, n_src, B, H, W, smooth_w = ctx.cfg[:6]
+        min_depth, max_depth, flags, automask, col_dtypes, src_dtypes = ctx.colour
+        ik = saved[0]
+        colors = [f32c(c) for c in saved[1:1 + S]]
+        srcs = [f32c(t) for t in saved[1 + S:1 + S + n_src]]
+        disps = saved[1 + S + n_src:1 + 2 * S + n_src]
+        sels = saved[1 + 2 * S + n_src:1 + 3 * S + n_src]
+        need_col = [bool(ctx.needs_input_grad[3 + s]) for s in range(S)]
+        need_src = [bool(ctx.needs_input_grad[3 + S + f]) for f in range(n_src)]
+        lib = _lib_()
+        g_col = [None] * S
+        g_src = [torch.empty_like(srcs[f]) if need_src[f] else None for f in range(n_src)]
+        if need_col[0]:
+            g_col[0] = torch.empty_like(colors[0])
+        if need_col[0] or any(need_src):
+            src_arr, gsrc_arr = ptr_array(srcs), ptr_array(g_src)
+            with _timed("identity_image_grad"):
+                check(lib.dmh_identity_image_grad(ptr(colors[0]), src_arr, n_src, ptr_array(sels), S, ptr(gt), ptr(gs),
+                                                  B, H, W, flags, int(automask), ptr(g_col[0]), gsrc_arr, stream()),
+                      "identity_image_grad")
+            T_arr = ptr_array(Ts)
+            for s in range(S):
+                d = disps[s]
+                with _timed("photo_image_grad"):
+                    check(lib.dmh_photo_image_grad(ptr(colors[0]), src_arr, T_arr, n_src, ptr(d), d.shape[2], d.shape[3],
+                                                   ptr(k), ptr(ik), ptr(sels[s]), s, S, ptr(gt), ptr(gs), B, H, W,
+                                                   min_depth, max_depth, flags, int(automask), ptr(g_col[0]), gsrc_arr,
+                                                   stream()), "photo_image_grad")
+        for s in range(S):
+            if not need_col[s]:
+                continue
+            d = disps[s]
+            if s > 0:
+                g_col[s] = torch.empty_like(colors[s])
+            check(lib.dmh_smooth_image_grad(ptr(d), ptr(colors[s]), B, d.shape[2], d.shape[3], ptr(img_scalars[s]),
+                                            smooth_w[s], s, S, ptr(gt), ptr(gs), int(s == 0), ptr(g_col[s]), stream()),
+                  "smooth_image_grad")
+        g_col = [g if g is None or g.dtype == dt else g.to(dt) for g, dt in zip(g_col, col_dtypes)]
+        g_src = [g if g is None or g.dtype == dt else g.to(dt) for g, dt in zip(g_src, src_dtypes)]
+        return g_col, g_src
 
 
 def objective(colors0, srcs, Ts, disps, K, inv_K, noises=None, min_depth=0.1, max_depth=100.0, no_ssim=False,

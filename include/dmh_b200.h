@@ -263,6 +263,31 @@ int dmh_disp_grad(const float* G_full, const float* gN, const float* img_scalars
                   const float* g_total, const float* g_scale, const float* g_smooth, float inv_S, int B, int h, int w,
                   int H, int W, float* grad_disp, dmh_stream_t stream);
 
+/* -- colour-frame gradients of the fused objective (backward of ops.objective w.r.t. the frames) ----------------
+ * Recomputed from the frames, the disparities and the forward's selections sel_s (B,H,W) (argmin in cat order, as
+ * dmh_photo_scale / dmh_photo_multiscale / dmh_photo_multisource emit it).  Upstream weight of scale s:
+ * u_s = *g_total / S + g_scales[s] (device scalars, either nullable), read on the device.  flags: DMH_PHOTO_NO_SSIM,
+ * DMH_PHOTO_AVG_REPROJECTION; automask: identity candidates present.  grad_target (B,3,H,W) and grad_src_host[f]
+ * (B,3,H,W) are nullable (that frame's gradient is not computed).
+ * dmh_identity_image_grad: ONE launch for all S scales: the identity candidates' terms (un-warped source f vs
+ *   target, gated by sum_s u_s [sel_s picked f's identity]).  INITIALISES grad_target and every grad_src[f].
+ * dmh_photo_image_grad: one launch per scale `scale`: the reprojection candidates' terms; ADDS into grad_target and
+ *   (atomically: the last bits depend on the order) into grad_src[f] through the bilinear taps of the warp.
+ * dmh_smooth_image_grad: u_s * smooth_weight * d(smoothness of scale s)/d(img) for img = colour(0, s) (B,3,h,w),
+ *   disp (B,1,h,w), img_scalars the (B,2) slice of dmh_objective_finish for scale s; accumulate: add into grad_img
+ *   instead of writing it.                                                                                         */
+int dmh_identity_image_grad(const float* target, const float* const* src_host, int F, const uint8_t* const* sel_host,
+                            int S, const float* g_total, const float* g_scales, int B, int H, int W, int flags,
+                            int automask, float* grad_target, float* const* grad_src_host, dmh_stream_t stream);
+int dmh_photo_image_grad(const float* target, const float* const* src_host, const float* const* T_host, int F,
+                         const float* disp, int disp_h, int disp_w, const float* K, const float* inv_K,
+                         const uint8_t* sel, int scale, int S, const float* g_total, const float* g_scales, int B,
+                         int H, int W, float min_depth, float max_depth, int flags, int automask, float* grad_target,
+                         float* const* grad_src_host, dmh_stream_t stream);
+int dmh_smooth_image_grad(const float* disp, const float* img, int B, int h, int w, const float* img_scalars,
+                          float smooth_weight, int scale, int S, const float* g_total, const float* g_scales,
+                          int accumulate, float* grad_img, dmh_stream_t stream);
+
 /* ======================= stage 1: physical patch attack ======================= */
 
 /* -- A2+A3 PhysicalTrans.project / project_w_trans (physicalTrans.py:130-196):

@@ -1,0 +1,101 @@
+#!/usr/bin/env python
+"""Forward + backward of the fused objective with and without the colour-frame gradients (CUDA events), and the
+kernel times of the colour-gradient launches, for BASELINE config 2 (B=32, 1024x320, [0,'s'], 4 scales) and
+mono+stereo (B=32, 1024x320, [0,-1,1,'s'], pose gradients).  Prints the card and its power limit with the numbers.
+usage: python profiles/image_grad_timing.py [--iters 20] [--batch 32]"""
+import argparse
+import os
+import subprocess
+import sys
+
+import torch
+
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+from depthmodelhardening_b200 import objective, ops, synth  # noqa: E402
+
+
+def card():
+    try:
+        q = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError):
+        q = "nvidia-smi unavailable"
+    return "%s | %s" % (torch.cuda.get_device_name(0), q)
+
+
+def bytes_per_px(F, S):
+    """Algorithmic bytes per target pixel of the colour-gradient launches (fp32): S reprojection launches and one
+    identity launch.  Per scale: read 12 target + 12 F gathered sources + <= 4 disparity + 1 sel, write 24 target
+    read-modify-write + 12 F source RED; identity: read 12 + 12 F + S sel, write 12 + 12 F."""
+    return S * (12 + 12 * F + 4 + 1 + 24 + 12 * F), (12 + 12 * F + S) + (12 + 12 * F)
+
+
+def run_case(name, frame_ids, B, H, W, iters, dev):
+    pb = synth.photo_batch(batch=B, height=H, width=W, frame_ids=frame_ids, seed=5).to(dev)
+    F = len(frame_ids) - 1
+    S = len(pb.scales)
+
+    def make(colour):
+        colors = {k: v.clone().requires_grad_(colour) for k, v in pb.color.items()}
+        disps = {s: v.clone().requires_grad_(True) for s, v in pb.disp.items()}
+        Ts = {k: v.clone().requires_grad_(k != "s") for k, v in pb.T.items()}
+
+        def step():
+            losses, _ = objective.photometric_losses(colors, disps, pb.K, pb.inv_K, Ts, pb.frame_ids, pb.scales, H, W,
+                                                     noise=pb.noise)
+            losses["loss"].backward()
+        return step
+
+    def timed(step):
+        for _ in range(3):
+            step()
+        torch.cuda.synchronize()
+        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        a.record()
+        for _ in range(iters):
+            step()
+        b.record()
+        torch.cuda.synchronize()
+        return a.elapsed_time(b) / iters
+
+    base, with_c = make(False), make(True)
+    t0 = timed(base)
+    t1 = timed(with_c)
+    t0b = timed(base)                              # alternate: the spread of the baseline shows in t0 vs t0b
+    ops.KERNEL_EVENTS = []
+    for _ in range(iters):
+        with_c()
+    torch.cuda.synchronize()
+    per = {}
+    for n, a, b in ops.KERNEL_EVENTS:
+        if n in ("identity_image_grad", "photo_image_grad"):
+            per.setdefault(n, []).append(a.elapsed_time(b))
+    ops.KERNEL_EVENTS = None
+    print("%s: B=%d %dx%d frames=%s scales=%d" % (name, B, W, H, list(frame_ids), S))
+    print("  fwd+bwd without colour grads  %.3f ms / %.3f ms (two runs)" % (t0, t0b))
+    print("  fwd+bwd with colour grads     %.3f ms" % t1)
+    npx = B * H * W
+    per_scale_b, ident_b = bytes_per_px(F, S)
+    for n, ts in sorted(per.items()):
+        ts = sorted(ts)
+        med = ts[len(ts) // 2]
+        nbytes = (per_scale_b / S if n == "photo_image_grad" else ident_b) * npx
+        print("  %-20s median %.3f ms per launch (%d launches), %.0f B/px algorithmic -> %.2f TB/s" % (
+            n, med, len(ts), nbytes / npx, nbytes / med / 1e9))
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--iters", type=int, default=20)
+    ap.add_argument("--batch", type=int, default=32)
+    a = ap.parse_args()
+    if not torch.cuda.is_available():
+        raise SystemExit("image_grad_timing.py needs a CUDA device")
+    dev = torch.device("cuda:0")
+    print(card())
+    run_case("config 2", (0, "s"), a.batch, 320, 1024, a.iters, dev)
+    run_case("mono+stereo", (0, -1, 1, "s"), a.batch, 320, 1024, a.iters, dev)
+
+
+if __name__ == "__main__":
+    main()
