@@ -80,6 +80,8 @@ SIGNATURES = {
     "dmh_photo_image_grad": (_i, [_f, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), _i, _f, _i, _i, _f, _f, _f, _i, _i,
                                   _f, _f, _i, _i, _i, _fl, _fl, _i, _i, _f, C.POINTER(C.c_void_p), _st]),
     "dmh_smooth_image_grad": (_i, [_f, _f, _i, _i, _i, _f, _fl, _i, _i, _f, _f, _i, _f, _st]),
+    "dmh_photo_image_grad_dh": (_i, [_f, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), _i, _f, _i, _i, _f, _f, _f, _f,
+                                     _i, _i, _i, _fl, _fl, _i, _f, C.POINTER(C.c_void_p), _st]),
     "dmh_compose_u8": (_i, [_f, _f, _f, _f, _i, _i, _i, _i, _f, _st]),
     "dmh_compose_patch_u8": (_i, [_f, _f, _f, _f, _f, _f, _f, _f, _i, _i, _i, _i, _i, _f, _f, _f, _st]),
     "dmh_lanczos_u8": (_i, [_f, _i, _i, _i, _i, _i, _f, _f, _i, _f, _f, _i, _f, _f, _f, _st]),

@@ -315,6 +315,14 @@ DMH_HD float reproj_gate(int sel, int f, int n_ident, int F, bool avg) {
     if (avg) return sel == n_ident ? 1.0f / (float)F : 0.0f;
     return sel == n_ident + f ? 1.0f : 0.0f;
 }
+// Depth-hints objective: `sel` = argmin over [reprojection, identity, hint] in bits 0-1 and the source frame whose
+// reprojection is the minimum over the frames in bits 2-3 (dmh_photo_scale_dh with DMH_PHOTO_SEL_SOURCE).  The
+// reprojection term counts wherever the identity did not win; it is the mean over the frames under avg_reprojection.
+DMH_HD float reproj_gate_dh(int sel, int f, int F, bool avg) {
+    if ((sel & 3) == 1) return 0.0f;
+    if (avg) return 1.0f / (float)F;
+    return (sel >> 2) == f ? 1.0f : 0.0f;
+}
 DMH_HD float ident_gate(int sel, int f, int n_ident, int F, bool avg) {
     if (n_ident == 0) return 0.0f;
     if (avg) return sel == 0 ? 1.0f / (float)F : 0.0f;

@@ -12,9 +12,14 @@
 //                            grad_target in place (each pixel is owned by one thread; launches run in stream order:
 //                            deterministic) and scattered into grad_src[f] through the bilinear taps by RED
 //                            (warp-aggregated, as dmh_warp_bwd).
+//   dmh_photo_image_grad_dh  the same kernel for the depth-hints objective (depth_hints.py): the reprojection term
+//                            counts wherever the identity did not win the argmin over [reprojection, identity,
+//                            hint] and goes to the forward's first-minimum source frame (or 1/F to each under
+//                            avg_reprojection); the identity and hint candidates carry no gradient there.
 //   dmh_smooth_image_grad    u_s * w_s * d(edge-aware smoothness)/d(colour(0, s)); scale 0 adds into grad_target.
 //
-// u_s = g_total / S + g_scale[s] is read on the device: no host synchronisation, CUDA-graph capturable.
+// u_s = g_total / S + g_scale[s] (depth hints: the masked mean's u_r[s]) is read on the device: no host
+// synchronisation, CUDA-graph capturable.
 //
 // Algorithmic bytes per target pixel (fp32, F source frames, S scales):
 //   dmh_photo_image_grad     read 12 (target) + 12 F (gathered sources) + <= 4 (disparity) + 1 (sel);
@@ -238,11 +243,14 @@ struct ReprojGradParams {
     int B, H, W, F, n_ident, flags;
     DepthScale ds;
     float rcw, rch;              // 1/(W-1), 1/(H-1) for the verified 3-instruction division
+    const float* u_dh;           // depth-hints mode: device scalar, the reprojection term's upstream weight of this scale
 };
 
 size_t reproj_smem_bytes() { return sizeof(float) * ((size_t)7 * IG_R2 + 13 * IG_R1 + IG_MAXF * 24); }
 
-template <bool FASTDIV>
+// DH: the depth-hints objective (sel from dmh_photo_scale_dh with DMH_PHOTO_SEL_SOURCE, gate reproj_gate_dh, upstream
+// weight *u_dh); otherwise monodepth2's (reproj_gate, upstream(...) * inv_den)
+template <bool FASTDIV, bool DH>
 __global__ void __launch_bounds__(IG_THREADS)
 reproj_grad_kernel(const ReprojGradParams p) {
     extern __shared__ float smem[];
@@ -281,7 +289,7 @@ reproj_grad_kernel(const ReprojGradParams p) {
             cams[f * 24 + t] = __ldg(p.inv_K + b * 16 + i * 4 + j);
         }
     }
-    if (tid == 0) s_u = upstream(p.g_total, p.g_scale, p.inv_S) * p.inv_den;
+    if (tid == 0) s_u = DH ? __ldg(p.u_dh) : upstream(p.g_total, p.g_scale, p.inv_S) * p.inv_den;
     for (int i = tid; i < IG_R2; i += IG_THREADS) {
         const int r = i / IG_R2W, c = i % IG_R2W;
         const int iy = ext_to_img(y0 - 2 + r, H), ix = ext_to_img(x0 - 2 + c, W);
@@ -299,8 +307,10 @@ reproj_grad_kernel(const ReprojGradParams p) {
         for (int i = tid; i < IG_R1; i += IG_THREADS) {
             const int qy = y0 - 1 + i / IG_R1W, qx = x0 - 1 + i % IG_R1W;
             float g = 0.f;
-            if (qy >= 0 && qy < H && qx >= 0 && qx < W)
-                g = u * reproj_gate(p.sel[(size_t)b * N + (size_t)qy * W + qx], f, p.n_ident, p.F, avg);
+            if (qy >= 0 && qy < H && qx >= 0 && qx < W) {
+                const int sel = p.sel[(size_t)b * N + (size_t)qy * W + qx];
+                g = u * (DH ? reproj_gate_dh(sel, f, p.F, avg) : reproj_gate(sel, f, p.n_ident, p.F, avg));
+            }
             gate[i] = g;
             any |= g != 0.f;
         }
@@ -431,6 +441,45 @@ smooth_img_grad_kernel(const float* __restrict__ disp, const float* __restrict__
     }
 }
 
+// dmh_photo_image_grad (DH = false) and dmh_photo_image_grad_dh: the argument checks and the launch shared by both.
+// p arrives with the upstream weight of its mode filled in; `name` is the public entry point, for the errors.
+template <bool DH>
+int reproj_grad_launch(const char* name, ReprojGradParams& p, const float* target, const float* const* src_host,
+                       const float* const* T_host, int F, const float* disp, int disp_h, int disp_w, const float* K,
+                       const float* inv_K, const uint8_t* sel, int B, int H, int W, float min_depth, float max_depth,
+                       int flags, float* grad_target, float* const* grad_src_host, cudaStream_t st) {
+    DMH_REQUIRE(target && src_host && T_host && disp && K && inv_K && sel && grad_src_host, "%s: null pointer", name);
+    DMH_REQUIRE(F >= 1 && F <= IG_MAXF, "%s: F=%d outside [1,%d]", name, F, IG_MAXF);
+    DMH_REQUIRE(B > 0 && B <= 65535 && H >= 2 && W >= 2, "%s: bad shape B=%d H=%d W=%d", name, B, H, W);
+    DMH_REQUIRE(disp_h >= 1 && disp_w >= 1 && disp_h <= H && disp_w <= W, "%s: bad disparity size %dx%d", name, disp_h,
+                disp_w);
+    DMH_REQUIRE(min_depth > 0.f && max_depth > min_depth, "%s: bad depth range", name);
+    p.target = target;
+    for (int f = 0; f < F; ++f) {
+        DMH_REQUIRE(src_host[f] && T_host[f], "%s: null src/T for frame %d", name, f);
+        p.src[f] = src_host[f];
+        p.T[f] = T_host[f];
+        p.grad_src[f] = grad_src_host[f];
+    }
+    p.disp.ptr = disp; p.disp.h = disp_h; p.disp.w = disp_w;
+    p.disp.sh = (float)disp_h / (float)H; p.disp.sw = (float)disp_w / (float)W;
+    p.K = K; p.inv_K = inv_K; p.sel = sel;
+    p.grad_target = grad_target;
+    p.B = B; p.H = H; p.W = W; p.F = F; p.flags = flags;
+    p.ds = depth_scale(min_depth, max_depth, false);
+    // the division rule of the forward kernels: bit-identical either way, the verified one is shorter
+    const bool fastdiv = const_div_exact(W - 1, &p.rcw, st) && const_div_exact(H - 1, &p.rch, st);
+    const size_t smem = reproj_smem_bytes();
+    static KernelSetup setup;
+    const void* kernels[2] = {(const void*)reproj_grad_kernel<false, DH>, (const void*)reproj_grad_kernel<true, DH>};
+    if (setup.sms(name, kernels, 2, smem) == 0) return DMH_ERR_CUDA;
+    const dim3 grid(ceil_div(W, IG_TW), ceil_div(H, IG_TH), B);
+    void (*kernel)(const ReprojGradParams) = fastdiv ? reproj_grad_kernel<true, DH> : reproj_grad_kernel<false, DH>;
+    DMH_LAUNCH(kernel, grid, IG_THREADS, smem, st)(p);
+    DMH_CHECK_LAUNCH(name);
+    return DMH_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -475,44 +524,28 @@ int dmh_photo_image_grad(const float* target, const float* const* src_host, cons
                          const uint8_t* sel, int scale, int S, const float* g_total, const float* g_scales, int B,
                          int H, int W, float min_depth, float max_depth, int flags, int automask, float* grad_target,
                          float* const* grad_src_host, dmh_stream_t stream) {
-    DMH_REQUIRE(target && src_host && T_host && disp && K && inv_K && sel && grad_src_host && (g_total || g_scales),
-                "dmh_photo_image_grad: null pointer");
-    DMH_REQUIRE(F >= 1 && F <= IG_MAXF, "dmh_photo_image_grad: F=%d outside [1,%d]", F, IG_MAXF);
+    DMH_REQUIRE(g_total || g_scales, "dmh_photo_image_grad: null pointer");
     DMH_REQUIRE(S >= 1 && scale >= 0 && scale < S, "dmh_photo_image_grad: scale %d of %d", scale, S);
-    DMH_REQUIRE(B > 0 && B <= 65535 && H >= 2 && W >= 2, "dmh_photo_image_grad: bad shape B=%d H=%d W=%d", B, H, W);
-    DMH_REQUIRE(disp_h >= 1 && disp_w >= 1 && disp_h <= H && disp_w <= W, "dmh_photo_image_grad: bad disparity size "
-                "%dx%d", disp_h, disp_w);
-    DMH_REQUIRE(min_depth > 0.f && max_depth > min_depth, "dmh_photo_image_grad: bad depth range");
     ReprojGradParams p = {};
-    p.target = target;
-    for (int f = 0; f < F; ++f) {
-        DMH_REQUIRE(src_host[f] && T_host[f], "dmh_photo_image_grad: null src/T for frame %d", f);
-        p.src[f] = src_host[f];
-        p.T[f] = T_host[f];
-        p.grad_src[f] = grad_src_host[f];
-    }
-    p.disp.ptr = disp; p.disp.h = disp_h; p.disp.w = disp_w;
-    p.disp.sh = (float)disp_h / (float)H; p.disp.sw = (float)disp_w / (float)W;
-    p.K = K; p.inv_K = inv_K; p.sel = sel;
     p.g_total = g_total; p.g_scale = g_scales ? g_scales + scale : nullptr;
     p.inv_S = 1.0f / (float)S;
     p.inv_den = (float)(1.0 / ((double)B * H * W));
-    p.grad_target = grad_target;
-    p.B = B; p.H = H; p.W = W; p.F = F; p.flags = flags;
     p.n_ident = automask ? ((flags & DMH_PHOTO_AVG_REPROJECTION) ? 1 : F) : 0;
-    p.ds = depth_scale(min_depth, max_depth, false);
-    cudaStream_t st = (cudaStream_t)stream;
-    // the division rule of the forward kernels: bit-identical either way, the verified one is shorter
-    const bool fastdiv = const_div_exact(W - 1, &p.rcw, st) && const_div_exact(H - 1, &p.rch, st);
-    const size_t smem = reproj_smem_bytes();
-    static KernelSetup setup;
-    const void* kernels[2] = {(const void*)reproj_grad_kernel<false>, (const void*)reproj_grad_kernel<true>};
-    if (setup.sms("dmh_photo_image_grad", kernels, 2, smem) == 0) return DMH_ERR_CUDA;
-    const dim3 grid(ceil_div(W, IG_TW), ceil_div(H, IG_TH), B);
-    if (fastdiv) DMH_LAUNCH(reproj_grad_kernel<true>, grid, IG_THREADS, smem, st)(p);
-    else DMH_LAUNCH(reproj_grad_kernel<false>, grid, IG_THREADS, smem, st)(p);
-    DMH_CHECK_LAUNCH("dmh_photo_image_grad");
-    return DMH_OK;
+    return reproj_grad_launch<false>("dmh_photo_image_grad", p, target, src_host, T_host, F, disp, disp_h, disp_w, K,
+                                     inv_K, sel, B, H, W, min_depth, max_depth, flags, grad_target, grad_src_host,
+                                     (cudaStream_t)stream);
+}
+
+int dmh_photo_image_grad_dh(const float* target, const float* const* src_host, const float* const* T_host, int F,
+                            const float* disp, int disp_h, int disp_w, const float* K, const float* inv_K,
+                            const uint8_t* sel, const float* u, int B, int H, int W, float min_depth, float max_depth,
+                            int flags, float* grad_target, float* const* grad_src_host, dmh_stream_t stream) {
+    DMH_REQUIRE(u, "dmh_photo_image_grad_dh: null pointer");
+    ReprojGradParams p = {};
+    p.u_dh = u;
+    return reproj_grad_launch<true>("dmh_photo_image_grad_dh", p, target, src_host, T_host, F, disp, disp_h, disp_w, K,
+                                    inv_K, sel, B, H, W, min_depth, max_depth, flags, grad_target, grad_src_host,
+                                    (cudaStream_t)stream);
 }
 
 int dmh_smooth_image_grad(const float* disp, const float* img, int B, int h, int w, const float* img_scalars,

@@ -92,6 +92,7 @@ photo_scale_kernel(const PhotoParams p) {
     const bool no_ssim = (p.flags & DMH_PHOTO_NO_SSIM) != 0;
     const bool avg = (p.flags & DMH_PHOTO_AVG_REPROJECTION) != 0;
     const bool is_depth = (p.flags & DMH_PHOTO_INPUT_IS_DEPTH) != 0;
+    const bool sel_src = (p.flags & DMH_PHOTO_SEL_SOURCE) != 0;
     const float w_ssim = no_ssim ? 0.0f : 0.85f / 3.0f;
     const float w_l1 = no_ssim ? 1.0f / 3.0f : 0.15f / 3.0f;
 
@@ -237,7 +238,9 @@ photo_scale_kernel(const PhotoParams p) {
                         const float gd = m_h * va * sg / a1;
                         p.grad_hint[(size_t)b * N + qo] = is_depth ? gd : gd * ddepth_ddisp(depth, p.ds);
                     }
-                    if (p.sel) p.sel[(size_t)b * N + qo] = (uint8_t)idx;
+                    // DMH_PHOTO_SEL_SOURCE: also the winning source, the decision the colour-gradient backward
+                    // (dmh_photo_image_grad_dh) routes the reprojection gradient by
+                    if (p.sel) p.sel[(size_t)b * N + qo] = (uint8_t)(sel_src ? idx | (fb << 2) : idx);
                 }
             } else {
             // candidates in the reference's cat order: identity first, then reprojection

@@ -148,15 +148,18 @@ def _prologue(colors, Ts, frame_ids, height, width, depth_hint, depth_hint_mask,
     with torch.no_grad():
         if not disable_automasking:
             ident = torch.empty(B, len(srcs), height, width, device=target.device, dtype=torch.float32)
+        # widened frames (a copy for non-fp32 frames) held until the launch: a copy made inside the call's argument
+        # list is freed as soon as its pointer is taken, and the next copy may then reuse its memory
+        target32, srcs32 = f32c(target), [f32c(s) for s in srcs]
         if pack_out is not None and len(srcs) == 1 and not no_ssim:
             # single source: the identity-loss kernel also writes the pixel-packed copy the fast kernel gathers from
             pk = torch.empty(B, height, width, 4, device=target.device, dtype=torch.float32)
-            check(_lib_().dmh_identity_loss_pack(ptr(f32c(target)), ptr(f32c(srcs[0])), B, height, width, 0, ptr(ident),
+            check(_lib_().dmh_identity_loss_pack(ptr(target32), ptr(srcs32[0]), B, height, width, 0, ptr(ident),
                                                  ptr(pk), stream()), "identity_loss_pack")
             pack_out.append(pk)
         elif ident is not None:
-            check(_lib_().dmh_identity_loss(ptr(f32c(target)), ptr_array([f32c(s) for s in srcs]), len(srcs), B, height,
-                                            width, int(no_ssim), ptr(ident), stream()), "identity_loss")
+            check(_lib_().dmh_identity_loss(ptr(target32), ptr_array(srcs32), len(srcs), B, height, width,
+                                            int(no_ssim), ptr(ident), stream()), "identity_loss")
     return srcs_ids, srcs, target, B, hint_rl, hint_pred, ident
 
 
@@ -167,8 +170,10 @@ class _ObjectiveDH(torch.autograd.Function):
     def forward(ctx, K, inv_K, cfg, ident, hint_rl, hint_depth, hint_valid, *tensors):
         (min_depth, max_depth, flags, smooth_w, want_sel, n_src, S, has_noise, src_pk) = cfg
         it = iter(tensors)
-        colors = [f32c(next(it)) for _ in range(S)]
-        srcs = [f32c(next(it)) for _ in range(n_src)]
+        colors_in = [next(it) for _ in range(S)]
+        srcs_in = [next(it) for _ in range(n_src)]
+        colors = [f32c(c) for c in colors_in]
+        srcs = [f32c(t) for t in srcs_in]
         Ts = [f32c(next(it)) for _ in range(n_src)]
         disps = [f32c(next(it)) for _ in range(S)]
         noises = [f32c(next(it)) for _ in range(S)] if has_noise else [None] * S
@@ -184,6 +189,12 @@ class _ObjectiveDH(torch.autograd.Function):
         hv = f32c(hint_valid) if hr is not None else None
         base = 7 + S + n_src
         need_T = any(ctx.needs_input_grad[base + i] for i in range(n_src))
+        # gradients for the colour frames (target, pyramid, sources): the backward recomputes them from the frames,
+        # the disparities and every scale's selection, so `sel` is requested internally -- with the winning source
+        # frame in its upper bits where several sources compete for the minimum
+        colour_grad = any(ctx.needs_input_grad[7 + i] for i in range(S + n_src))
+        sel_src = colour_grad and n_src > 1 and not (flags & ops.FLAG_AVG_REPROJECTION)
+        want_sels = want_sel or colour_grad
         tiles = lib.dmh_photo_tiles(H, W)
         nblk = B * tiles
         src_arr, T_arr = ptr_array(srcs), ptr_array(Ts)
@@ -198,10 +209,11 @@ class _ObjectiveDH(torch.autograd.Function):
             g_r = torch.empty(B, 1, H, W, device=dev, dtype=torch.float32)
             g_h = torch.empty(B, 1, H, W, device=dev, dtype=torch.float32) if hr is not None else None
             gP = torch.empty(n_src, B, tiles, 12, device=dev, dtype=torch.float32) if need_T else None
-            sel = torch.empty(B, H, W, device=dev, dtype=torch.uint8) if want_sel else None
+            sel = torch.empty(B, H, W, device=dev, dtype=torch.uint8) if want_sels else None
             check(lib.dmh_photo_scale_dh(ptr(target), src_arr, T_arr, n_src, ptr(d), h, w, ptr(k), ptr(ik), ptr(idn),
-                                         ptr(noises[s]), ptr(hr), ptr(hd), ptr(hv), B, H, W, min_depth, max_depth, flags,
-                                         ptr(part), ptr(g_r), ptr(g_h), ptr(gP), ptr(sel), stream()), "photo_scale_dh")
+                                         ptr(noises[s]), ptr(hr), ptr(hd), ptr(hv), B, H, W, min_depth, max_depth,
+                                         flags | (ops.FLAG_SEL_SOURCE if sel_src else 0), ptr(part), ptr(g_r), ptr(g_h),
+                                         ptr(gP), ptr(sel), stream()), "photo_scale_dh")
             sm = torch.empty(4, device=dev, dtype=torch.float32)
             check(lib.dmh_reduce_rows(ptr(part), 4 if hr is not None else 2, nblk, 1.0, ptr(sm), stream()), "reduce_rows")
             ws = torch.empty(lib.dmh_smooth_fused_workspace_floats(B, h, w), device=dev, dtype=torch.float32)
@@ -233,9 +245,18 @@ class _ObjectiveDH(torch.autograd.Function):
         total = per_scale.sum() / S
         ctx.cfg = (S, n_src, B, H, W, tuple(float(x) for x in smooth_w), need_T, [tuple(d.shape) for d in disps],
                    has_noise, hr is not None)
-        ctx.save_for_backward(img_scalars, k, inv_r, inv_h, *G_r, *[g for g in G_h if g is not None], *gN, *Ts,
-                              *[g for g in gPs if g is not None])
-        out_sels = tuple(sels) if want_sel else ()
+        gPs = [g for g in gPs if g is not None]
+        ctx.n_gP = len(gPs)
+        ctx.colour = None
+        colour_saved = []
+        if colour_grad:
+            ctx.colour = (float(min_depth), float(max_depth), flags & (ops.FLAG_NO_SSIM | ops.FLAG_AVG_REPROJECTION),
+                          [c.dtype for c in colors_in], [t.dtype for t in srcs_in])
+            colour_saved = [ik, *colors, *srcs, *disps, *sels]
+        ctx.save_for_backward(img_scalars, k, inv_r, inv_h, *G_r, *[g for g in G_h if g is not None], *gN, *Ts, *gPs,
+                              *colour_saved)
+        # the argmin index over [reprojection, identity, hint], as without the source bits
+        out_sels = tuple(t & 3 if sel_src else t for t in sels) if want_sel else ()
         for t in out_sels:
             ctx.mark_non_differentiable(t)
         return (total, per_scale, loss_r, loss_h) + out_sels
@@ -251,7 +272,7 @@ class _ObjectiveDH(torch.autograd.Function):
         pos += S if hints else 0
         gN = saved[pos:pos + S]; pos += S
         Ts = saved[pos:pos + n_src]; pos += n_src
-        gPs = saved[pos:]
+        gPs = saved[pos:pos + ctx.n_gP]; pos += ctx.n_gP
         lib = _lib_()
         dev = G_r[0].device
         zero = torch.zeros((), device=dev)
@@ -285,8 +306,55 @@ class _ObjectiveDH(torch.autograd.Function):
             for f in range(n_src):
                 if ctx.needs_input_grad[base + f]:
                     g_T[f] = ops._pose_grad_T(gPs, u_r, f, k, Ts[f])
-        return (None,) * 7 + (None,) * S + (None,) * n_src + tuple(g_T) + tuple(grads_disp) + \
+        g_col, g_src = [None] * S, [None] * n_src
+        if ctx.colour is not None:
+            g_col, g_src = _ObjectiveDH._colour_grads(ctx, saved[pos:], img_scalars, k, Ts, u_all, u_r)
+        return (None,) * 7 + tuple(g_col) + tuple(g_src) + tuple(g_T) + tuple(grads_disp) + \
             ((None,) * S if has_noise else ())
+
+    @staticmethod
+    def _colour_grads(ctx, saved, img_scalars, k, Ts, u_all, u_r):
+        """d(loss)/d(colour(0, s)) and d(loss)/d(source f) for the inputs that require them (None for the rest).
+        Only the reprojection term (one launch per scale, weight u_r[s]) and the smoothness term (one launch per
+        scale, weight u_all[s]; scale 0 adds into the target's) depend on the colours: the identity and the hint
+        candidates only decide the masks.  Computed on the fp32 frames; returned in each input's dtype."""
+        S, n_src, B, H, W, smooth_w = ctx.cfg[:6]
+        min_depth, max_depth, flags, col_dtypes, src_dtypes = ctx.colour
+        ik = saved[0]
+        colors = saved[1:1 + S]
+        srcs = saved[1 + S:1 + S + n_src]
+        disps = saved[1 + S + n_src:1 + 2 * S + n_src]
+        sels = saved[1 + 2 * S + n_src:1 + 3 * S + n_src]
+        need_col = [bool(ctx.needs_input_grad[7 + s]) for s in range(S)]
+        need_src = [bool(ctx.needs_input_grad[7 + S + f]) for f in range(n_src)]
+        lib = _lib_()
+        u_all, u_r = f32c(u_all), f32c(u_r)
+        g_col = [None] * S
+        g_src = [torch.zeros_like(srcs[f]) if need_src[f] else None for f in range(n_src)]
+        if need_col[0]:
+            g_col[0] = torch.zeros_like(colors[0])
+        if need_col[0] or any(need_src):
+            src_arr, T_arr, gsrc_arr = ptr_array(srcs), ptr_array(Ts), ptr_array(g_src)
+            for s in range(S):
+                d = disps[s]
+                with ops._timed("photo_image_grad_dh"):
+                    check(lib.dmh_photo_image_grad_dh(ptr(colors[0]), src_arr, T_arr, n_src, ptr(d), d.shape[2],
+                                                      d.shape[3], ptr(k), ptr(ik), ptr(sels[s]), ptr(u_r[s:s + 1]), B, H,
+                                                      W, min_depth, max_depth, flags, ptr(g_col[0]), gsrc_arr, stream()),
+                          "photo_image_grad_dh")
+        for s in range(S):
+            if not need_col[s]:
+                continue
+            d = disps[s]
+            if s > 0:
+                g_col[s] = torch.empty_like(colors[s])
+            # upstream u_all[s] = g_total / S + g_scales[s], already formed: passed as the per-scale weights
+            check(lib.dmh_smooth_image_grad(ptr(d), ptr(colors[s]), B, d.shape[2], d.shape[3], ptr(img_scalars[s]),
+                                            smooth_w[s], s, S, None, ptr(u_all), int(s == 0), ptr(g_col[s]), stream()),
+                  "smooth_image_grad")
+        g_col = [g if g is None or g.dtype == dt else g.to(dt) for g, dt in zip(g_col, col_dtypes)]
+        g_src = [g if g is None or g.dtype == dt else g.to(dt) for g, dt in zip(g_src, src_dtypes)]
+        return g_col, g_src
 
 
 def _depth_hint_losses_fused(colors, disps, K, inv_K, Ts, frame_ids, scales, height, width, depth_hint,
@@ -361,8 +429,9 @@ def _depth_hint_losses_oplevel(colors: Dict, disps: Dict, K, inv_K, Ts: Dict, fr
     if not disable_automasking:
         with torch.no_grad():
             ident = torch.empty(B, len(srcs), height, width, device=target.device, dtype=torch.float32)
-            check(_lib_().dmh_identity_loss(ptr(f32c(target)), ptr_array([f32c(s) for s in srcs]), len(srcs), B, height,
-                                            width, int(no_ssim), ptr(ident), stream()), "identity_loss")
+            target32, srcs32 = f32c(target), [f32c(s) for s in srcs]      # held until the launch (see _prologue)
+            check(_lib_().dmh_identity_loss(ptr(target32), ptr_array(srcs32), len(srcs), B, height, width,
+                                            int(no_ssim), ptr(ident), stream()), "identity_loss")
     losses, aux = {}, {}
     total = 0
     for scale in scales:

@@ -372,6 +372,7 @@ def warp_with_aux(disp, src, K, inv_K, T, min_depth=0.1, max_depth=100.0, input_
 FLAG_NO_SSIM = 1
 FLAG_AVG_REPROJECTION = 2
 FLAG_INPUT_IS_DEPTH = 4
+FLAG_SEL_SOURCE = 8          # dmh_photo_scale_dh: sel also records the winning source frame (sel >> 2)
 FLAG_SRC_PACKED = 16
 
 

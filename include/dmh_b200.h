@@ -166,6 +166,7 @@ int dmh_identity_loss_pack_bf16(const uint16_t* target_bf16, const uint16_t* src
 #define DMH_PHOTO_NO_SSIM 1
 #define DMH_PHOTO_AVG_REPROJECTION 2
 #define DMH_PHOTO_INPUT_IS_DEPTH 4
+#define DMH_PHOTO_SEL_SOURCE 8  /* dmh_photo_scale_dh only: sel = argmin | (winning source frame << 2), see there */
 #define DMH_PHOTO_SRC_PACKED 16 /* src_host[0] is the (B,H,W,4) layout of dmh_identity_loss_pack; F == 1, no pose grad */
 #define DMH_PHOTO_MAX_FRAMES 4
 int dmh_photo_tiles(int H, int W);           /* CTAs per batch item */
@@ -227,7 +228,12 @@ int dmh_selftest_reciprocals(unsigned long long* mismatches, unsigned int seed, 
  * Outputs: sums_partial = 4 x B*dmh_photo_tiles floats, per-CTA partial sums of [reproj*mask_r, mask_r,
  * log(|hint-depth|+1)*valid*mask_h, mask_h]; grad_disp = d(sum reproj*mask_r)/d(up-sampled disp) and
  * grad_disp_hint = d(sum proxy*mask_h)/d(up-sampled disp), both UN-normalised (the masked-mean denominators are
- * known only after the pass: the caller divides); grad_P_partial as in dmh_photo_scale; sel = argmin index.   */
+ * known only after the pass: the caller divides); grad_P_partial as in dmh_photo_scale; sel = argmin index.
+ * With DMH_PHOTO_SEL_SOURCE in flags, sel also records the source frame whose reprojection is the (first) minimum
+ * over the frames: sel = argmin | (frame << 2), so sel & 3 is the argmin index as without the flag.  It is the
+ * decision dmh_photo_image_grad_dh routes the reprojection gradient by.  On the single-source fast path (F == 1) the
+ * flag is accepted and the upper bits are 0; under DMH_PHOTO_AVG_REPROJECTION they are 0 as well (no minimum is
+ * taken).  dmh_photo_scale ignores the flag.                                                                      */
 int dmh_photo_scale_dh(const float* target, const float* const* src_host, const float* const* T_host, int F,
                        const float* disp, int disp_h, int disp_w, const float* K, const float* inv_K,
                        const float* ident, const float* noise, const float* hint_reproj, const float* hint_depth,
@@ -287,6 +293,18 @@ int dmh_photo_image_grad(const float* target, const float* const* src_host, cons
 int dmh_smooth_image_grad(const float* disp, const float* img, int B, int h, int w, const float* img_scalars,
                           float smooth_weight, int scale, int S, const float* g_total, const float* g_scales,
                           int accumulate, float* grad_img, dmh_stream_t stream);
+/* dmh_photo_image_grad_dh: the reprojection terms of ONE scale of the depth-hints objective (backward of
+ * depth_hints.depth_hint_losses w.r.t. the frames), the contract of dmh_photo_image_grad otherwise.  sel (B,H,W) as
+ * dmh_photo_scale_dh writes it with DMH_PHOTO_SEL_SOURCE (needed when F > 1 without DMH_PHOTO_AVG_REPROJECTION):
+ * pixels whose argmin (sel & 3) is the identity get nothing, the others send their reprojection term's gradient to
+ * source frame sel >> 2 (to every frame with weight 1/F under DMH_PHOTO_AVG_REPROJECTION).  u: device scalar, the
+ * upstream weight of the term's per-pixel losses, (d loss / d reproj_loss_s) / (sum(mask_r) + 1e-7).  The identity
+ * and hint candidates only decide the mask: there is no identity launch, so the caller zeroes grad_target and every
+ * grad_src[f] before the first scale.  ADDS into grad_target, and atomically into grad_src[f].                   */
+int dmh_photo_image_grad_dh(const float* target, const float* const* src_host, const float* const* T_host, int F,
+                            const float* disp, int disp_h, int disp_w, const float* K, const float* inv_K,
+                            const uint8_t* sel, const float* u, int B, int H, int W, float min_depth, float max_depth,
+                            int flags, float* grad_target, float* const* grad_src_host, dmh_stream_t stream);
 
 /* ======================= stage 1: physical patch attack ======================= */
 

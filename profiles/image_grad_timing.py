@@ -1,7 +1,9 @@
 #!/usr/bin/env python
 """Forward + backward of the fused objective with and without the colour-frame gradients (CUDA events), and the
-kernel times of the colour-gradient launches, for BASELINE config 2 (B=32, 1024x320, [0,'s'], 4 scales) and
-mono+stereo (B=32, 1024x320, [0,-1,1,'s'], pose gradients).  Prints the card and its power limit with the numbers.
+kernel times of the colour-gradient launches, for BASELINE config 2 (B=32, 1024x320, [0,'s'], 4 scales),
+mono+stereo (B=32, 1024x320, [0,-1,1,'s'], pose gradients) and the depth-hints objective of BASELINE config 4
+(B=32, 1024x320, [0,'s'], 4 scales, depth_hints.depth_hint_losses).  The runs without and with colour gradients
+alternate.  Prints the card and its power limit with the numbers.
 usage: python profiles/image_grad_timing.py [--iters 20] [--batch 32]"""
 import argparse
 import os
@@ -11,7 +13,7 @@ import sys
 import torch
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-from depthmodelhardening_b200 import objective, ops, synth  # noqa: E402
+from depthmodelhardening_b200 import depth_hints, objective, ops, synth  # noqa: E402
 
 
 def card():
@@ -25,15 +27,17 @@ def card():
 
 def bytes_per_px(F, S):
     """Algorithmic bytes per target pixel of the colour-gradient launches (fp32): S reprojection launches and one
-    identity launch.  Per scale: read 12 target + 12 F gathered sources + <= 4 disparity + 1 sel, write 24 target
-    read-modify-write + 12 F source RED; identity: read 12 + 12 F + S sel, write 12 + 12 F."""
+    identity launch (none for the depth-hints objective).  Per scale: read 12 target + 12 F gathered sources + <= 4
+    disparity + 1 sel, write 24 target read-modify-write + 12 F source RED; identity: read 12 + 12 F + S sel, write
+    12 + 12 F."""
     return S * (12 + 12 * F + 4 + 1 + 24 + 12 * F), (12 + 12 * F + S) + (12 + 12 * F)
 
 
-def run_case(name, frame_ids, B, H, W, iters, dev):
-    pb = synth.photo_batch(batch=B, height=H, width=W, frame_ids=frame_ids, seed=5).to(dev)
+def run_case(name, frame_ids, B, H, W, iters, dev, hints=False):
+    pb = synth.photo_batch(batch=B, height=H, width=W, frame_ids=frame_ids, seed=5, depth_hints=hints).to(dev)
     F = len(frame_ids) - 1
     S = len(pb.scales)
+    noise1 = {s: pb.noise[s][:, :1].contiguous() for s in pb.scales}
 
     def make(colour):
         colors = {k: v.clone().requires_grad_(colour) for k, v in pb.color.items()}
@@ -41,8 +45,13 @@ def run_case(name, frame_ids, B, H, W, iters, dev):
         Ts = {k: v.clone().requires_grad_(k != "s") for k, v in pb.T.items()}
 
         def step():
-            losses, _ = objective.photometric_losses(colors, disps, pb.K, pb.inv_K, Ts, pb.frame_ids, pb.scales, H, W,
-                                                     noise=pb.noise)
+            if hints:
+                losses, _ = depth_hints.depth_hint_losses(colors, disps, pb.K, pb.inv_K, Ts, pb.frame_ids, pb.scales, H,
+                                                          W, pb.extras["depth_hint"], pb.extras["depth_hint_mask"], True,
+                                                          noise=noise1)
+            else:
+                losses, _ = objective.photometric_losses(colors, disps, pb.K, pb.inv_K, Ts, pb.frame_ids, pb.scales, H,
+                                                         W, noise=pb.noise)
             losses["loss"].backward()
         return step
 
@@ -62,24 +71,25 @@ def run_case(name, frame_ids, B, H, W, iters, dev):
     t0 = timed(base)
     t1 = timed(with_c)
     t0b = timed(base)                              # alternate: the spread of the baseline shows in t0 vs t0b
+    t1b = timed(with_c)
     ops.KERNEL_EVENTS = []
     for _ in range(iters):
         with_c()
     torch.cuda.synchronize()
     per = {}
     for n, a, b in ops.KERNEL_EVENTS:
-        if n in ("identity_image_grad", "photo_image_grad"):
+        if n in ("identity_image_grad", "photo_image_grad", "photo_image_grad_dh"):
             per.setdefault(n, []).append(a.elapsed_time(b))
     ops.KERNEL_EVENTS = None
     print("%s: B=%d %dx%d frames=%s scales=%d" % (name, B, W, H, list(frame_ids), S))
     print("  fwd+bwd without colour grads  %.3f ms / %.3f ms (two runs)" % (t0, t0b))
-    print("  fwd+bwd with colour grads     %.3f ms" % t1)
+    print("  fwd+bwd with colour grads     %.3f ms / %.3f ms (two runs)" % (t1, t1b))
     npx = B * H * W
     per_scale_b, ident_b = bytes_per_px(F, S)
     for n, ts in sorted(per.items()):
         ts = sorted(ts)
         med = ts[len(ts) // 2]
-        nbytes = (per_scale_b / S if n == "photo_image_grad" else ident_b) * npx
+        nbytes = (ident_b if n == "identity_image_grad" else per_scale_b / S) * npx
         print("  %-20s median %.3f ms per launch (%d launches), %.0f B/px algorithmic -> %.2f TB/s" % (
             n, med, len(ts), nbytes / npx, nbytes / med / 1e9))
 
@@ -95,6 +105,7 @@ def main():
     print(card())
     run_case("config 2", (0, "s"), a.batch, 320, 1024, a.iters, dev)
     run_case("mono+stereo", (0, -1, 1, "s"), a.batch, 320, 1024, a.iters, dev)
+    run_case("config 4 (depth hints)", (0, "s"), a.batch, 320, 1024, a.iters, dev, hints=True)
 
 
 if __name__ == "__main__":
