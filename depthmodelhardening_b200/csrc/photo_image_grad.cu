@@ -12,6 +12,9 @@
 //                            grad_target in place (each pixel is owned by one thread; launches run in stream order:
 //                            deterministic) and scattered into grad_src[f] through the bilinear taps by RED
 //                            (warp-aggregated, as dmh_warp_bwd).
+//                            With DMH_PHOTO_INPUT_IS_DEPTH the network output is a depth map, used as it is (the
+//                            forward's chain); with DMH_PHOTO_PIXEL_SUM the loss is the sum over the pixels, not
+//                            their mean (ops.photo_scale_sum).
 //   dmh_photo_image_grad_dh  the same kernel for the depth-hints objective (depth_hints.py): the reprojection term
 //                            counts wherever the identity did not win the argmin over [reprojection, identity,
 //                            hint] and goes to the forward's first-minimum source frame (or 1/F to each under
@@ -249,8 +252,9 @@ struct ReprojGradParams {
 size_t reproj_smem_bytes() { return sizeof(float) * ((size_t)7 * IG_R2 + 13 * IG_R1 + IG_MAXF * 24); }
 
 // DH: the depth-hints objective (sel from dmh_photo_scale_dh with DMH_PHOTO_SEL_SOURCE, gate reproj_gate_dh, upstream
-// weight *u_dh); otherwise monodepth2's (reproj_gate, upstream(...) * inv_den)
-template <bool FASTDIV, bool DH>
+// weight *u_dh); otherwise monodepth2's (reproj_gate, upstream(...) * inv_den).  DEPTH_IN: the network output is a
+// depth map (DMH_PHOTO_INPUT_IS_DEPTH), not a disparity.
+template <bool FASTDIV, bool DH, bool DEPTH_IN>
 __global__ void __launch_bounds__(IG_THREADS)
 reproj_grad_kernel(const ReprojGradParams p) {
     extern __shared__ float smem[];
@@ -296,7 +300,8 @@ reproj_grad_kernel(const ReprojGradParams p) {
         const size_t o = (size_t)iy * W + ix;
 #pragma unroll
         for (int ch = 0; ch < 3; ++ch) tgt[ch * IG_R2 + i] = __ldg(p.target + ((size_t)b * 3 + ch) * N + o);
-        dep[i] = disp_to_depth(load_disp(p.disp, b, iy, ix, H, W), p.ds);
+        const float dv = load_disp(p.disp, b, iy, ix, H, W);
+        dep[i] = DEPTH_IN ? dv : disp_to_depth(dv, p.ds);
     }
     __syncthreads();
     const float u = s_u;
@@ -442,7 +447,8 @@ smooth_img_grad_kernel(const float* __restrict__ disp, const float* __restrict__
 }
 
 // dmh_photo_image_grad (DH = false) and dmh_photo_image_grad_dh: the argument checks and the launch shared by both.
-// p arrives with the upstream weight of its mode filled in; `name` is the public entry point, for the errors.
+// p arrives with the upstream weight of its mode filled in; `name` is the public entry point, for the errors.  A depth
+// input is a mode of dmh_photo_image_grad only.
 template <bool DH>
 int reproj_grad_launch(const char* name, ReprojGradParams& p, const float* target, const float* const* src_host,
                        const float* const* T_host, int F, const float* disp, int disp_h, int disp_w, const float* K,
@@ -453,7 +459,9 @@ int reproj_grad_launch(const char* name, ReprojGradParams& p, const float* targe
     DMH_REQUIRE(B > 0 && B <= 65535 && H >= 2 && W >= 2, "%s: bad shape B=%d H=%d W=%d", name, B, H, W);
     DMH_REQUIRE(disp_h >= 1 && disp_w >= 1 && disp_h <= H && disp_w <= W, "%s: bad disparity size %dx%d", name, disp_h,
                 disp_w);
-    DMH_REQUIRE(min_depth > 0.f && max_depth > min_depth, "%s: bad depth range", name);
+    const bool depth_in = (flags & DMH_PHOTO_INPUT_IS_DEPTH) != 0;
+    DMH_REQUIRE(!(DH && depth_in), "%s: no depth-input mode", name);
+    DMH_REQUIRE(depth_in || (min_depth > 0.f && max_depth > min_depth), "%s: bad depth range", name);
     p.target = target;
     for (int f = 0; f < F; ++f) {
         DMH_REQUIRE(src_host[f] && T_host[f], "%s: null src/T for frame %d", name, f);
@@ -466,15 +474,21 @@ int reproj_grad_launch(const char* name, ReprojGradParams& p, const float* targe
     p.K = K; p.inv_K = inv_K; p.sel = sel;
     p.grad_target = grad_target;
     p.B = B; p.H = H; p.W = W; p.F = F; p.flags = flags;
-    p.ds = depth_scale(min_depth, max_depth, false);
+    p.ds = depth_scale(min_depth, max_depth, depth_in);
     // the division rule of the forward kernels: bit-identical either way, the verified one is shorter
     const bool fastdiv = const_div_exact(W - 1, &p.rcw, st) && const_div_exact(H - 1, &p.rch, st);
     const size_t smem = reproj_smem_bytes();
     static KernelSetup setup;
-    const void* kernels[2] = {(const void*)reproj_grad_kernel<false, DH>, (const void*)reproj_grad_kernel<true, DH>};
-    if (setup.sms(name, kernels, 2, smem) == 0) return DMH_ERR_CUDA;
+    // the depth-input instantiations exist for DH = false only (for DH = true the last two repeat the first two)
+    const void* kernels[4] = {(const void*)reproj_grad_kernel<false, DH, false>,
+                              (const void*)reproj_grad_kernel<true, DH, false>,
+                              (const void*)reproj_grad_kernel<false, DH, !DH>,
+                              (const void*)reproj_grad_kernel<true, DH, !DH>};
+    if (setup.sms(name, kernels, DH ? 2 : 4, smem) == 0) return DMH_ERR_CUDA;
     const dim3 grid(ceil_div(W, IG_TW), ceil_div(H, IG_TH), B);
-    void (*kernel)(const ReprojGradParams) = fastdiv ? reproj_grad_kernel<true, DH> : reproj_grad_kernel<false, DH>;
+    void (*kernel)(const ReprojGradParams) =
+        depth_in ? (fastdiv ? reproj_grad_kernel<true, DH, !DH> : reproj_grad_kernel<false, DH, !DH>)
+                 : (fastdiv ? reproj_grad_kernel<true, DH, false> : reproj_grad_kernel<false, DH, false>);
     DMH_LAUNCH(kernel, grid, IG_THREADS, smem, st)(p);
     DMH_CHECK_LAUNCH(name);
     return DMH_OK;
@@ -529,7 +543,7 @@ int dmh_photo_image_grad(const float* target, const float* const* src_host, cons
     ReprojGradParams p = {};
     p.g_total = g_total; p.g_scale = g_scales ? g_scales + scale : nullptr;
     p.inv_S = 1.0f / (float)S;
-    p.inv_den = (float)(1.0 / ((double)B * H * W));
+    p.inv_den = (flags & DMH_PHOTO_PIXEL_SUM) ? 1.0f : (float)(1.0 / ((double)B * H * W));
     p.n_ident = automask ? ((flags & DMH_PHOTO_AVG_REPROJECTION) ? 1 : F) : 0;
     return reproj_grad_launch<false>("dmh_photo_image_grad", p, target, src_host, T_host, F, disp, disp_h, disp_w, K,
                                      inv_K, sel, B, H, W, min_depth, max_depth, flags, grad_target, grad_src_host,

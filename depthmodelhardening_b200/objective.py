@@ -178,27 +178,56 @@ def fused_compute_losses(self, inputs, outputs):
 
 
 # ----------------------------------------------------------------------------- CUDA-graph replay (small batches)
+# keyword options of each objective (everything else is fixed by the constructor's arguments)
+_OPTS = {"photometric": frozenset({"min_depth", "max_depth", "no_ssim", "avg_reprojection", "disable_automasking",
+                                   "disparity_smoothness", "noise_mode", "want_selection"})}
+_OPTS["depth_hints"] = _OPTS["photometric"] | {"use_depth_hints"}
+
+
 class GraphedObjective:
-    """Forward + backward of `photometric_losses` captured once into a CUDA graph and replayed.
+    """Forward + backward of `photometric_losses` (or, given `depth_hint` and `depth_hint_mask`, of the fused
+    `depth_hints.depth_hint_losses`) captured once into a CUDA graph and replayed.
 
     At the reference's CPU-runnable configuration (B=4, 640x192) one step is ~25 short launches and eager
     PyTorch is launch-bound (0.55 ms per step against 0.22 ms of GPU work, measured on B200); replaying a graph
     removes the Python / launch overhead.  Shapes, options and the set of tensors are frozen at construction;
     `__call__` copies new values into the static buffers (device-to-device), replays, and returns the static
-    loss / per-scale losses / disparity gradients (valid until the next call).  Tie-break noise: a static
-    buffer per scale that the caller may refresh through `noise=`; it is NOT redrawn by the replay."""
+    losses and gradients (valid until the next call).
+
+    Gradients: `grads[scale]` is d(loss)/d(disps[scale]), always.  A `colors[(f, s)]` or `Ts[f]` entry that requires
+    grad when the object is built is differentiated too: `grads[("color", f, s)]` and `grads[("T", f)]`, in the
+    input's dtype.  Only the frames the objective reads (colour(0, s) for every scale, colour(f, 0) for every source)
+    and the sources' poses are considered.  With none marked, the capture is the disparity-only one.
+
+    Tie-break noise: a static buffer per scale, (B, Fi, H, W) for `photometric_losses` and (B, 1, H, W) for the
+    depth-hints objective, that the caller may refresh through `noise=`; it is NOT redrawn by the replay.  The noise,
+    K / inv_K and the depth hint get no gradient."""
 
     def __init__(self, colors: Dict, disps: Dict, K, inv_K, Ts: Dict, frame_ids, scales, height, width,
-                 noise: Optional[Dict] = None, warmup: int = 3, **opts):
+                 noise: Optional[Dict] = None, warmup: int = 3, depth_hint=None, depth_hint_mask=None, **opts):
+        if (depth_hint is None) != (depth_hint_mask is None):
+            raise ValueError("GraphedObjective: depth_hint and depth_hint_mask go together")
+        kind = "photometric" if depth_hint is None else "depth_hints"
+        unknown = sorted(set(opts) - _OPTS[kind])
+        if unknown:
+            raise TypeError("GraphedObjective: option(s) %s not accepted by the %s objective" % (", ".join(unknown), kind))
         dev = colors[(0, 0)].device
         self.frame_ids, self.scales, self.hw, self.opts = list(frame_ids), list(scales), (height, width), dict(opts)
-        self.colors = {k: v.detach().clone() for k, v in colors.items()}
+        self.colors = {k: v.detach().clone().requires_grad_(v.requires_grad) for k, v in colors.items()}
         self.disps = {s: disps[s].detach().clone().requires_grad_(True) for s in self.scales}
         self.K, self.inv_K = K.detach().clone(), inv_K.detach().clone()
-        self.Ts = {k: v.detach().clone() for k, v in Ts.items()}
-        n_src = len(self.frame_ids) - 1
+        self.Ts = {k: v.detach().clone().requires_grad_(v.requires_grad) for k, v in Ts.items()}
+        self.hint = depth_hint.detach().clone() if depth_hint is not None else None
+        self.hint_mask = depth_hint_mask.detach().clone() if depth_hint_mask is not None else None
+        srcs = self.frame_ids[1:]
+        used = [(0, s) for s in self.scales] + [(f, 0) for f in srcs]
+        self.colour_keys = [k for k in used if self.colors[k].requires_grad]
+        self.T_keys = [f for f in srcs if self.Ts[f].requires_grad]
         automask = not self.opts.get("disable_automasking", False)
-        n_ident = 0 if not automask else (1 if self.opts.get("avg_reprojection", False) else n_src)
+        if self.hint is not None:
+            n_ident = 1 if automask else 0
+        else:
+            n_ident = 0 if not automask else (1 if self.opts.get("avg_reprojection", False) else len(srcs))
         self.noise = None
         if n_ident:
             B = self.colors[(0, 0)].shape[0]
@@ -206,7 +235,9 @@ class GraphedObjective:
                               tie_break_noise((B, n_ident, height, width), dev, "device")) for s in self.scales}
         side = torch.cuda.Stream(device=dev)
         side.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(side):                       # warm-up outside the capture (lazy one-time set-up)
+        # warm-up outside the capture, with the gradients the capture takes: lazy one-time set-up (side streams,
+        # kernel attributes, division constants) of every path the replay runs
+        with torch.cuda.stream(side):
             for _ in range(max(1, warmup)):
                 self._run()
         torch.cuda.current_stream().wait_stream(side)
@@ -215,22 +246,34 @@ class GraphedObjective:
             self.losses, self.grads = self._run()
 
     def _run(self):
-        losses, _ = photometric_losses(self.colors, self.disps, self.K, self.inv_K, self.Ts, self.frame_ids,
-                                       self.scales, self.hw[0], self.hw[1], noise=self.noise, **self.opts)
-        grads = torch.autograd.grad(losses["loss"], [self.disps[s] for s in self.scales])
-        return losses, dict(zip(self.scales, grads))
+        if self.hint is None:
+            losses, _ = photometric_losses(self.colors, self.disps, self.K, self.inv_K, self.Ts, self.frame_ids,
+                                           self.scales, self.hw[0], self.hw[1], noise=self.noise, **self.opts)
+        else:
+            from . import depth_hints
+            losses, _ = depth_hints.depth_hint_losses(self.colors, self.disps, self.K, self.inv_K, self.Ts,
+                                                      self.frame_ids, self.scales, self.hw[0], self.hw[1], self.hint,
+                                                      self.hint_mask, noise=self.noise, fused=True, **self.opts)
+        S, nc = len(self.scales), len(self.colour_keys)
+        grads = torch.autograd.grad(losses["loss"], [self.disps[s] for s in self.scales] +
+                                    [self.colors[k] for k in self.colour_keys] + [self.Ts[f] for f in self.T_keys])
+        out = dict(zip(self.scales, grads[:S]))
+        out.update({("color",) + k: g for k, g in zip(self.colour_keys, grads[S:S + nc])})
+        out.update({("T", f): g for f, g in zip(self.T_keys, grads[S + nc:])})
+        return losses, out
 
     @torch.no_grad()
     def __call__(self, colors: Optional[Dict] = None, disps: Optional[Dict] = None, K=None, inv_K=None,
-                 Ts: Optional[Dict] = None, noise: Optional[Dict] = None):
+                 Ts: Optional[Dict] = None, noise: Optional[Dict] = None, depth_hint=None, depth_hint_mask=None):
         for dst, src in ((self.colors, colors), (self.disps, disps), (self.Ts, Ts), (self.noise, noise)):
             if src is not None and dst is not None:
                 for k, v in src.items():
                     if k in dst:
                         dst[k].copy_(v if dst is not self.noise else v[:, :dst[k].shape[1]], non_blocking=True)
-        if K is not None:
-            self.K.copy_(K, non_blocking=True)
-        if inv_K is not None:
-            self.inv_K.copy_(inv_K, non_blocking=True)
+        for dst, src in ((self.K, K), (self.inv_K, inv_K), (self.hint, depth_hint), (self.hint_mask, depth_hint_mask)):
+            if src is not None:
+                if dst is None:
+                    raise ValueError("GraphedObjective: built without a depth hint")
+                dst.copy_(src, non_blocking=True)
         self.graph.replay()
         return self.losses, self.grads

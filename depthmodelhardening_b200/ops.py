@@ -374,12 +374,14 @@ FLAG_AVG_REPROJECTION = 2
 FLAG_INPUT_IS_DEPTH = 4
 FLAG_SEL_SOURCE = 8          # dmh_photo_scale_dh: sel also records the winning source frame (sel >> 2)
 FLAG_SRC_PACKED = 16
+FLAG_PIXEL_SUM = 32          # dmh_photo_image_grad: the loss is the sum over the pixels (photo_scale_sum), not the mean
 
 
 class _PhotoScale(torch.autograd.Function):
     """sum over (B,H,W) of the per-pixel min-reprojection loss for one scale, with
     its gradient w.r.t. the full-resolution disparity (and poses) produced in the
-    same kernel launch."""
+    same kernel launch.  Gradients for the target, the sources and the identity losses
+    are recomputed in the backward from the saved frames and the forward's `sel`."""
 
     @staticmethod
     def forward(ctx, disp, target, ident, noise, K, inv_K, min_depth, max_depth, flags, want_sel, n_src, *src_and_T):
@@ -394,17 +396,28 @@ class _PhotoScale(torch.autograd.Function):
         part = torch.empty(B * tiles, device=d.device, dtype=torch.float32)
         gdisp = torch.empty_like(d)
         need_T = any(ctx.needs_input_grad[11 + n_src + i] for i in range(n_src))
+        # gradients for the frames and the identity losses follow the forward's decision, so `sel` is requested
+        # internally
+        colour_grad = ctx.needs_input_grad[1] or any(ctx.needs_input_grad[11 + i] for i in range(n_src))
+        ident_grad = ctx.needs_input_grad[2]
         gP = torch.empty(n_src, B, tiles, 12, device=d.device, dtype=torch.float32) if need_T else None
-        sel = torch.empty(B, H, W, device=d.device, dtype=torch.uint8) if want_sel else None
+        want_sels = want_sel or colour_grad or ident_grad
+        sel = torch.empty(B, H, W, device=d.device, dtype=torch.uint8) if want_sels else None
         with _timed("photo_scale"):
             check(lib.dmh_photo_scale(ptr(tg), ptr_array(srcs), ptr_array(Ts), n_src, ptr(d), H, W, ptr(k), ptr(ik),
                                       ptr(idn), ptr(nz), B, H, W, min_depth, max_depth, flags, 1.0, ptr(part),
                                       ptr(gdisp), ptr(gP), ptr(sel), None, stream()), "photo_scale")
         total = torch.empty((), device=d.device, dtype=torch.float32)
         check(lib.dmh_reduce_sum(ptr(part), part.numel(), 1.0, 0, ptr(total), stream()), "reduce_sum")
-        ctx.save_for_backward(gdisp, gP, k, *Ts)
         ctx.n_src = n_src
         ctx.dshape = disp.shape
+        ctx.colour = None
+        extra = []
+        if colour_grad or ident_grad:
+            ctx.colour = (float(min_depth), float(max_depth), flags, target.dtype, [t.dtype for t in src_and_T[:n_src]],
+                          ident.dtype if ident is not None else None, ident.shape[1] if ident is not None else 0)
+            extra = [sel, ik, d, tg, *srcs] if colour_grad else [sel]
+        ctx.save_for_backward(gdisp, gP, k, *Ts, *extra)
         if want_sel:
             ctx.mark_non_differentiable(sel)
             return total, sel
@@ -414,8 +427,8 @@ class _PhotoScale(torch.autograd.Function):
     def backward(ctx, g_total, _g_sel):
         saved = ctx.saved_tensors
         gdisp, gP, k = saved[0], saved[1], saved[2]
-        Ts = saved[3:]
         n_src = ctx.n_src
+        Ts = saved[3:3 + n_src]
         g_d = (gdisp * g_total).view(ctx.dshape) if ctx.needs_input_grad[0] else None
         g_T: List[Optional[torch.Tensor]] = [None] * n_src
         if gP is not None:
@@ -423,12 +436,59 @@ class _PhotoScale(torch.autograd.Function):
             for i in range(n_src):
                 if ctx.needs_input_grad[11 + n_src + i]:
                     _, g_T[i] = _grad_KT_from_P(gPs[i].view(-1, 3, 4), k, Ts[i], False, True)
-        return (g_d, None, None, None, None, None, None, None, None, None, None) + (None,) * n_src + tuple(g_T)
+        g_tg, g_id, g_src = None, None, [None] * n_src
+        if ctx.colour is not None:
+            g_tg, g_id, g_src = _PhotoScale._input_grads(ctx, saved[3 + n_src:], k, Ts, f32c(g_total).reshape(1))
+        return (g_d, g_tg, g_id, None, None, None, None, None, None, None, None) + tuple(g_src) + tuple(g_T)
+
+    @staticmethod
+    def _input_grads(ctx, saved, k, Ts, gt):
+        """d(sum)/d(target), d(sum)/d(source f) and d(sum)/d(ident) for the inputs that require them (None for the
+        rest), in each input's dtype.  The identity losses are inputs here, so the frames only receive the
+        reprojection terms (one dmh_photo_image_grad launch); an identity plane receives g_total where `sel` picked
+        it (g_total / F on every plane under avg_reprojection, which compares their mean)."""
+        min_depth, max_depth, flags, tg_dtype, src_dtypes, id_dtype, n_planes = ctx.colour
+        n_src = ctx.n_src
+        sel = saved[0]
+        g_tg, g_id, g_src = None, None, [None] * n_src
+        if ctx.needs_input_grad[2]:
+            if flags & FLAG_AVG_REPROJECTION:
+                g_id = ((sel == 0).unsqueeze(1) * (gt / n_planes)).expand(-1, n_planes, -1, -1)
+            else:
+                planes = torch.arange(n_planes, device=sel.device, dtype=sel.dtype).view(1, -1, 1, 1)
+                g_id = (sel.unsqueeze(1) == planes) * gt
+            g_id = g_id.to(id_dtype).contiguous()
+        need_tg = ctx.needs_input_grad[1]
+        need_src = [bool(ctx.needs_input_grad[11 + i]) for i in range(n_src)]
+        if need_tg or any(need_src):
+            ik, d, tg = saved[1], saved[2], saved[3]
+            srcs = saved[4:4 + n_src]
+            B, _, H, W = tg.shape
+            g_tg = torch.zeros_like(tg) if need_tg else None
+            g_src = [torch.zeros_like(srcs[i]) if need_src[i] else None for i in range(n_src)]
+            with _timed("photo_image_grad"):
+                check(_lib_().dmh_photo_image_grad(ptr(tg), ptr_array(srcs), ptr_array(Ts), n_src, ptr(d), H, W,
+                                                   ptr(k), ptr(ik), ptr(sel), 0, 1, ptr(gt), None, B, H, W, min_depth,
+                                                   max_depth, (flags & (FLAG_NO_SSIM | FLAG_AVG_REPROJECTION |
+                                                                        FLAG_INPUT_IS_DEPTH)) | FLAG_PIXEL_SUM,
+                                                   int(n_planes > 0), ptr(g_tg), ptr_array(g_src), stream()),
+                      "photo_image_grad")
+            g_tg = g_tg if g_tg is None or g_tg.dtype == tg_dtype else g_tg.to(tg_dtype)
+            g_src = [g if g is None or g.dtype == dt else g.to(dt) for g, dt in zip(g_src, src_dtypes)]
+        return g_tg, g_id, g_src
 
 
 def photo_scale_sum(disp_full, target, srcs: Sequence[torch.Tensor], Ts: Sequence[torch.Tensor], K, inv_K,
                     ident=None, noise=None, min_depth=0.1, max_depth=100.0, no_ssim=False, avg_reprojection=False,
                     input_is_depth=False, want_sel=False):
+    """Sum over (B,H,W) of the per-pixel minimum over [ident (+ noise), reprojection of each source] at full
+    resolution.  disp_full (B,1,H,W) [or depth with input_is_depth]; ident (B,F,H,W) identity losses (averaged over
+    the frames under avg_reprojection) or None; noise (B,F,H,W) ((B,1,H,W) under avg_reprojection) or None.
+    Differentiable w.r.t. disp_full, the poses, the target, the sources and ident (not noise, K or inv_K).
+    Returns (total, sel or None)."""
+    if tuple(disp_full.shape[-2:]) != tuple(target.shape[-2:]):
+        raise ValueError("photo_scale_sum: the disparity (%dx%d) must have the target's resolution (%dx%d)" %
+                         (*disp_full.shape[-2:], *target.shape[-2:]))
     flags = (FLAG_NO_SSIM if no_ssim else 0) | (FLAG_AVG_REPROJECTION if avg_reprojection else 0) | \
             (FLAG_INPUT_IS_DEPTH if input_is_depth else 0)
     B = target.shape[0]

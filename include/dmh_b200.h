@@ -168,6 +168,7 @@ int dmh_identity_loss_pack_bf16(const uint16_t* target_bf16, const uint16_t* src
 #define DMH_PHOTO_INPUT_IS_DEPTH 4
 #define DMH_PHOTO_SEL_SOURCE 8  /* dmh_photo_scale_dh only: sel = argmin | (winning source frame << 2), see there */
 #define DMH_PHOTO_SRC_PACKED 16 /* src_host[0] is the (B,H,W,4) layout of dmh_identity_loss_pack; F == 1, no pose grad */
+#define DMH_PHOTO_PIXEL_SUM 32  /* dmh_photo_image_grad only: the loss is the sum of the per-pixel losses, see there */
 #define DMH_PHOTO_MAX_FRAMES 4
 int dmh_photo_tiles(int H, int W);           /* CTAs per batch item */
 int dmh_photo_scale(const float* target, const float* const* src_host, const float* const* T_host, int F,
@@ -278,7 +279,10 @@ int dmh_disp_grad(const float* G_full, const float* gN, const float* img_scalars
  * dmh_identity_image_grad: ONE launch for all S scales: the identity candidates' terms (un-warped source f vs
  *   target, gated by sum_s u_s [sel_s picked f's identity]).  INITIALISES grad_target and every grad_src[f].
  * dmh_photo_image_grad: one launch per scale `scale`: the reprojection candidates' terms; ADDS into grad_target and
- *   (atomically: the last bits depend on the order) into grad_src[f] through the bilinear taps of the warp.
+ *   (atomically: the last bits depend on the order) into grad_src[f] through the bilinear taps of the warp.  It also
+ *   takes DMH_PHOTO_INPUT_IS_DEPTH (disp is a depth map, used as it is; min_depth / max_depth are ignored) and
+ *   DMH_PHOTO_PIXEL_SUM (the loss is the sum of the per-pixel losses, as dmh_photo_scale computes it with
+ *   inv_den = 1: the per-pixel weight is u_s, not u_s / (B*H*W)).
  * dmh_smooth_image_grad: u_s * smooth_weight * d(smoothness of scale s)/d(img) for img = colour(0, s) (B,3,h,w),
  *   disp (B,1,h,w), img_scalars the (B,2) slice of dmh_objective_finish for scale s; accumulate: add into grad_img
  *   instead of writing it.                                                                                         */
