@@ -31,7 +31,8 @@ SIGNATURES = {
     "dmh_const_div_exact": (_i, [_i]),
     "dmh_disp_to_depth": (_i, [_f, _ll, _fl, _fl, _f, _f, _st]),
     "dmh_backproject_fwd": (_i, [_f, _f, _i, _i, _i, _f, _st]),
-    "dmh_backproject_bwd": (_i, [_f, _f, _i, _i, _i, _f, _st]),
+    "dmh_backproject_bwd_blocks": (_i, [_i, _i]),
+    "dmh_backproject_bwd": (_i, [_f, _f, _f, _i, _i, _i, _f, _f, _st]),
     "dmh_project3d_fwd": (_i, [_f, _f, _f, _i, _i, _i, _fl, _f, _st]),
     "dmh_project3d_bwd_blocks": (_i, [_i, _i]),
     "dmh_project3d_bwd": (_i, [_f, _f, _f, _f, _i, _i, _i, _fl, _f, _f, _st]),

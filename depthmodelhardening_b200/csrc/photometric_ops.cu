@@ -50,22 +50,49 @@ __global__ void backproject_fwd_kernel(const float* __restrict__ depth, const fl
     out[(size_t)3 * N] = 1.0f;
 }
 
-__global__ void backproject_bwd_kernel(const float* __restrict__ gpts, const float* __restrict__ inv_K, int H, int W,
-                                       float* __restrict__ gdepth) {
+#define BP_BWD_THREADS 256
+// grad_depth (nullable) and, when giK_partial != nullptr, the per-block partials of
+// d/d(inv_K[:3,:3])_ij = sum_n g_i(n) * depth(n) * pix_j(n), pix = (x, y, 1)
+__global__ void __launch_bounds__(BP_BWD_THREADS)
+backproject_bwd_kernel(const float* __restrict__ gpts, const float* __restrict__ depth,
+                       const float* __restrict__ inv_K, int H, int W, float* __restrict__ gdepth,
+                       float* __restrict__ giK_partial) {
+    __shared__ float red[32];
     const int b = blockIdx.y;
     const int N = H * W;
     const int n = blockIdx.x * blockDim.x + threadIdx.x;
-    if (n >= N) return;
-    Camera cam;
-    const float* iK = inv_K + b * 16;
+    float gd[3] = {0.f, 0.f, 0.f};
+    float pix[3] = {0.f, 0.f, 0.f};
+    if (n < N) {
+        const float* g = gpts + (size_t)b * 4 * N + n;
+        gd[0] = g[0]; gd[1] = g[(size_t)N]; gd[2] = g[(size_t)2 * N];
+        pix[0] = (float)(n % W); pix[1] = (float)(n / W); pix[2] = 1.0f;
+        if (gdepth) {
+            Camera cam;
+            const float* iK = inv_K + b * 16;
 #pragma unroll
-    for (int i = 0; i < 3; ++i)
+            for (int i = 0; i < 3; ++i)
 #pragma unroll
-        for (int j = 0; j < 3; ++j) cam.iK[i * 3 + j] = __ldg(iK + i * 4 + j);
-    float ray[3];
-    pixel_ray(cam, (float)(n % W), (float)(n / W), ray);
-    const float* g = gpts + (size_t)b * 4 * N + n;
-    gdepth[(size_t)b * N + n] = g[0] * ray[0] + g[(size_t)N] * ray[1] + g[(size_t)2 * N] * ray[2];
+                for (int j = 0; j < 3; ++j) cam.iK[i * 3 + j] = __ldg(iK + i * 4 + j);
+            float ray[3];
+            pixel_ray(cam, pix[0], pix[1], ray);
+            gdepth[(size_t)b * N + n] = gd[0] * ray[0] + gd[1] * ray[1] + gd[2] * ray[2];
+        }
+        if (giK_partial) {
+            const float d = depth[(size_t)b * N + n];
+            gd[0] *= d; gd[1] *= d; gd[2] *= d;
+        }
+    }
+    if (giK_partial) {
+        float* out = giK_partial + ((size_t)b * gridDim.x + blockIdx.x) * 9;
+#pragma unroll
+        for (int i = 0; i < 3; ++i)
+#pragma unroll
+            for (int j = 0; j < 3; ++j) {
+                const float s = block_sum(gd[i] * pix[j], red);
+                if (threadIdx.x == 0) out[i * 3 + j] = s;
+            }
+    }
 }
 
 // ------------------------------------------------------------------ A11
@@ -165,15 +192,18 @@ __global__ void project3d_bwd_kernel(const float* __restrict__ ggrid, const floa
 // ------------------------------------------------------------------ A12
 struct SampleCoord { float ix, iy, mx, my; };
 
+// A NaN coordinate under border padding: ATen's CUDA forward clips with fmin/fmax (NaN -> 0, the sample reads
+// column / row 0), while its backward clips with comparisons (clip_coordinates_set_grad lets NaN through) and then
+// safe_downgrade_to_int_range sends it to -100, so the gradient pass scatters nothing.  `for_grad` picks the latter.
 __device__ __forceinline__ SampleCoord sample_coord(float gx, float gy, int Ws, int Hs, int padding_mode,
-                                                    bool align_corners) {
+                                                    bool align_corners, bool for_grad) {
     SampleCoord s;
     float ux = unnormalise_coord(gx, Ws, align_corners);
     float uy = unnormalise_coord(gy, Hs, align_corners);
     float cx = 1.0f, cy = 1.0f;
     if (padding_mode == DMH_PAD_BORDER) {
-        ux = (ux == ux) ? clip_coord(ux, Ws, cx) : (cx = 0.0f, 0.0f);
-        uy = (uy == uy) ? clip_coord(uy, Hs, cy) : (cy = 0.0f, 0.0f);
+        ux = (ux == ux || for_grad) ? clip_coord(ux, Ws, cx) : (cx = 0.0f, 0.0f);
+        uy = (uy == uy || for_grad) ? clip_coord(uy, Hs, cy) : (cy = 0.0f, 0.0f);
     }
     s.ix = safe_coord(ux);
     s.iy = safe_coord(uy);
@@ -190,7 +220,7 @@ __global__ void grid_sample_fwd_kernel(const float* __restrict__ src, const floa
     const int n = blockIdx.x * blockDim.x + threadIdx.x;
     if (n >= No) return;
     const float2 g = reinterpret_cast<const float2*>(grid)[(size_t)b * No + n];
-    const SampleCoord sc = sample_coord(g.x, g.y, Ws, Hs, padding_mode, align_corners != 0);
+    const SampleCoord sc = sample_coord(g.x, g.y, Ws, Hs, padding_mode, align_corners != 0, false);
     const Bilinear bl = bilinear_setup(sc.ix, sc.iy);
     const bool x0in = bl.x0 >= 0 && bl.x0 < Ws, x1in = bl.x0 + 1 >= 0 && bl.x0 + 1 < Ws;
     const bool y0in = bl.y0 >= 0 && bl.y0 < Hs, y1in = bl.y0 + 1 >= 0 && bl.y0 + 1 < Hs;
@@ -217,7 +247,7 @@ __global__ void grid_sample_bwd_kernel(const float* __restrict__ gout, const flo
     const int n = blockIdx.x * blockDim.x + threadIdx.x;
     if (n >= No) return;
     const float2 g = reinterpret_cast<const float2*>(grid)[(size_t)b * No + n];
-    const SampleCoord sc = sample_coord(g.x, g.y, Ws, Hs, padding_mode, align_corners != 0);
+    const SampleCoord sc = sample_coord(g.x, g.y, Ws, Hs, padding_mode, align_corners != 0, true);
     const Bilinear bl = bilinear_setup(sc.ix, sc.iy);
     const bool x0in = bl.x0 >= 0 && bl.x0 < Ws, x1in = bl.x0 + 1 >= 0 && bl.x0 + 1 < Ws;
     const bool y0in = bl.y0 >= 0 && bl.y0 < Hs, y1in = bl.y0 + 1 >= 0 && bl.y0 + 1 < Hs;
@@ -443,12 +473,16 @@ int dmh_backproject_fwd(const float* depth, const float* inv_K, int B, int H, in
     return DMH_OK;
 }
 
-int dmh_backproject_bwd(const float* grad_points, const float* inv_K, int B, int H, int W, float* grad_depth,
-                        dmh_stream_t stream) {
-    DMH_REQUIRE(grad_points && inv_K && grad_depth, "dmh_backproject_bwd: null pointer");
+int dmh_backproject_bwd_blocks(int H, int W) { return ceil_div((long long)H * W, BP_BWD_THREADS); }
+
+int dmh_backproject_bwd(const float* grad_points, const float* depth, const float* inv_K, int B, int H, int W,
+                        float* grad_depth, float* grad_inv_K_partial, dmh_stream_t stream) {
+    DMH_REQUIRE(grad_points && inv_K && (grad_depth || grad_inv_K_partial), "dmh_backproject_bwd: null pointer");
+    DMH_REQUIRE(depth || !grad_inv_K_partial, "dmh_backproject_bwd: null pointer (depth is needed for grad_inv_K)");
     DMH_REQUIRE(B > 0 && H > 0 && W > 0 && B <= 65535, "dmh_backproject_bwd: bad shape");
-    dim3 grid(ceil_div((long long)H * W, 256), B);
-    DMH_LAUNCH(backproject_bwd_kernel, grid, 256, 0, (cudaStream_t)stream)(grad_points, inv_K, H, W, grad_depth);
+    dim3 grid(dmh_backproject_bwd_blocks(H, W), B);
+    DMH_LAUNCH(backproject_bwd_kernel, grid, BP_BWD_THREADS, 0, (cudaStream_t)stream)(grad_points, depth, inv_K, H, W,
+                                                                                  grad_depth, grad_inv_K_partial);
     DMH_CHECK_LAUNCH("dmh_backproject_bwd");
     return DMH_OK;
 }

@@ -52,6 +52,8 @@ class Project3D(nn.Module):
         self.eps = eps
 
     def forward(self, points, K, T):
+        if points.dim() != 3 or points.shape[1] != 4:
+            raise RuntimeError("Project3D: expected homogeneous points of shape (B,4,N), got %s" % (tuple(points.shape),))
         if points.shape[0] != self.batch_size or points.shape[-1] != self.height * self.width:
             raise RuntimeError("shape '[%d, 2, %d, %d]' is invalid for input of size %d" %
                                (self.batch_size, self.height, self.width, points.shape[0] * 2 * points.shape[-1]))

@@ -58,6 +58,21 @@ def _mat_batch(m: torch.Tensor, B: int, name: str) -> torch.Tensor:
     raise RuntimeError("%s holds %d matrices but the batch is %d (only a batch of 1 broadcasts)" % (name, m.shape[0], B))
 
 
+def _same_shape(op, a, b, an, bn):
+    """Raise (as torch would) when two inputs that a kernel indexes with one set of dimensions disagree in shape."""
+    if a.shape != b.shape:
+        raise RuntimeError("%s: %s and %s must have the same shape, got %s and %s" %
+                           (op, an, bn, tuple(a.shape), tuple(b.shape)))
+
+
+def _disp_matches(op, disp, img, img_name):
+    """A (B,1,H,W) disparity / depth map and the (B,C,H,W) image it belongs to."""
+    if disp.dim() != 4 or img.dim() != 4 or disp.shape[1] != 1 or disp.shape[0] != img.shape[0] \
+            or disp.shape[2:] != img.shape[2:]:
+        raise RuntimeError("%s: expected disp of shape (B,1,H,W) matching %s (B,C,H,W), got disp %s and %s %s" %
+                           (op, img_name, tuple(disp.shape), img_name, tuple(img.shape)))
+
+
 # ----------------------------------------------------------------------------- A9
 def disp_to_depth_cuda(disp: torch.Tensor, min_depth: float, max_depth: float):
     d = f32c(disp)
@@ -95,18 +110,26 @@ class _Backproject(torch.autograd.Function):
         d, ik = f32c(depth), f32c(inv_K)
         pts = torch.empty(B, 4, H * W, device=d.device, dtype=torch.float32)
         check(_lib_().dmh_backproject_fwd(ptr(d), ptr(ik), B, H, W, ptr(pts), stream()), "backproject_fwd")
-        ctx.save_for_backward(ik)
+        ctx.save_for_backward(d if ctx.needs_input_grad[1] else None, ik)     # depth: only for d/d(inv_K)
         ctx.dims = (B, H, W, depth.shape)
         return pts
 
     @staticmethod
     def backward(ctx, g_pts):
-        (ik,) = ctx.saved_tensors
+        d, ik = ctx.saved_tensors
         B, H, W, shape = ctx.dims
         g = f32c(g_pts)
-        gd = torch.empty(B, 1, H, W, device=g.device, dtype=torch.float32)
-        check(_lib_().dmh_backproject_bwd(ptr(g), ptr(ik), B, H, W, ptr(gd), stream()), "backproject_bwd")
-        return gd.view(shape), None, None, None, None
+        gd = torch.empty(B, 1, H, W, device=g.device, dtype=torch.float32) if ctx.needs_input_grad[0] else None
+        nblk = _lib_().dmh_backproject_bwd_blocks(H, W)
+        giK_part = torch.empty(B, nblk, 9, device=g.device, dtype=torch.float32) if ctx.needs_input_grad[1] else None
+        check(_lib_().dmh_backproject_bwd(ptr(g), ptr(d), ptr(ik), B, H, W, ptr(gd), ptr(giK_part), stream()),
+              "backproject_bwd")
+        giK = None
+        if giK_part is not None:
+            # cam = depth * (inv_K[:3,:3] @ pix): only the 3x3 block receives a gradient
+            giK = torch.zeros(B, 4, 4, device=g.device, dtype=torch.float32)
+            giK[:, :3, :3] = giK_part.sum(1).view(B, 3, 3)
+        return (gd.view(shape) if gd is not None else None), giK, None, None, None
 
 
 # ----------------------------------------------------------------------------- A11
@@ -165,6 +188,15 @@ def _pose_grad_T(gPs, u, f, K, T):
 class _GridSample(torch.autograd.Function):
     @staticmethod
     def forward(ctx, src, grid, padding_mode, align_corners):
+        if src.dim() != 4 or grid.dim() != 4:
+            raise RuntimeError("grid_sample: expected 4-D input and grid, got input %s and grid %s" %
+                               (tuple(src.shape), tuple(grid.shape)))
+        if grid.shape[0] != src.shape[0]:
+            raise RuntimeError("grid_sample: expected grid and input to have same batch size, but got input with "
+                               "sizes %s and grid with sizes %s" % (list(src.shape), list(grid.shape)))
+        if grid.shape[3] != 2:
+            raise RuntimeError("grid_sample: expected grid to have size 2 in last dimension, but got grid with "
+                               "sizes %s" % list(grid.shape))
         s, g = f32c(src), f32c(grid)
         B, Cc, Hs, Ws = s.shape
         _, Ho, Wo, _ = g.shape
@@ -202,6 +234,7 @@ def grid_sample(src, grid, mode="bilinear", padding_mode="zeros", align_corners=
 class _SSIM(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, y):
+        _same_shape("SSIM", x, y, "x", "y")
         a, b = f32c(x), f32c(y)
         B, Cc, H, W = a.shape
         out = torch.empty_like(a)
@@ -224,6 +257,7 @@ class _SSIM(torch.autograd.Function):
 class _ReprojLoss(torch.autograd.Function):
     @staticmethod
     def forward(ctx, pred, target, no_ssim):
+        _same_shape("reprojection_loss", pred, target, "pred", "target")
         a, b = f32c(pred), f32c(target)
         B, Cc, H, W = a.shape
         out = torch.empty(B, 1, H, W, device=a.device, dtype=torch.float32)
@@ -253,6 +287,7 @@ def reprojection_loss(pred, target, no_ssim=False):
 class _Smooth(torch.autograd.Function):
     @staticmethod
     def forward(ctx, disp, img, normalise):
+        _disp_matches("smooth_loss", disp, img, "img")
         d, im = f32c(disp), f32c(img)
         B, _, h, w = d.shape
         Cc = im.shape[1]
@@ -312,6 +347,7 @@ def upsample_bilinear(x, size):
 class _WarpFused(torch.autograd.Function):
     @staticmethod
     def forward(ctx, disp, src, K, inv_K, T, min_depth, max_depth, input_is_depth):
+        _disp_matches("warp_reproject", disp, src, "src")
         d, s, k, ik, t = f32c(disp), f32c(src), f32c(K), f32c(inv_K), f32c(T)
         B, Cc, H, W = s.shape
         out = torch.empty_like(s)
@@ -344,7 +380,11 @@ class _WarpFused(torch.autograd.Function):
 def warp_reproject(disp, src, K, inv_K, T, min_depth=0.1, max_depth=100.0, input_is_depth=False):
     """disp (B,1,H,W) [or depth] + src (B,C,H,W) -> src warped into the target view.
     One gather kernel for trainer.py:485-519 (disp_to_depth, BackprojectDepth,
-    Project3D, grid_sample(border, align_corners=True))."""
+    Project3D, grid_sample(border, align_corners=True)).  Differentiable w.r.t. disp, src, K and T, not inv_K: an
+    inv_K that requires grad is refused rather than given a zero gradient."""
+    if inv_K.requires_grad and torch.is_grad_enabled():
+        raise RuntimeError("warp_reproject: no gradient w.r.t. inv_K; detach it (or use BackprojectDepth / Project3D, "
+                           "which return one)")
     B = src.shape[0]
     return _WarpFused.apply(disp, src, _mat_batch(K, B, "K"), _mat_batch(inv_K, B, "inv_K"), _mat_batch(T, B, "T"),
                             float(min_depth), float(max_depth), bool(input_is_depth))
@@ -354,7 +394,11 @@ def warp_with_aux(disp, src, K, inv_K, T, min_depth=0.1, max_depth=100.0, input_
                   want_aux=True):
     """No-grad variant also returning the sampling grid and the depth map
     (the tensors the reference stores in `outputs` for logging).  align_corners=False: the sampling convention of
-    the depth-hints warp (`F.grid_sample` default, DH/trainer.py:523-525)."""
+    the depth-hints warp (`F.grid_sample` default, DH/trainer.py:523-525).  Returns no gradient, so an input that
+    requires grad is refused while grad mode is on."""
+    if torch.is_grad_enabled() and any(t.requires_grad for t in (disp, src, K, inv_K, T)):
+        raise RuntimeError("warp_with_aux returns no gradient; call it under torch.no_grad() or use warp_reproject")
+    _disp_matches("warp_with_aux", disp, src, "src")
     B = src.shape[0]
     d, s, k, ik, t = (f32c(disp), f32c(src), f32c(_mat_batch(K, B, "K")), f32c(_mat_batch(inv_K, B, "inv_K")),
                       f32c(_mat_batch(T, B, "T")))

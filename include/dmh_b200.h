@@ -49,11 +49,14 @@ int dmh_disp_to_depth(const float* disp, long long n, float min_depth, float max
                       float* depth, dmh_stream_t stream);
 
 /* -- A10 BackprojectDepth.forward (M2/layers.py:163-168) ------------------
- * depth (B,1,H,W), inv_K (B,4,4) -> points (B,4,H*W) [x,y,z,1 planes]        */
+ * depth (B,1,H,W), inv_K (B,4,4) -> points (B,4,H*W) [x,y,z,1 planes]
+ * bwd: grad_depth (B,1,H,W) (nullable); grad_inv_K_partial (B, nblk, 9) per-block partial sums of
+ * d/d(inv_K[:3,:3]) with nblk = dmh_backproject_bwd_blocks(H,W) (nullable; needs depth).          */
 int dmh_backproject_fwd(const float* depth, const float* inv_K, int B, int H, int W, float* points,
                         dmh_stream_t stream);
-int dmh_backproject_bwd(const float* grad_points, const float* inv_K, int B, int H, int W, float* grad_depth,
-                        dmh_stream_t stream);
+int dmh_backproject_bwd_blocks(int H, int W);
+int dmh_backproject_bwd(const float* grad_points, const float* depth, const float* inv_K, int B, int H, int W,
+                        float* grad_depth, float* grad_inv_K_partial, dmh_stream_t stream);
 
 /* -- A11 Project3D.forward (M2/layers.py:182-198) -------------------------
  * points (B,4,N), K,T (B,4,4) -> grid (B,H,W,2) in [-1,1] (unclamped)

@@ -22,7 +22,7 @@ import torch.nn.functional as F
 
 from depthmodelhardening_b200 import synth
 from oracle import photometric as OP
-from tests.util import assert_close, assert_grad_close
+from tests.util import assert_close, assert_grad_close, assert_within, up_weights
 
 pytestmark = pytest.mark.gpu
 U = 2.0 ** -24
@@ -60,44 +60,7 @@ def _at_offset(src, off):
     return v
 
 
-def _assert_within(got, ref, bound, what, mask=None):
-    """|got - ref| <= bound for every element (float64 arithmetic); `mask` selects the elements compared."""
-    got = got.double()
-    assert torch.isfinite(got).all(), "%s: non-finite elements" % what
-    err = (got - ref).abs()
-    bad = err > bound
-    if mask is not None:
-        bad &= mask
-    n = int(bad.sum())
-    if n:
-        idx = tuple(int(i) for i in bad.nonzero()[0])
-        ratio = float((err / bound.clamp_min(1e-300))[bad].max())
-        raise AssertionError("%s: %d of %d elements beyond the rounding bound (worst %.3g x the bound; first at %s: "
-                             "got %r, expected %r, bound %.3g)" % (what, n, bad.numel(), ratio, idx, float(got[idx]),
-                                                                   float(ref[idx]), float(bound[idx])))
-
-
 # ----------------------------------------------------------------------------- dmh_disp_grad
-def _up_weights(n_out, n_in):
-    """(n_out, n_in) float64 matrix of F.interpolate(bilinear, align_corners=False) weights with the kernels' fp32
-    arithmetic (dmh_common.cuh up_tap, compiled to src = fma(in/out, dst + 0.5, -0.5): one rounding), l1 = src - i0,
-    l0 = 1 - l1, and a tap clamped at the last pixel counts l0 + l1 (added in fp32)."""
-    sc = np.float32(n_in) / np.float32(n_out)
-    t = np.arange(n_out, dtype=np.float32) + np.float32(0.5)
-    src = (np.float64(sc) * t.astype(np.float64) - 0.5).astype(np.float32)     # exact product, one rounding
-    src = np.maximum(src, np.float32(0.0))
-    i0 = np.minimum(src.astype(np.int64), n_in - 1)
-    i1 = np.where(i0 < n_in - 1, i0 + 1, i0)
-    l1 = (src - i0.astype(np.float32)).astype(np.float32)
-    l0 = (np.float32(1.0) - l1).astype(np.float32)
-    A = np.zeros((n_out, n_in))
-    r = np.arange(n_out)
-    same = i0 == i1
-    A[r, i0] = np.where(same, (l0 + l1).astype(np.float32), l0)
-    A[r[~same], i1[~same]] = l1[~same]
-    return A
-
-
 def _dg_regime(h, w, H, W, p_g, p_gn, p_out):
     """Host restatement of dmh_disp_grad's kernel choice (objective_fused.cu)."""
     R = H // h if (H % h == 0 and W % w == 0 and H // h == W // w) else 0
@@ -174,8 +137,8 @@ def test_disp_grad_every_element_vs_fp64(lib, B, h, w, H, W, offs, regime):
     scald = scal.to(DEV)
     new_out = lambda: _at_offset(torch.full((B, 1, h, w), float("nan"), device=DEV), oo)
     assert _dg_regime(h, w, H, W, Gd.data_ptr(), gNd.data_ptr(), new_out().data_ptr()) == regime
-    Ay = torch.from_numpy(_up_weights(H, h)).to(DEV)
-    Ax = torch.from_numpy(_up_weights(W, w)).to(DEV)
+    Ay = torch.from_numpy(up_weights(H, h)).to(DEV)
+    Ax = torch.from_numpy(up_weights(W, w)).to(DEV)
     G64 = G.double().to(DEV)[:, 0]
     acc = torch.einsum("Yy,bYX,Xx->byx", Ay, G64, Ax)
     acc_abs = torch.einsum("Yy,bYX,Xx->byx", Ay, G64.abs(), Ax)
@@ -212,7 +175,7 @@ def test_disp_grad_every_element_vs_fp64(lib, B, h, w, H, W, offs, regime):
         else:
             ref = up * (acc + sm)
             terms = up_abs * (acc_abs + sm_abs)
-        _assert_within(out[:, 0], ref, k * U * terms, "%s %s (%d,%d)->(%d,%d)" % (regime, form, h, w, H, W))
+        assert_within(out[:, 0], ref, k * U * terms, "%s %s (%d,%d)->(%d,%d)" % (regime, form, h, w, H, W))
 
 
 def test_disp_grad_refuses_missing_upstream(lib):
@@ -317,12 +280,12 @@ def test_smooth_fused_and_finish_vs_fp64(lib, B, C_, sizes):
         k_l = 16 + 8 + (C_ + 6) + k_m + 6
         tie = r["tie"]
         assert float(tie.double().mean()) < 1e-2, "too many near-tied edges for a meaningful comparison"
-        _assert_within(gNs[s].cpu(), r["g"], k_g * U * r["T"], "gN scale %d (%dx%d, C=%d)" % (s, h, w, C_), mask=~tie)
-        _assert_within(scal[s, :, 0], r["inv_m"], k_m * U * r["inv_m"], "1/(mean+eps) scale %d" % s)
+        assert_within(gNs[s].cpu(), r["g"], k_g * U * r["T"], "gN scale %d (%dx%d, C=%d)" % (s, h, w, C_), mask=~tie)
+        assert_within(scal[s, :, 0], r["inv_m"], k_m * U * r["inv_m"], "1/(mean+eps) scale %d" % s)
         gd, dT, tie_c = r["corr_terms"]
         inv_m2 = r["inv_m"] ** 2
         cb = inv_m2 / (h * w) * (k_g * U * dT + 24 * U * gd + tie_c) + (2 * k_m + 3) * U * r["corr"].abs()
-        _assert_within(scal[s, :, 1], r["corr"], cb, "corr scale %d" % s)
+        assert_within(scal[s, :, 1], r["corr"], cb, "corr scale %d" % s)
         lref = sw[s] * r["loss"]
         lb = sw[s] * k_l * U * r["loss_terms"]
         assert abs(float(losses[s]) - lref) <= lb, "loss/%d: %r vs %r (bound %.3g)" % (s, float(losses[s]), lref, lb)
@@ -382,9 +345,9 @@ def test_objective_finish_vs_fp64(lib, S, B):
         sp = ws[s][B * 64:].double().view(B, -1, 3)
         inv_m = 1.0 / (mp.sum(1) / hw + 1e-7)
         corr = sp[..., 2].sum(1) / hw * inv_m ** 2
-        _assert_within(scal[s, :, 0], inv_m, 10 * U * inv_m, "inv_m scale %d" % s)
+        assert_within(scal[s, :, 0], inv_m, 10 * U * inv_m, "inv_m scale %d" % s)
         cterms = sp[..., 2].abs().sum(1) / hw * inv_m ** 2
-        _assert_within(scal[s, :, 1], corr, 23 * U * corr.abs() + 2.0 ** -45 * cterms, "corr scale %d" % s)
+        assert_within(scal[s, :, 1], corr, 23 * U * corr.abs() + 2.0 ** -45 * cterms, "corr scale %d" % s)
         ph = parts[s][:pns[s]].double().sum()
         inx, iny = 1.0 / (B * h * (w - 1)), 1.0 / (B * (h - 1) * w)
         loss = float(ph / den + sw[s] * (sp[..., 0].sum() * inx + sp[..., 1].sum() * iny))

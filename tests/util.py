@@ -118,3 +118,44 @@ def assert_selection_close(sel, ref, what="argmin", frac=1e-4):
     allowed = max(2, int(np.ceil(frac * sel.size)))
     _record("selection", what, differ=bad, allowed=allowed, elements=sel.size)
     assert bad <= allowed, "%s: %d of %d selections differ (allowed %d)" % (what, bad, sel.size, allowed)
+
+
+def assert_within(got, ref, bound, what, mask=None):
+    """|got - ref| <= bound for every element (float64 arithmetic); `mask` selects the elements compared."""
+    got, ref, bound = got.detach().double(), ref.detach(), bound.detach()
+    assert torch.isfinite(got).all(), "%s: non-finite elements" % what
+    err = (got - ref).abs()
+    bad = err > bound
+    if mask is not None:
+        bad &= mask
+    n = int(bad.sum())
+    ratio = err / bound.clamp_min(1e-300)
+    compared = ratio if mask is None else ratio[mask]
+    _record("within", what, worst_over_bound=float(compared.max()) if compared.numel() else 0.0, outside=n,
+            elements=compared.numel())
+    if n:
+        idx = tuple(int(i) for i in bad.nonzero()[0])
+        ratio = float(ratio[bad].max())
+        raise AssertionError("%s: %d of %d elements beyond the rounding bound (worst %.3g x the bound; first at %s: "
+                             "got %r, expected %r, bound %.3g)" % (what, n, bad.numel(), ratio, idx, float(got[idx]),
+                                                                   float(ref[idx]), float(bound[idx])))
+
+
+def up_weights(n_out, n_in):
+    """(n_out, n_in) float64 matrix of F.interpolate(bilinear, align_corners=False) weights with the kernels' fp32
+    arithmetic (dmh_common.cuh up_tap, compiled to src = fma(in/out, dst + 0.5, -0.5): one rounding), l1 = src - i0,
+    l0 = 1 - l1, and a tap clamped at the last pixel counts l0 + l1 (added in fp32)."""
+    sc = np.float32(n_in) / np.float32(n_out)
+    t = np.arange(n_out, dtype=np.float32) + np.float32(0.5)
+    src = (np.float64(sc) * t.astype(np.float64) - 0.5).astype(np.float32)     # exact product, one rounding
+    src = np.maximum(src, np.float32(0.0))
+    i0 = np.minimum(src.astype(np.int64), n_in - 1)
+    i1 = np.where(i0 < n_in - 1, i0 + 1, i0)
+    l1 = (src - i0.astype(np.float32)).astype(np.float32)
+    l0 = (np.float32(1.0) - l1).astype(np.float32)
+    A = np.zeros((n_out, n_in))
+    r = np.arange(n_out)
+    same = i0 == i1
+    A[r, i0] = np.where(same, (l0 + l1).astype(np.float32), l0)
+    A[r[~same], i1[~same]] = l1[~same]
+    return A
