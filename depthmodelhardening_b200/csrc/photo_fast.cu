@@ -69,19 +69,7 @@ photo_fast_kernel(const FastParams p, const __grid_constant__ CUtensorMap tgt_ma
     const int N = H * W;                      // per-item offsets fit 32 bits (checked by the launcher)
     const float w_ssim = 0.85f / 3.0f, w_l1 = 0.15f / 3.0f;
 
-    if (tid < 12) {
-        const int i = tid / 4, j = tid % 4;
-        const float* k = p.K + b * 16 + i * 4;
-        const float* tt = p.T + b * 16 + j;
-        float acc = __ldg(k) * __ldg(tt);
-        acc = fmaf(__ldg(k + 1), __ldg(tt + 4), acc);
-        acc = fmaf(__ldg(k + 2), __ldg(tt + 8), acc);
-        acc = fmaf(__ldg(k + 3), __ldg(tt + 12), acc);
-        cams[tid] = acc;
-    } else if (tid < 21) {
-        const int i = (tid - 12) / 3, j = (tid - 12) % 3;
-        cams[tid] = __ldg(p.inv_K + b * 16 + i * 4 + j);
-    }
+    load_camera(cams, p, b, tid);
     if (TMA) {
         // ---- target tile by TMA: in flight during the whole gather phase
         if (tid == 0) {
@@ -184,21 +172,7 @@ photo_fast_kernel(const FastParams p, const __grid_constant__ CUtensorMap tgt_ma
     __syncthreads();
     if (TMA) {
         mbar_wait(&tgt_bar, 0);
-        // ReflectionPad2d(1) at the image border: TMA zero-fills out-of-image elements; patch them from the
-        // in-image rows / columns of the same tile (sources are never patched themselves)
-        if (x0 < 2 || y0 < 2 || x0 + FT_T + 2 > W || y0 + FT_T + 2 > H) {
-            for (int i = tid; i < FT_N2; i += FT_THREADS) {
-                const int r = i / FT_R2, c = i - r * FT_R2;
-                const int ey = y0 - 2 + r, ex = x0 - 2 + c;
-                if (ey < 0 || ey >= H || ex < 0 || ex >= W) {
-                    const int sr = ext_to_img(ey, H) - (y0 - 2), sc = ext_to_img(ex, W) - (x0 - 2);
-#pragma unroll
-                    for (int ch = 0; ch < 3; ++ch)
-                        tgt[ch * FT_NT + r * FT_TP + c + FT_TO] = tgt[ch * FT_NT + sr * FT_TP + sc + FT_TO];
-                }
-            }
-            __syncthreads();
-        }
+        patch_target_border(tgt, tid, x0, y0, H, W);       // (sources are never patched themselves)
     }
 
     TileSmem sm;

@@ -28,19 +28,10 @@
 //   dmh_photo_image_grad     read 12 (target) + 12 F (gathered sources) + <= 4 (disparity) + 1 (sel);
 //                            write 24 (target read-modify-write) + 12 F (source RED)
 //   dmh_identity_image_grad  read 12 + 12 F + S (sel); write 12 + 12 F
-#include "photo_launch.cuh"
+#include "photo_general.cuh"
 
 namespace {
 
-#define IG_TW 32
-#define IG_TH 16
-#define IG_R2W (IG_TW + 4)
-#define IG_R2H (IG_TH + 4)
-#define IG_R1W (IG_TW + 2)
-#define IG_R1H (IG_TH + 2)
-#define IG_R2 (IG_R2W * IG_R2H)
-#define IG_R1 (IG_R1W * IG_R1H)
-#define IG_THREADS 256
 #define IG_MAXF DMH_PHOTO_MAX_FRAMES
 #define IG_MAXS 8
 
@@ -48,26 +39,12 @@ __device__ __forceinline__ float upstream(const float* g_total, const float* g_s
     return add_rn(g_total ? mul_rn(g_total[0], inv_S) : 0.0f, g_scale ? g_scale[0] : 0.0f);
 }
 
-// 3x3 window statistics of one channel plane pair in shared memory around R2 position (r+1, c+1), with the
-// arithmetic of the forward kernels (row sums of 3, then 3 rows)
-__device__ __forceinline__ SsimStatsRows window_stats(const float* __restrict__ xs, const float* __restrict__ ys, int r,
-                                                      int c) {
-    Row5 rows[3];
-#pragma unroll
-    for (int dy = 0; dy < 3; ++dy) {
-        const float* x = xs + (r + dy) * IG_R2W + c;
-        const float* y = ys + (r + dy) * IG_R2W + c;
-        rows[dy] = row5(x[0], x[1], x[2], y[0], y[1], y[2]);
-    }
-    return ssim_stats_rows(rows[0], rows[1], rows[2]);
-}
-
 // Gated SSIM coefficient planes k[4][3][R1] (ax, b, c, ay) of R(x, y) at every ring position whose gate is non-zero
 // (zero elsewhere).  xs / ys: [3][R2] tiles of the prediction / the target.
 __device__ __forceinline__ void coef_planes(const float* __restrict__ xs, const float* __restrict__ ys,
                                             const float* __restrict__ gate, float w_ssim, float* __restrict__ k) {
-    for (int i = threadIdx.x; i < IG_R1; i += IG_THREADS) {
-        const int r = i / IG_R1W, c = i % IG_R1W;
+    for (int i = threadIdx.x; i < PH_R1; i += PH_THREADS) {
+        const int r = i / PH_R1W, c = i % PH_R1W;
         const float g = gate[i];
 #pragma unroll
         for (int ch = 0; ch < 3; ++ch) {
@@ -75,14 +52,14 @@ __device__ __forceinline__ void coef_planes(const float* __restrict__ xs, const 
             if (g != 0.f) {
                 float pass;
                 SsimCoef kk;
-                ssim_value_coef(window_stats(xs + ch * IG_R2, ys + ch * IG_R2, r, c), pass, kk);
+                ssim_value_coef(window_stats(xs + ch * PH_R2, ys + ch * PH_R2, r, c), pass, kk);
                 const float gg = g * w_ssim * pass;
                 a = gg * kk.ax; bq = gg * kk.b; cq = gg * kk.c; d = gg * kk.ay;
             }
-            k[(0 * 3 + ch) * IG_R1 + i] = a;
-            k[(1 * 3 + ch) * IG_R1 + i] = bq;
-            k[(2 * 3 + ch) * IG_R1 + i] = cq;
-            k[(3 * 3 + ch) * IG_R1 + i] = d;
+            k[(0 * 3 + ch) * PH_R1 + i] = a;
+            k[(1 * 3 + ch) * PH_R1 + i] = bq;
+            k[(2 * 3 + ch) * PH_R1 + i] = cq;
+            k[(3 * 3 + ch) * PH_R1 + i] = d;
         }
     }
 }
@@ -93,8 +70,8 @@ __device__ __forceinline__ void pixel_grads(const float* __restrict__ xs, const 
                                             const float* __restrict__ k, const float* __restrict__ gate, int r, int c,
                                             int py, int px, int H, int W, bool ssim, float w_l1, float gx[3],
                                             float gy[3]) {
-    const int ci2 = (r + 2) * IG_R2W + (c + 2);
-    const float gl1 = gate[(r + 1) * IG_R1W + (c + 1)] * w_l1;
+    const int ci2 = (r + 2) * PH_R2W + (c + 2);
+    const float gl1 = gate[(r + 1) * PH_R1W + (c + 1)] * w_l1;
     float wy[3], wx[3];
 #pragma unroll
     for (int d = 0; d < 3; ++d) {
@@ -110,14 +87,14 @@ __device__ __forceinline__ void pixel_grads(const float* __restrict__ xs, const 
 #pragma unroll
                 for (int dx = 0; dx < 3; ++dx) {
                     const float w = wy[dy] * wx[dx];
-                    const int o = ch * IG_R1 + (r + dy) * IG_R1W + c + dx;
+                    const int o = ch * PH_R1 + (r + dy) * PH_R1W + c + dx;
                     sa = fmaf(w, k[o], sa);
-                    sb = fmaf(w, k[3 * IG_R1 + o], sb);
-                    sc = fmaf(w, k[6 * IG_R1 + o], sc);
-                    sd = fmaf(w, k[9 * IG_R1 + o], sd);
+                    sb = fmaf(w, k[3 * PH_R1 + o], sb);
+                    sc = fmaf(w, k[6 * PH_R1 + o], sc);
+                    sd = fmaf(w, k[9 * PH_R1 + o], sd);
                 }
         }
-        reproj_pixel_grad(sa, sb, sc, sd, xs[ch * IG_R2 + ci2], ys[ch * IG_R2 + ci2], gl1, gx[ch], gy[ch]);
+        reproj_pixel_grad(sa, sb, sc, sd, xs[ch * PH_R2 + ci2], ys[ch * PH_R2 + ci2], gl1, gx[ch], gy[ch]);
     }
 }
 
@@ -125,11 +102,11 @@ __device__ __forceinline__ void pixel_grads(const float* __restrict__ xs, const 
 __device__ __forceinline__ void load_tile(const float* __restrict__ img, int b, int x0, int y0, int H, int W,
                                           float* __restrict__ out) {
     const size_t N = (size_t)H * W;
-    for (int i = threadIdx.x; i < IG_R2; i += IG_THREADS) {
-        const int r = i / IG_R2W, c = i % IG_R2W;
+    for (int i = threadIdx.x; i < PH_R2; i += PH_THREADS) {
+        const int r = i / PH_R2W, c = i % PH_R2W;
         const size_t o = (size_t)ext_to_img(y0 - 2 + r, H) * W + ext_to_img(x0 - 2 + c, W);
 #pragma unroll
-        for (int ch = 0; ch < 3; ++ch) out[ch * IG_R2 + i] = __ldg(img + ((size_t)b * 3 + ch) * N + o);
+        for (int ch = 0; ch < 3; ++ch) out[ch * PH_R2 + i] = __ldg(img + ((size_t)b * 3 + ch) * N + o);
     }
 }
 
@@ -146,19 +123,19 @@ struct IdentGradParams {
     int B, H, W, F, S, n_ident, flags;
 };
 
-size_t ident_smem_bytes() { return sizeof(float) * ((size_t)6 * IG_R2 + 13 * IG_R1); }
+size_t ident_smem_bytes() { return sizeof(float) * ((size_t)6 * PH_R2 + 13 * PH_R1); }
 
-__global__ void __launch_bounds__(IG_THREADS)
+__global__ void __launch_bounds__(PH_THREADS)
 identity_grad_kernel(const IdentGradParams p) {
     extern __shared__ float smem[];
     float* tgt = smem;                          // [3][R2]
-    float* xs = tgt + 3 * IG_R2;                // [3][R2] source frame f
-    float* k = xs + 3 * IG_R2;                  // [4][3][R1]
-    float* gate = k + 12 * IG_R1;               // [R1]
+    float* xs = tgt + 3 * PH_R2;                // [3][R2] source frame f
+    float* k = xs + 3 * PH_R2;                  // [4][3][R1]
+    float* gate = k + 12 * PH_R1;               // [R1]
     __shared__ float us[IG_MAXS];
 
     const int H = p.H, W = p.W, b = blockIdx.z;
-    const int x0 = blockIdx.x * IG_TW, y0 = blockIdx.y * IG_TH;
+    const int x0 = blockIdx.x * PH_TW, y0 = blockIdx.y * PH_TH;
     const size_t N = (size_t)H * W;
     const bool no_ssim = (p.flags & DMH_PHOTO_NO_SSIM) != 0;
     const bool avg = (p.flags & DMH_PHOTO_AVG_REPROJECTION) != 0;
@@ -173,8 +150,8 @@ identity_grad_kernel(const IdentGradParams p) {
     float g_tgt[2][3] = {{0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}};
     for (int f = 0; f < p.F; ++f) {
         bool any = false;
-        for (int i = threadIdx.x; i < IG_R1; i += IG_THREADS) {
-            const int qy = y0 - 1 + i / IG_R1W, qx = x0 - 1 + i % IG_R1W;
+        for (int i = threadIdx.x; i < PH_R1; i += PH_THREADS) {
+            const int qy = y0 - 1 + i / PH_R1W, qx = x0 - 1 + i % PH_R1W;
             float g = 0.f;
             if (p.n_ident > 0 && qy >= 0 && qy < H && qx >= 0 && qx < W) {
                 const size_t qo = (size_t)b * N + (size_t)qy * W + qx;
@@ -187,8 +164,8 @@ identity_grad_kernel(const IdentGradParams p) {
         if (!__syncthreads_or(any)) {
             // no pixel of the tile picked this identity at any scale: the tile's source gradient starts at zero
             for (int slot = 0; slot < 2 && gs; ++slot) {
-                const int i = threadIdx.x + slot * IG_THREADS;
-                const int py = y0 + i / IG_TW, px = x0 + i % IG_TW;
+                const int i = threadIdx.x + slot * PH_THREADS;
+                const int py = y0 + i / PH_TW, px = x0 + i % PH_TW;
                 if (py < H && px < W)
                     for (int ch = 0; ch < 3; ++ch) gs[ch * N + (size_t)py * W + px] = 0.f;
             }
@@ -202,8 +179,8 @@ identity_grad_kernel(const IdentGradParams p) {
         }
 #pragma unroll
         for (int slot = 0; slot < 2; ++slot) {
-            const int i = threadIdx.x + slot * IG_THREADS;
-            const int r = i / IG_TW, c = i % IG_TW;
+            const int i = threadIdx.x + slot * PH_THREADS;
+            const int r = i / PH_TW, c = i % PH_TW;
             const int py = y0 + r, px = x0 + c;
             if (py >= H || px >= W) continue;
             float gx[3], gy[3];
@@ -219,8 +196,8 @@ identity_grad_kernel(const IdentGradParams p) {
     if (p.grad_target) {
 #pragma unroll
         for (int slot = 0; slot < 2; ++slot) {
-            const int i = threadIdx.x + slot * IG_THREADS;
-            const int py = y0 + i / IG_TW, px = x0 + i % IG_TW;
+            const int i = threadIdx.x + slot * PH_THREADS;
+            const int py = y0 + i / PH_TW, px = x0 + i % PH_TW;
             if (py >= H || px >= W) continue;
 #pragma unroll
             for (int ch = 0; ch < 3; ++ch)
@@ -249,26 +226,26 @@ struct ReprojGradParams {
     const float* u_dh;           // depth-hints mode: device scalar, the reprojection term's upstream weight of this scale
 };
 
-size_t reproj_smem_bytes() { return sizeof(float) * ((size_t)7 * IG_R2 + 13 * IG_R1 + IG_MAXF * 24); }
+size_t reproj_smem_bytes() { return sizeof(float) * ((size_t)7 * PH_R2 + 13 * PH_R1 + IG_MAXF * 24); }
 
 // DH: the depth-hints objective (sel from dmh_photo_scale_dh with DMH_PHOTO_SEL_SOURCE, gate reproj_gate_dh, upstream
 // weight *u_dh); otherwise monodepth2's (reproj_gate, upstream(...) * inv_den).  DEPTH_IN: the network output is a
 // depth map (DMH_PHOTO_INPUT_IS_DEPTH), not a disparity.
 template <bool FASTDIV, bool DH, bool DEPTH_IN>
-__global__ void __launch_bounds__(IG_THREADS)
+__global__ void __launch_bounds__(PH_THREADS)
 reproj_grad_kernel(const ReprojGradParams p) {
     extern __shared__ float smem[];
     float* tgt = smem;                          // [3][R2]
-    float* dep = tgt + 3 * IG_R2;               // [R2]
-    float* pred = dep + IG_R2;                  // [3][R2] source f warped into the target view
-    float* k = pred + 3 * IG_R2;                // [4][3][R1]
-    float* gate = k + 12 * IG_R1;               // [R1]
-    float* cams = gate + IG_R1;                 // [F][24]
+    float* dep = tgt + 3 * PH_R2;               // [R2]
+    float* pred = dep + PH_R2;                  // [3][R2] source f warped into the target view
+    float* k = pred + 3 * PH_R2;                // [4][3][R1]
+    float* gate = k + 12 * PH_R1;               // [R1]
+    float* cams = gate + PH_R1;                 // [F][24]
     __shared__ float s_u;
 
     const int tid = threadIdx.x;
     const int H = p.H, W = p.W, b = blockIdx.z;
-    const int x0 = blockIdx.x * IG_TW, y0 = blockIdx.y * IG_TH;
+    const int x0 = blockIdx.x * PH_TW, y0 = blockIdx.y * PH_TH;
     const size_t N = (size_t)H * W;
     const bool no_ssim = (p.flags & DMH_PHOTO_NO_SSIM) != 0;
     const bool avg = (p.flags & DMH_PHOTO_AVG_REPROJECTION) != 0;
@@ -277,40 +254,17 @@ reproj_grad_kernel(const ReprojGradParams p) {
     const unsigned lane = tid & 31;
 
     // ---- cameras, target tile and depth: the forward's operations (photo_scale_kernel)
-    if (tid < p.F * 21) {
-        const int f = tid / 21, t = tid % 21;
-        if (t < 12) {
-            const int i = t / 4, j = t % 4;
-            const float* kk = p.K + b * 16 + i * 4;
-            const float* tt = p.T[f] + b * 16 + j;
-            float acc = __ldg(kk) * __ldg(tt);
-            acc = fmaf(__ldg(kk + 1), __ldg(tt + 4), acc);
-            acc = fmaf(__ldg(kk + 2), __ldg(tt + 8), acc);
-            acc = fmaf(__ldg(kk + 3), __ldg(tt + 12), acc);
-            cams[f * 24 + t] = acc;
-        } else {
-            const int i = (t - 12) / 3, j = (t - 12) % 3;
-            cams[f * 24 + t] = __ldg(p.inv_K + b * 16 + i * 4 + j);
-        }
-    }
+    load_cameras(cams, p, p.F, b, tid);
     if (tid == 0) s_u = DH ? __ldg(p.u_dh) : upstream(p.g_total, p.g_scale, p.inv_S) * p.inv_den;
-    for (int i = tid; i < IG_R2; i += IG_THREADS) {
-        const int r = i / IG_R2W, c = i % IG_R2W;
-        const int iy = ext_to_img(y0 - 2 + r, H), ix = ext_to_img(x0 - 2 + c, W);
-        const size_t o = (size_t)iy * W + ix;
-#pragma unroll
-        for (int ch = 0; ch < 3; ++ch) tgt[ch * IG_R2 + i] = __ldg(p.target + ((size_t)b * 3 + ch) * N + o);
-        const float dv = load_disp(p.disp, b, iy, ix, H, W);
-        dep[i] = DEPTH_IN ? dv : disp_to_depth(dv, p.ds);
-    }
+    load_target_depth(p.target, p.disp, p.ds, DEPTH_IN, b, x0, y0, H, W, N, tgt, dep);
     __syncthreads();
     const float u = s_u;
 
     float g_tgt[2][3] = {{0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}};
     for (int f = 0; f < p.F; ++f) {
         bool any = false;
-        for (int i = tid; i < IG_R1; i += IG_THREADS) {
-            const int qy = y0 - 1 + i / IG_R1W, qx = x0 - 1 + i % IG_R1W;
+        for (int i = tid; i < PH_R1; i += PH_THREADS) {
+            const int qy = y0 - 1 + i / PH_R1W, qx = x0 - 1 + i % PH_R1W;
             float g = 0.f;
             if (qy >= 0 && qy < H && qx >= 0 && qx < W) {
                 const int sel = p.sel[(size_t)b * N + (size_t)qy * W + qx];
@@ -326,8 +280,8 @@ reproj_grad_kernel(const ReprojGradParams p) {
 #pragma unroll
         for (int i = 0; i < 9; ++i) cam.iK[i] = cams[f * 24 + 12 + i];
         const float* sp = p.src[f] + (size_t)b * 3 * N;
-        for (int i = tid; i < IG_R2; i += IG_THREADS) {
-            const int r = i / IG_R2W, c = i % IG_R2W;
+        for (int i = tid; i < PH_R2; i += PH_THREADS) {
+            const int r = i / PH_R2W, c = i % PH_R2W;
             const int iy = ext_to_img(y0 - 2 + r, H), ix = ext_to_img(x0 - 2 + c, W);
             const WarpCoord wc = warp_coord<FASTDIV>(cam, (float)ix, (float)iy, dep[i], W, H, 1e-7f, p.rcw, p.rch);
             const Bilinear bl = bilinear_setup(wc.ix, wc.iy);
@@ -340,7 +294,7 @@ reproj_grad_kernel(const ReprojGradParams p) {
                 if (t.ne) acc = fmaf(__ldg(s + t.o00 + 1), bl.wne, acc);
                 if (t.sw) acc = fmaf(__ldg(s + t.o00 + W), bl.wsw, acc);
                 if (t.se) acc = fmaf(__ldg(s + t.o00 + W + 1), bl.wse, acc);
-                pred[ch * IG_R2 + i] = acc;
+                pred[ch * PH_R2 + i] = acc;
             }
         }
         __syncthreads();
@@ -352,8 +306,8 @@ reproj_grad_kernel(const ReprojGradParams p) {
 #pragma unroll
         for (int slot = 0; slot < 2; ++slot) {
             // a warp holds 32 consecutive pixels of one tile row: every lane takes part in the aggregated scatter
-            const int i = tid + slot * IG_THREADS;
-            const int r = i / IG_TW, c = i % IG_TW;
+            const int i = tid + slot * PH_THREADS;
+            const int r = i / PH_TW, c = i % PH_TW;
             const int py = y0 + r, px = x0 + c;
             const bool active = py < H && px < W;
             float gx[3] = {0.f, 0.f, 0.f}, gy[3];
@@ -366,7 +320,7 @@ reproj_grad_kernel(const ReprojGradParams p) {
             Bilinear bl = {};
             Taps t = {};
             if (active) {
-                const WarpCoord wc = warp_coord<FASTDIV>(cam, (float)px, (float)py, dep[(r + 2) * IG_R2W + (c + 2)], W,
+                const WarpCoord wc = warp_coord<FASTDIV>(cam, (float)px, (float)py, dep[(r + 2) * PH_R2W + (c + 2)], W,
                                                          H, 1e-7f, p.rcw, p.rch);
                 bl = bilinear_setup(wc.ix, wc.iy);
                 t = make_taps(bl, H, W);
@@ -392,8 +346,8 @@ reproj_grad_kernel(const ReprojGradParams p) {
     if (p.grad_target) {
 #pragma unroll
         for (int slot = 0; slot < 2; ++slot) {
-            const int i = tid + slot * IG_THREADS;
-            const int py = y0 + i / IG_TW, px = x0 + i % IG_TW;
+            const int i = tid + slot * PH_THREADS;
+            const int py = y0 + i / PH_TW, px = x0 + i % PH_TW;
             if (py >= H || px >= W) continue;
 #pragma unroll
             for (int ch = 0; ch < 3; ++ch) p.grad_target[((size_t)b * 3 + ch) * N + (size_t)py * W + px] += g_tgt[slot][ch];
@@ -485,11 +439,11 @@ int reproj_grad_launch(const char* name, ReprojGradParams& p, const float* targe
                               (const void*)reproj_grad_kernel<false, DH, !DH>,
                               (const void*)reproj_grad_kernel<true, DH, !DH>};
     if (setup.sms(name, kernels, DH ? 2 : 4, smem) == 0) return DMH_ERR_CUDA;
-    const dim3 grid(ceil_div(W, IG_TW), ceil_div(H, IG_TH), B);
+    const dim3 grid(ceil_div(W, PH_TW), ceil_div(H, PH_TH), B);
     void (*kernel)(const ReprojGradParams) =
         depth_in ? (fastdiv ? reproj_grad_kernel<true, DH, !DH> : reproj_grad_kernel<false, DH, !DH>)
                  : (fastdiv ? reproj_grad_kernel<true, DH, false> : reproj_grad_kernel<false, DH, false>);
-    DMH_LAUNCH(kernel, grid, IG_THREADS, smem, st)(p);
+    DMH_LAUNCH(kernel, grid, PH_THREADS, smem, st)(p);
     DMH_CHECK_LAUNCH(name);
     return DMH_OK;
 }
@@ -527,8 +481,8 @@ int dmh_identity_image_grad(const float* target, const float* const* src_host, i
     static KernelSetup setup;
     const void* kernel = (const void*)identity_grad_kernel;
     if (setup.sms("dmh_identity_image_grad", &kernel, 1, smem) == 0) return DMH_ERR_CUDA;
-    const dim3 grid(ceil_div(W, IG_TW), ceil_div(H, IG_TH), B);
-    DMH_LAUNCH(identity_grad_kernel, grid, IG_THREADS, smem, (cudaStream_t)stream)(p);
+    const dim3 grid(ceil_div(W, PH_TW), ceil_div(H, PH_TH), B);
+    DMH_LAUNCH(identity_grad_kernel, grid, PH_THREADS, smem, (cudaStream_t)stream)(p);
     DMH_CHECK_LAUNCH("dmh_identity_image_grad");
     return DMH_OK;
 }

@@ -1,6 +1,6 @@
-// Host-side set-up shared by the launchers of the photometric kernels (photo_fast.cu, photo_ms.cu, photo_mf.cu,
-// photo_objective.cu): the TMA descriptor of the target frames, the one-time kernel attributes per device, the
-// disparity-to-depth constants and the wave split of the multi-scale kernels.
+// Set-up shared by the photometric kernels (photo_fast.cu, photo_ms.cu, photo_mf.cu, photo_objective.cu,
+// photo_image_grad.cu).  Host: the TMA descriptor of the target frames, the one-time kernel attributes per device, the
+// disparity-to-depth constants and the wave split of the multi-scale kernels.  Device: the cameras in shared memory.
 #pragma once
 #include <cuda.h>
 #include <string.h>
@@ -90,6 +90,47 @@ int split_last_wave(int n_tiles, int S, int slots) {
         if (tail > 0 && (tail * S + slots - 1) / slots < S) return n_tiles - tail;
     }
     return n_tiles;
+}
+
+// The cameras of the photometric kernels in shared memory, 24 floats per source frame f of batch item b:
+// P = (K @ T_f)[:3, :] row-major (accumulated in the order of compose_camera), then inv_K[:3, :3].  One thread per
+// float: threads [0, 21 F) take part.  p: the kernel's parameters (K, T[f], inv_K).
+template <class P>
+__device__ __forceinline__ void load_cameras(float* cams, const P& p, int F, int b, int tid) {
+    if (tid < F * 21) {
+        const int f = tid / 21, t = tid % 21;
+        if (t < 12) {
+            const int i = t / 4, j = t % 4;
+            const float* k = p.K + b * 16 + i * 4;
+            const float* tt = p.T[f] + b * 16 + j;
+            float acc = __ldg(k) * __ldg(tt);
+            acc = fmaf(__ldg(k + 1), __ldg(tt + 4), acc);
+            acc = fmaf(__ldg(k + 2), __ldg(tt + 8), acc);
+            acc = fmaf(__ldg(k + 3), __ldg(tt + 12), acc);
+            cams[f * 24 + t] = acc;
+        } else {
+            const int i = (t - 12) / 3, j = (t - 12) % 3;
+            cams[f * 24 + t] = __ldg(p.inv_K + b * 16 + i * 4 + j);
+        }
+    }
+}
+// the same for the single source frame of photo_fast_kernel and photo_ms_kernel (p.T: its pose), in the form that
+// keeps their prologues short (no division by 21)
+template <class P>
+__device__ __forceinline__ void load_camera(float* cams, const P& p, int b, int tid) {
+    if (tid < 12) {
+        const int i = tid / 4, j = tid % 4;
+        const float* k = p.K + b * 16 + i * 4;
+        const float* tt = p.T + b * 16 + j;
+        float acc = __ldg(k) * __ldg(tt);
+        acc = fmaf(__ldg(k + 1), __ldg(tt + 4), acc);
+        acc = fmaf(__ldg(k + 2), __ldg(tt + 8), acc);
+        acc = fmaf(__ldg(k + 3), __ldg(tt + 12), acc);
+        cams[tid] = acc;
+    } else if (tid < 21) {
+        const int i = (tid - 12) / 3, j = (tid - 12) % 3;
+        cams[tid] = __ldg(p.inv_K + b * 16 + i * 4 + j);
+    }
 }
 
 }  // namespace

@@ -70,41 +70,6 @@ struct MfParams {
 
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
-// scratch accessors: `base` already points at this thread's column (float4 index tid), idx4 = multiple of 256
-// The scratch is re-written every work item and must stay in L2 while the frames stream through it: its accesses carry
-// an evict_last cache policy (ncu, first version without it: 1.65 GB of DRAM writes per launch for 0.1 GB of outputs).
-__device__ __forceinline__ uint64_t scratch_policy() {
-    uint64_t pol;
-    asm("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-    return pol;
-}
-#if defined(MF_NO_HINT)
-__device__ __forceinline__ void st4(float4* base, int idx4, float a, float b, float c, float d) {
-    base[idx4] = make_float4(a, b, c, d);
-}
-__device__ __forceinline__ float4 ld4(const float4* base, int idx4) { return base[idx4]; }
-__device__ __forceinline__ void st1(float* ptr, float a) { *ptr = a; }
-__device__ __forceinline__ float ld1s(const float* ptr) { return *ptr; }
-#else
-__device__ __forceinline__ void st4(float4* base, int idx4, float a, float b, float c, float d) {
-    asm volatile("st.global.L2::cache_hint.v4.f32 [%0], {%1, %2, %3, %4}, %5;" ::"l"(base + idx4), "f"(a), "f"(b), "f"(c),
-                 "f"(d), "l"(scratch_policy()) : "memory");
-}
-__device__ __forceinline__ float4 ld4(const float4* base, int idx4) {
-    float4 v;
-    asm volatile("ld.global.L2::cache_hint.v4.f32 {%0, %1, %2, %3}, [%4], %5;"
-                 : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(base + idx4), "l"(scratch_policy()) : "memory");
-    return v;
-}
-__device__ __forceinline__ void st1(float* ptr, float a) {
-    asm volatile("st.global.L2::cache_hint.f32 [%0], %1, %2;" ::"l"(ptr), "f"(a), "l"(scratch_policy()) : "memory");
-}
-__device__ __forceinline__ float ld1s(const float* ptr) {
-    float v;
-    asm volatile("ld.global.L2::cache_hint.f32 %0, [%1], %2;" : "=f"(v) : "l"(ptr), "l"(scratch_policy()) : "memory");
-    return v;
-}
-#endif
 // one (CTA, source) scratch as seen by one thread
 struct Scr {
     float4* q;       // + tid: Q1 at [k*256], Q2 at [(5+k)*256]
@@ -161,93 +126,6 @@ __device__ __noinline__ void gather_generic_mf(const MsView& v, const float* cam
                 aux_out[k * 12 + 6 + ch] = gzy * g.diy[ch];
             }
             aux_out[k * 12 + 9] = wc.u_raw; aux_out[k * 12 + 10] = wc.v_raw; aux_out[k * 12 + 11] = depth;
-        }
-    }
-}
-
-// Phase A of one (item, source): the register tap pipeline of photo_ms_common.cuh gather_tile_regs, with what the
-// later passes need of the interior pixels parked in the scratch at retire time (nothing extra stays in registers):
-//   KEEP_D   the backward factors stay in registers (last source); otherwise AUX slots 0 / 1 receive them together
-//            with the warped centre values
-//   POSE     AUX slots 2 / 3 (and the depth in slot 0) for the pose-gradient epilogue
-template <bool FASTDIV, bool KEEP_D, bool POSE>
-__device__ __forceinline__ void gather_tile_mf(const MsView& v, const float* cams, const float* src_packed, int tid, int b,
-                                               int x0, int y0, float* pred, float4* aux, float (&D)[4][3], float& lo,
-                                               float& hi) {
-    const int H = v.H, W = v.W;
-    const size_t N = (size_t)H * W;
-    const int oc = tid & 31, os = tid >> 5;
-    int hr, hc;
-    halo_rc(tid, hr, hc);
-    const int ixo = tile_to_img(x0 + oc, W);
-    const int hy = ext_to_img(y0 - 2 + hr, H), hx = ext_to_img(x0 - 2 + hc, W);
-    const bool extra = tid < 272 - FT_THREADS;
-    int er = 0, ec = 0;
-    if (extra) halo_rc(tid + FT_THREADS, er, ec);
-    const float4* sp4 = reinterpret_cast<const float4*>(src_packed) + (size_t)b * N;
-    const float* dp = v.disp.ptr + (size_t)b * (v.disp.h * v.disp.w);
-    const bool up = !(v.disp.h == H && v.disp.w == W);
-    const Camera& cam = *reinterpret_cast<const Camera*>(cams);
-    int py[4];
-#pragma unroll
-    for (int k = 0; k < 4; ++k) py[k] = tile_to_img(y0 + 4 * os + k, H);
-    float dv[5];
-    if (!up) {
-#pragma unroll
-        for (int k = 0; k < 4; ++k) dv[k] = __ldg(dp + (unsigned)(py[k] * W + ixo));
-        dv[4] = __ldg(dp + (unsigned)(hy * W + hx));
-    } else {
-        const UpTap txo = up_tap(ixo, v.disp.sw, v.disp.w);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) dv[k] = up_sample_at(dp, v.disp.w, up_tap(py[k], v.disp.sh, v.disp.h), txo);
-        dv[4] = up_sample_at(dp, v.disp.w, up_tap(hy, v.disp.sh, v.disp.h), up_tap(hx, v.disp.sw, v.disp.w));
-    }
-    Tap tq;
-    float gxq = 0.f, gyq = 0.f;
-    TapAux axq;
-    float4 tvq[4];
-#pragma unroll
-    for (int k = 0; k < 7; ++k) {
-        const bool live = k < 5 || (k == 5 && extra);
-        Tap tn;
-        float gxn = 0.f, gyn = 0.f;
-        TapAux axn;
-        if (k < 4) tn = pixel_tap_nb<FASTDIV, true, POSE>(cam, v, ixo, py[k], dv[k], gxn, gyn, lo, hi, &axn);
-        else if (k == 4) tn = pixel_tap_nb<FASTDIV, false>(cam, v, hx, hy, dv[4], gxn, gyn, lo, hi);
-        else if (k == 5 && extra) {
-            const int iy = ext_to_img(y0 - 2 + er, H), ix = ext_to_img(x0 - 2 + ec, W);
-            const float dvh = up ? up_sample_at(dp, v.disp.w, up_tap(iy, v.disp.sh, v.disp.h), up_tap(ix, v.disp.sw, v.disp.w))
-                                 : __ldg(dp + (unsigned)(iy * W + ix));
-            tn = pixel_tap_nb<FASTDIV, false>(cam, v, ix, iy, dvh, gxn, gyn, lo, hi);
-        }
-        const int j = k - 1;                                // pixel to retire: its taps were requested one chain ago
-        if (j >= 0 && (j < 5 || extra)) {
-            const Gathered g = combine_taps4(tvq, tq, j < 4);
-            const int i2 = j < 4 ? (4 * os + j + 2) * FT_R2 + oc + 2 : (j == 4 ? hr * FT_R2 + hc : er * FT_R2 + ec);
-#pragma unroll
-            for (int ch = 0; ch < 3; ++ch) pred[ch * FT_N2 + i2] = g.v[ch];
-            if (j < 4) {
-                float d[3];
-#pragma unroll
-                for (int ch = 0; ch < 3; ++ch) d[ch] = g.dix[ch] * gxq + g.diy[ch] * gyq;
-                if (KEEP_D) {
-#pragma unroll
-                    for (int ch = 0; ch < 3; ++ch) D[j][ch] = d[ch];
-                    if (POSE) st4(aux, (j * 4 + 0) * FT_THREADS, 0.f, 0.f, 0.f, axq.depth);
-                } else {
-                    st4(aux, (j * 4 + 0) * FT_THREADS, d[0], d[1], d[2], POSE ? axq.depth : 0.f);
-                    st4(aux, (j * 4 + 1) * FT_THREADS, g.v[0], g.v[1], g.v[2], 0.f);
-                }
-                if (POSE) {
-                    st4(aux, (j * 4 + 2) * FT_THREADS, axq.gzx * g.dix[0], axq.gzx * g.dix[1], axq.gzx * g.dix[2], axq.u);
-                    st4(aux, (j * 4 + 3) * FT_THREADS, axq.gzy * g.diy[0], axq.gzy * g.diy[1], axq.gzy * g.diy[2], axq.v);
-                }
-            }
-        }
-        if (live) {
-            load_taps4(sp4, W, tn, tvq);
-            tq = tn; gxq = gxn; gyq = gyn;
-            if (POSE && k < 4) axq = axn;
         }
     }
 }
@@ -434,7 +312,7 @@ __device__ __forceinline__ void source_pass(const MfParams& p, const MsView& v, 
     {
         int tidA = threadIdx.x, bA = geo[0], x0A = geo[1], y0A = geo[2];
         asm volatile("" : "+r"(tidA), "+r"(bA), "+r"(x0A), "+r"(y0A));
-        gather_tile_mf<FASTDIV, LAST, POSE>(v, cams + f * 24, p.src[f], tidA, bA, x0A, y0A, pred, scr.aux, D, lo, hi);
+        gather_tile<FASTDIV, LAST, POSE>(v, cams + f * 24, p.src[f], tidA, bA, x0A, y0A, pred, scr.aux, D, lo, hi);
     }
     if (has_ident) {
 #pragma unroll
@@ -470,21 +348,7 @@ __device__ __forceinline__ void source_pass(const MfParams& p, const MsView& v, 
     }
     if (f == 0 && first_scale) {
         mbar_wait(tgt_bar, it & 1u);
-        // ReflectionPad2d(1) at the image border: TMA zero-fills out-of-image elements; patch them from the
-        // in-image rows / columns of the same tile
-        if (x0B < 2 || y0B < 2 || x0B + FT_T + 2 > W || y0B + FT_T + 2 > H) {
-            for (int i = tidB; i < FT_N2; i += FT_THREADS) {
-                const int r = i / FT_R2, c = i - r * FT_R2;
-                const int ey = y0B - 2 + r, ex = x0B - 2 + c;
-                if (ey < 0 || ey >= H || ex < 0 || ex >= W) {
-                    const int sr = ext_to_img(ey, H) - (y0B - 2), sc = ext_to_img(ex, W) - (x0B - 2);
-#pragma unroll
-                    for (int ch = 0; ch < 3; ++ch)
-                        tgt[ch * FT_NT + r * FT_TP + c + FT_TO] = tgt[ch * FT_NT + sr * FT_TP + sc + FT_TO];
-                }
-            }
-            __syncthreads();
-        }
+        patch_target_border(tgt, tidB, x0B, y0B, H, W);
     }
     // ---- phase B
     phase_b_multi<LAST>(sm, tidB, f, has_ident, okbits, bi, br, idx_r, scr);
@@ -544,22 +408,7 @@ photo_mf_kernel(const MfParams p, const __grid_constant__ CUtensorMap tgt_map) {
         }
         if (b0 != cam_b) {                   // (uniform) the cameras stay in shared memory while the batch item does
             cam_b = b0;
-            if (tid0 < F * 21) {
-                const int f = tid0 / 21, t = tid0 % 21;
-                if (t < 12) {
-                    const int i = t / 4, j = t % 4;
-                    const float* k = p.K + b0 * 16 + i * 4;
-                    const float* tt = p.T[f] + b0 * 16 + j;
-                    float acc = __ldg(k) * __ldg(tt);
-                    acc = fmaf(__ldg(k + 1), __ldg(tt + 4), acc);
-                    acc = fmaf(__ldg(k + 2), __ldg(tt + 8), acc);
-                    acc = fmaf(__ldg(k + 3), __ldg(tt + 12), acc);
-                    cams[f * 24 + t] = acc;
-                } else {
-                    const int i = (t - 12) / 3, j = (t - 12) % 3;
-                    cams[f * 24 + t] = __ldg(p.inv_K + b0 * 16 + i * 4 + j);
-                }
-            }
+            load_cameras(cams, p, F, b0, tid0);
             __syncthreads();
         }
 

@@ -15,19 +15,10 @@
 //   read  12 (target) + 12 F (sources, gathered via L2) + 4 (disp) + 4 Fi (ident)
 //         + 4 Fi (noise);  write 4 (grad_disp)  [+1 sel]
 // Shared memory per CTA: (3 + 1 + 3F) * 720 + 9 * 612 + 612 floats (~43 KB, F=1).
-#include "photo_launch.cuh"
+#include "photo_general.cuh"
 
 namespace {
 
-#define PH_TW 32
-#define PH_TH 16
-#define PH_R2W (PH_TW + 4)
-#define PH_R2H (PH_TH + 4)
-#define PH_R1W (PH_TW + 2)
-#define PH_R1H (PH_TH + 2)
-#define PH_R2 (PH_R2W * PH_R2H)
-#define PH_R1 (PH_R1W * PH_R1H)
-#define PH_THREADS 256
 #define PH_MAXF DMH_PHOTO_MAX_FRAMES
 
 struct PhotoParams {
@@ -54,21 +45,6 @@ struct PhotoParams {
     const float* hint_valid;       // (B,1,H,W)
     float* grad_hint;              // (B,1,H,W) d(sum proxy*mask_h)/d(up-sampled disp)
 };
-
-// 3x3 window statistics for one channel plane in shared memory around R2 position (r+1, c+1).
-// Same arithmetic as the single-source fast kernel and the identity-loss kernel (row sums of 3, then 3 rows,
-// mean = sum * (1/9)) so that the automask compares like with like.
-__device__ __forceinline__ SsimStatsRows window_stats(const float* __restrict__ xs, const float* __restrict__ ys, int r,
-                                                  int c) {
-    Row5 rows[3];
-#pragma unroll
-    for (int dy = 0; dy < 3; ++dy) {
-        const float* x = xs + (r + dy) * PH_R2W + c;
-        const float* y = ys + (r + dy) * PH_R2W + c;
-        rows[dy] = row5(x[0], x[1], x[2], y[0], y[1], y[2]);
-    }
-    return ssim_stats_rows(rows[0], rows[1], rows[2]);
-}
 
 template <int F>
 __global__ void __launch_bounds__(PH_THREADS)
@@ -97,32 +73,9 @@ photo_scale_kernel(const PhotoParams p) {
     const float w_l1 = no_ssim ? 1.0f / 3.0f : 0.15f / 3.0f;
 
     // ---- cameras
-    if (tid < F * 21) {
-        const int f = tid / 21, t = tid % 21;
-        if (t < 12) {
-            const int i = t / 4, j = t % 4;
-            const float* k = p.K + b * 16 + i * 4;
-            const float* tt = p.T[f] + b * 16 + j;
-            float acc = __ldg(k) * __ldg(tt);
-            acc = fmaf(__ldg(k + 1), __ldg(tt + 4), acc);
-            acc = fmaf(__ldg(k + 2), __ldg(tt + 8), acc);
-            acc = fmaf(__ldg(k + 3), __ldg(tt + 12), acc);
-            cams[f * 24 + t] = acc;
-        } else {
-            const int i = (t - 12) / 3, j = (t - 12) % 3;
-            cams[f * 24 + t] = __ldg(p.inv_K + b * 16 + i * 4 + j);
-        }
-    }
+    load_cameras(cams, p, F, b, tid);
     // ---- target tile + depth, 2-px reflect halo
-    for (int i = tid; i < PH_R2; i += PH_THREADS) {
-        const int r = i / PH_R2W, c = i % PH_R2W;
-        const int iy = ext_to_img(y0 - 2 + r, H), ix = ext_to_img(x0 - 2 + c, W);
-        const size_t o = (size_t)iy * W + ix;
-#pragma unroll
-        for (int ch = 0; ch < 3; ++ch) tgt[ch * PH_R2 + i] = __ldg(p.target + ((size_t)b * 3 + ch) * N + o);
-        const float dv = load_disp(p.disp, b, iy, ix, H, W);
-        dep[i] = is_depth ? dv : disp_to_depth(dv, p.ds);
-    }
+    load_target_depth(p.target, p.disp, p.ds, is_depth, b, x0, y0, H, W, N, tgt, dep);
     __syncthreads();
 
     // ---- warp every source frame into shared memory

@@ -51,6 +51,25 @@ __device__ __forceinline__ void tma_load_4d(void* dst, const CUtensorMap* map, u
 #define FT_STRIPS 7
 #define FT_ROWS 5                // 7 strips x 5 rows >= 34 ring rows
 
+// ReflectionPad2d(1) at the image border of the target tile tgt [3][36][40] of the tile at (x0, y0): the TMA load
+// zero-fills out-of-image elements; a border tile patches them from the in-image rows / columns of the same tile (and
+// ends with a barrier).  Uniform across the CTA.
+__device__ __forceinline__ void patch_target_border(float* tgt, int tid, int x0, int y0, int H, int W) {
+    if (x0 < 2 || y0 < 2 || x0 + FT_T + 2 > W || y0 + FT_T + 2 > H) {
+        for (int i = tid; i < FT_N2; i += FT_THREADS) {
+            const int r = i / FT_R2, c = i - r * FT_R2;
+            const int ey = y0 - 2 + r, ex = x0 - 2 + c;
+            if (ey < 0 || ey >= H || ex < 0 || ex >= W) {
+                const int sr = ext_to_img(ey, H) - (y0 - 2), sc = ext_to_img(ex, W) - (x0 - 2);
+#pragma unroll
+                for (int ch = 0; ch < 3; ++ch)
+                    tgt[ch * FT_NT + r * FT_TP + c + FT_TO] = tgt[ch * FT_NT + sr * FT_TP + sc + FT_TO];
+            }
+        }
+        __syncthreads();
+    }
+}
+
 // dynamic shared memory of photo_fast_kernel and photo_ms_kernel: target tile, warped tile, the 9 coefficient planes,
 // camera (24 floats), reduction slots (32 floats) and the gate bytes
 size_t tile_smem_bytes() { return sizeof(float) * (3 * FT_NT + 3 * FT_N2 + 9 * FT_N1 + 24 + 32) + FT_N1; }
